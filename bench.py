@@ -1,12 +1,14 @@
 """Headline benchmark: clips/sec of one `r21d_byol` pretraining step (main_byol.py:60-91) on 16x112x112 clips.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B_per_gpu] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B_per_gpu] [--impl native|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); per-GPU work is fixed (weak scaling).  Rank 0 prints ONE JSON
 line.  A "step" = online fwd (2 views) + predictor + EMA + target fwd (2 views) + BYOL / 6 CE losses + backward +
 (grad all-reduce) + clip + SGD + bf16 re-pack, on synthetic U(-1,1) clips and seeded random-init weights.
 `value` = samples/s with inputs resident in HBM; `e2e` = the same through R21DBYOL.train_step with pinned HOST clips
 and labels copied in and the loss vector copied out every step.  1 clip = 1 sample = two views (SURVEY.md 8d).
+`--dump-outputs DIR` writes what the last device-resident timed step left to its caller (rank 0): the loss vector and a
+fixed sample of every state_dict entry, as DIR/<name>.npy (see dump_outputs), so two builds can be compared value by value.
 """
 from __future__ import annotations
 
@@ -331,6 +333,36 @@ def ncu_traffic(kernel: str, B: int):
     return (total / len(ids) if ids else None), (src + (" [" + note + "]" if note else ""))
 
 
+DUMP_SAMPLE = 16384             # values kept of a larger tensor: r21d_byol's 351 state entries come to 4.1 MB
+DUMP_LIMIT = 64 << 20
+
+
+def dump_sample(t: torch.Tensor, k: int = DUMP_SAMPLE) -> torch.Tensor:
+    """t flattened; above k elements, the values at k seeded positions that depend only on t's size (the same on every run)."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= k:
+        return flat
+    idx = torch.randint(0, flat.numel(), (k,), generator=torch.Generator().manual_seed(0))
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(out_dir: str, losses: torch.Tensor, state: dict) -> int:
+    """Writes what one train_step hands its caller -- the returned loss vector and the module state it leaves -- as
+    <out_dir>/losses.npy (the 8 values of R21DBYOL.train_step) and <out_dir>/state.<key>.npy per state_dict entry
+    (dump_sample of it).  Floating-point values as float32, integer counters as float64.  Returns the bytes written."""
+    import numpy as np
+    arrays = {"losses": losses, **{f"state.{k}": dump_sample(v) for k, v in state.items()}}
+    arrays = {n: t.detach().cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64)
+              for n, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
+    return total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -344,7 +376,15 @@ def main():
     ap.add_argument("--config5-timeout", type=float, default=240.0, help="seconds before a hung config 5 sub-record is cut off")
     ap.add_argument("--bn-sync", default="local", choices=["local", "world", "world-p2p"],
                     help="local: per-GPU BatchNorm statistics (the reference's behaviour); world: SyncBN over all ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss vector and a fixed sample of the model state after the last timed step as "
+                         "DIR/<name>.npy (rank 0).  Native arm only: the reference arm times a sampled batch of "
+                         "--ref-batch clips, not the --batch clips of the native step, so its outputs would not compare")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs")
     claim_stdout()
     from cstp_b200 import parallel
     rank, world, local = parallel.env_world()
@@ -412,6 +452,9 @@ def main():
         bs.check()                        # a timed-out peer exchange must not produce a number
     clk = clocks.stop() if rank == 0 else None
     final = losses.tolist()
+    if args.dump_outputs and rank == 0:
+        # before the end-to-end region steps the same model on: `losses` and the state are the last timed step's
+        dump_outputs(args.dump_outputs, losses, model.state_dict())
 
     # ---------------- end-to-end region: pinned host clips in, loss vector out, every step.  Each step's clips and labels
     # are copied host -> device inside the timed region (the copy of step i+1 runs on a side stream while step i

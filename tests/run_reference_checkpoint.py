@@ -1,4 +1,5 @@
-"""Checkpoint hand-off with the UNMODIFIED reference in both directions -- TEST INFRASTRUCTURE, build container only.
+"""Checkpoint hand-off with the UNMODIFIED reference (the checkout named by CSTP_REFERENCE) in both directions -- TEST
+INFRASTRUCTURE.
 
     python tests/run_reference_checkpoint.py <out_dir>
 
@@ -18,7 +19,7 @@ import types
 
 import torch
 
-REF = os.environ.get("CSTP_REFERENCE", "/root/reference")
+REF = os.environ["CSTP_REFERENCE"]          # the reference checkout (tests/test_reference_integration.py)
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = sys.argv[1]
 B, T, S = 4, 4, 32

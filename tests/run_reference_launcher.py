@@ -1,5 +1,5 @@
-"""Runs the UNMODIFIED reference launcher loop (main_byol.py: main_worker -> train_BYOL, imported from /root/reference,
-never copied) on top of the cstp_b200 drop-in modules -- TEST INFRASTRUCTURE, build container only.
+"""Runs the UNMODIFIED reference launcher loop (main_byol.py: main_worker -> train_BYOL, imported from the checkout named by
+CSTP_REFERENCE, never copied) on top of the cstp_b200 drop-in modules -- TEST INFRASTRUCTURE.
 
     python tests/run_reference_launcher.py <out_dir>
 
@@ -20,7 +20,7 @@ import types
 
 import torch
 
-REF = os.environ.get("CSTP_REFERENCE", "/root/reference")
+REF = os.environ["CSTP_REFERENCE"]          # the reference checkout (tests/test_reference_integration.py)
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = sys.argv[1]
 B, T, S, EPOCHS = 4, 4, 32, 2

@@ -1,9 +1,11 @@
-"""bench.py pieces that run without a GPU: the reference arm's JSON line (the CPU oracle port on a bounded sample) and the
-helper behind roofline.traffic."""
+"""bench.py pieces that run without a GPU: the reference arm's JSON line (the CPU oracle port on a bounded sample), the
+helper behind roofline.traffic and the --dump-outputs writer; on a GPU, --dump-outputs through the native arm."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,6 +32,64 @@ def test_roofline_traffic_comes_from_a_committed_capture_with_its_provenance():
     assert src.startswith("profiles/r02_ncu_conv_halo_b60_dram.csv") and "commit" in src
     assert 1.5e9 < per_launch < 2.5e9          # ~1.88 GB per launch = the algorithmic bytes of the layers it runs
     assert bench.ncu_traffic("conv_halo_kernel", 7) == (None, None)
+
+
+def test_dump_outputs_writes_the_loss_vector_and_a_fixed_sample_of_the_state(tmp_path):
+    """--dump-outputs: float32 / float64 arrays, within 64 MB for the flagship model, the same positions on every run."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    from cstp_b200.models.pace.r21d_byol import R21DBYOL
+    torch.manual_seed(1)
+    state = R21DBYOL(pretrain=True).state_dict()
+    losses = torch.arange(8, dtype=torch.float32)
+    total = bench.dump_outputs(str(tmp_path / "a"), losses, state)
+    assert total <= bench.DUMP_LIMIT
+    assert bench.dump_outputs(str(tmp_path / "b"), losses, state) == total
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(["losses.npy"] + [f"state.{k}.npy" for k in state])
+    assert sum((tmp_path / "a" / n).stat().st_size for n in names) < bench.DUMP_LIMIT
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), n
+    assert np.array_equal(np.load(tmp_path / "a" / "losses.npy"), losses.numpy())
+    w = state["online_net.conv2.block1.conv1.spatial_conv.weight"].reshape(-1)
+    got = np.load(tmp_path / "a" / "state.online_net.conv2.block1.conv1.spatial_conv.weight.npy")
+    assert w.numel() > bench.DUMP_SAMPLE and got.shape == (bench.DUMP_SAMPLE,) and np.isin(got, w.numpy()).all()
+    bn = state["online_net.conv1.bn.running_mean"]
+    assert np.array_equal(np.load(tmp_path / "a" / "state.online_net.conv1.bn.running_mean.npy"), bn.numpy())
+    assert np.load(tmp_path / "a" / "state.online_net.conv1.bn.num_batches_tracked.npy").dtype == np.float64
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path_repeat_run_to_run(tmp_path):
+    """--dump-outputs through main() on the GPU: the loss vector of the last timed step (the one the JSON line reports) and
+    the CUDA-resident model state it left, bit-identical on two runs with the same arguments."""
+    import numpy as np
+
+    def run(d):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "3",
+                              "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900,
+                             cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-3000:]
+        return json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+
+    line = run(tmp_path / "a")
+    run(tmp_path / "b")
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(p.name for p in (tmp_path / "b").iterdir()) and len(names) == 352
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert np.isfinite(a).all() and np.array_equal(a, b), n
+    losses = np.load(tmp_path / "a" / "losses.npy")
+    assert losses.tolist() == [*line["losses_last_step"]["ce"], losses[6], line["losses_last_step"]["byol"]]
+
+
+def test_bench_rejects_a_run_without_timed_steps():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps must be at least 1" in out.stderr
 
 
 def test_watchdog_prints_the_measured_line_when_a_sub_record_hangs():

@@ -89,7 +89,10 @@ def _worker(rank, world, path, out):
     dist.destroy_process_group()
 
 
-def test_ddp_wrapped_dropin_equals_fused_gradsync_world2():
+def test_ddp_wrapped_dropin_equals_fused_gradsync_world2(monkeypatch):
+    # the ranks run the host logic over the CPU stand-in of the kernel layer: they must see no GPU, or generate_model places
+    # rank r on cuda:r (which a one-GPU machine does not have)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     d = tempfile.mkdtemp()
     mp.spawn(_worker, args=(2, os.path.join(d, "rdzv"), os.path.join(d, "out")), nprocs=2, join=True)
     r0, r1 = (torch.load(os.path.join(d, f"out.{r}"), weights_only=False) for r in range(2))
