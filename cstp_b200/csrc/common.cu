@@ -1,5 +1,4 @@
 #include "common.h"
-#include <cstdlib>
 
 #include <cudaTypedefs.h>
 
@@ -72,38 +71,6 @@ int num_sms() {
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
   }
   return sms;
-}
-
-static int env_int(const char* name, int dflt, int lo, int hi) {
-  const char* v = getenv(name);
-  if (v == nullptr || *v == 0) return dflt;
-  const int x = atoi(v);
-  return x < lo ? lo : (x > hi ? hi : x);
-}
-
-int smem_budget() {
-  static int b = env_int("CSTP_SMEM_KB", 227, 64, 227) * 1024;
-  return b;
-}
-
-int conv_cluster() {
-  static int c = env_int("CSTP_CONV_CLUSTER", 1, 0, 1);
-  return c;
-}
-
-int bn_bwd_rows() {
-  static int c = env_int("CSTP_BN_BWD_ROWS", 4, 2, 4);
-  return c;
-}
-
-int bn_apply_rows() {
-  static int c = env_int("CSTP_BN_APPLY_ROWS", 2, 2, 4);
-  return c;
-}
-
-int stream_ctas_per_sm() {
-  static int c = env_int("CSTP_STREAM_CTAS_PER_SM", 8, 1, 16);
-  return c;
 }
 
 }  // namespace cstp

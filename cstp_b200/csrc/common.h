@@ -53,13 +53,10 @@ int num_sms();
 
 // Shared-memory budget (bytes) of the one-CTA-per-SM tensor-core kernels and the CTAs-per-SM share of the streaming
 // kernels: together they decide whether an HBM-bound kernel on one stream can be co-resident with a tensor-bound
-// kernel on the other (every resident CTA also costs 1 KB of reserved shared memory).  Tunable for experiments through
-// CSTP_SMEM_KB / CSTP_STREAM_CTAS_PER_SM (read once).
-int smem_budget();
-int stream_ctas_per_sm();
-int bn_bwd_rows();           // CSTP_BN_BWD_ROWS (2 or 4, default 4): rows per trip of bn_bwd_apply_kernel
-int bn_apply_rows();         // CSTP_BN_APPLY_ROWS (2 or 4, default 2: 4 measured neutral): rows per trip of bn_apply_kernel without a second coefficient set
-int conv_cluster();          // CSTP_CONV_CLUSTER (default 1): conv_gemm as CTA pairs with the weight tile multicast
+// kernel on the other (every resident CTA also costs 1 KB of reserved shared memory; the co-residency sweep of
+// profiles/r01_overlap_sweep.txt kept these values).  ops.py SMEM_LIMIT is the same budget.
+constexpr int kSmemBudget = 227 * 1024;
+constexpr int kStreamCtasPerSm = 8;
 
 inline int ceil_div(long long a, long long b) { return static_cast<int>((a + b - 1) / b); }
 

@@ -482,7 +482,7 @@ extern "C" int cstp_conv_plan_create(const cstp_conv_desc* d, cstp_conv_plan** o
   const uint32_t stage_bytes = kABytes + k.b_bytes;
   const int bar_bytes = 256;       // 5 + 3 * kMaxStages mbarriers + the TMEM slot
   const int xtab_bytes = xform ? static_cast<int>(xform_table_bytes(d->pro.groups, d->pro.Cp)) : 0;      // prologue coefficient table
-  int stages = (smem_budget() - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(stage_bytes);
+  int stages = (kSmemBudget - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(stage_bytes);
   if (stages > kMaxStages) stages = kMaxStages;
   if (stages < 2) {
     delete plan;
@@ -500,7 +500,7 @@ extern "C" int cstp_conv_plan_create(const cstp_conv_desc* d, cstp_conv_plan** o
   plan->grid = static_cast<int>(total < sms ? total : sms);
   plan->cluster = 1;
   // CTA pairs when the persistent grid is full anyway (deep layers: many tiles, weight tiles of 16-32 KB per K-block)
-  if (conv_cluster() && !xform && total >= 2LL * sms && m_tiles >= 2 && d->n_tile % 16 == 0 && d->n_tile >= 32) {
+  if (!xform && total >= 2LL * sms && m_tiles >= 2 && d->n_tile % 16 == 0 && d->n_tile >= 32) {
     static int max_pairs = -1;        // co-resident clusters of two with this kernel's footprint (one CTA per SM)
     if (max_pairs < 0) {
       max_pairs = 0;

@@ -8,12 +8,13 @@
 //     atom aligned);
 //   * when all weight K-blocks of one N tile fit next to the activation pipeline they are loaded ONCE per CTA
 //     ("resident B"); every CTA then keeps its N tile for its whole life (blockIdx.y) and walks M tiles only.
-//   * "slab mode" (64-column layers): a tcgen05.mma of 128 x 64 x 16 cannot be fed faster than one per ~76 cycles
-//     (its 4 KB A slice comes out of shared memory at 64 B/clk) while the tensor pipe needs 32.  So G consecutive output
-//     slabs along the tap axis share one accumulator of G x 64 columns: every INPUT slab is staged once and multiplied,
-//     in ONE MMA of up to 3 x 64 columns, with the stacked weights [tap +1 | tap 0 | tap -1] of the output slabs it
-//     feeds (a row offset into the resident weight block picks the sub-range at the tile's borders).  36 tap units
-//     of a 1x3x3 tile with G = 4 take 18 MMA series instead of 36, and every A slice is read once instead of three times.
+//   * "slab mode" (64-column dgrad of the 1x3x3 layers): a tcgen05.mma of 128 x 64 x 16 cannot be fed faster than one
+//     per ~76 cycles (its 4 KB A slice comes out of shared memory at 64 B/clk) while the tensor pipe needs 32.  So G
+//     consecutive output rows (slabs along h) share one accumulator of G x 64 columns: every INPUT slab is staged once
+//     and multiplied, in ONE MMA of up to 3 x 64 columns, with the stacked weights [tap +1 | tap 0 | tap -1] of the
+//     output slabs it feeds (a row offset into the resident weight block picks the sub-range at the tile's borders).
+//     36 tap units of a 1x3x3 tile with G = 4 take 18 MMA series instead of 36, and every A slice is read once instead
+//     of three times.
 // Same math, epilogue and output layout as conv_gemm.cu.
 // Replaces cuDNN conv3d fwd/dgrad behind models/pace/r21d_byol.py:81-97 (main_byol.py:87 for the dgrad).
 #include "common.h"
@@ -27,7 +28,7 @@ constexpr int kHcMaxStages = 8;
 constexpr int kHcSmemLimit = 232448;
 constexpr int kHcMaxGroups = 4;
 constexpr int kHcMaxTaps = 16;
-constexpr int kHcMaxSlabs = 8;           // staged input slabs per tile in slab mode (G + taps along the slab axis - 1)
+constexpr int kHcMaxSlabs = 8;           // staged input slabs per tile in slab mode (G + taps along h - 1)
 
 struct HcGroup {
   int dw, dh, dt;       // origin offset of the staged (halo) box from the tile origin
@@ -70,11 +71,11 @@ struct ConvHaloKParams {
   float* out_f32;
   const float* bias;
   long long out_off, osw, osh, ost, osn;
-  int step_h, step_t;      // tile step along h / t (bh / bt, or G along the slab axis in slab mode)
-  // slab mode (slab_g > 1): G output slabs of slab_cols columns each on the accumulator's N axis
-  int slab_g, slab_axis;   // axis 1: h, 2: t
+  int step_h;              // tile step along h (bh, or G in slab mode)
+  // slab mode (slab_g > 1): G output rows of slab_cols columns each on the accumulator's N axis
+  int slab_g;
   int slab_in;             // staged input slabs per tile
-  int slab_nslots;         // taps along the slab axis (weights of one w tap: nslots stacked blocks of slab_cols rows)
+  int slab_nslots;         // taps along h (weights of one w tap: nslots stacked blocks of slab_cols rows)
   int slab_cols;
   uint32_t res_tap_stride, res_chunk_stride, res_tail_base, res_tail_tap_stride;     // resident weight block layout
   int slab_order[kHcMaxSlabs];    // load / issue order of the input slabs (the first MMA of an accumulator column range
@@ -201,9 +202,8 @@ __global__ void __launch_bounds__(kXform ? kHcThreads + kHcXformThreads : kHcThr
   // the producer / issuer warpgroup and the transform warpgroup hand registers to the epilogue warpgroup (setmaxnreg at
   // the head of each warpgroup's branch, where ptxas can see which code runs under which budget).
   constexpr bool kRealloc = kStats && kXform;
-  // slab mode is compiled into every instantiation but the prologue-without-statistics one (no layer needs it there, and its
-  // 128-register budget spills with the extra paths)
-  constexpr bool kSlabOk = !(kXform && !kStats);
+  // slab mode (plain dgrad only) is compiled into the instantiation without prologue and statistics
+  constexpr bool kSlabOk = !kStats && !kXform;
 
   // Roles run WARP-CONVERGED: all 32 lanes walk the loops and poll the mbarriers, one elected lane issues the TMA /
   // tcgen05 instructions.  (With a single-lane branch the compiler cannot keep descriptors and addresses in uniform
@@ -237,16 +237,12 @@ __global__ void __launch_bounds__(kXform ? kHcThreads + kHcXformThreads : kHcThr
       pt /= p.tiles_w;
       const int h0 = (pt % p.tiles_h) * p.step_h;
       pt /= p.tiles_h;
-      const int t0 = (pt % p.tiles_t) * p.step_t;
+      const int t0 = (pt % p.tiles_t) * p.bt;
       pt /= p.tiles_t;
       const int n0 = pt * p.bn;
       for (int g = 0; g < n_loads; ++g) {
         HcGroup gr = p.groups[pslab ? 0 : g];
-        if (pslab) {               // input slab s of the tile: the first slab's origin moved s steps along the slab axis
-          const int sl = p.slab_order[g];
-          gr.dh += p.slab_axis == 1 ? sl : 0;
-          gr.dt += p.slab_axis == 2 ? sl : 0;
-        }
+        if (pslab) gr.dh += p.slab_order[g];      // input slab s of the tile: the first slab's origin moved s rows along h
         for (int c = 0; c < p.chunks; ++c) {
           mbar_wait(&empty[stage], phase ^ 1u);
           if (leader) {
@@ -406,7 +402,7 @@ __global__ void __launch_bounds__(kXform ? kHcThreads + kHcXformThreads : kHcThr
     const uint32_t xtab_addr = smem_u32(xtab);
     const uint32_t stage_addr0 = smem_u32(stage0);
     const uint32_t stage_bytes = p.stage_bytes;
-    const int n_groups = (kSlabOk && p.slab_g) ? p.slab_in : p.n_groups, chunks = p.chunks, stages = p.stages;
+    const int n_groups = p.n_groups, chunks = p.chunks, stages = p.stages;
     const bool has_tail = p.tail != 0;
     const uint32_t units_full = p.a_bytes >> 4, units_tail = p.a_bytes_tail >> 4;
     const uint32_t mask_tail = p.tail == 16 ? 1u : 3u;
@@ -465,7 +461,7 @@ __global__ void __launch_bounds__(kXform ? kHcThreads + kHcXformThreads : kHcThr
       pt /= p.tiles_w;
       const int h = (pt % p.tiles_h) * p.step_h + rh;
       pt /= p.tiles_h;
-      const int t = (pt % p.tiles_t) * p.step_t + rt;
+      const int t = (pt % p.tiles_t) * p.bt + rt;
       pt /= p.tiles_t;
       const int n_first = pt * p.bn;                          // first sample of the tile
       const int n = n_first + rn;
@@ -483,37 +479,27 @@ __global__ void __launch_bounds__(kXform ? kHcThreads + kHcXformThreads : kHcThr
           if (cur_group >= 0) stats_flush(acc, wsum, tot + cur_group * 128, q, lane);
           cur_group = g;
         }
-        // slab mode: G column blocks of 64 = G output slabs along the slab axis, all of them feed the same 64 channel sums
-        const int n_os = p.slab_g ? p.slab_g : 1;
-        const long long ostep = p.slab_axis == 1 ? p.osh : p.ost;
-        const int pos = p.slab_axis == 1 ? h : t, lim = p.slab_g ? (p.slab_axis == 1 ? p.Ht : p.Tt) : 0x7fffffff;
-        for (int o = 0; o < n_os; ++o) {
-          const bool ok = valid && pos + o < lim;
-          __nv_bfloat16* dst = p.out + off + o * ostep;
-          const uint32_t ta = taddr + static_cast<uint32_t>(o * 64);
-          uint32_t va[16], vb[16];
-          tmem_ld16(ta, va);
-          tmem_ld_wait();
-          tmem_ld16(ta + 16, vb);
-          stats_chunk<0>(va, dst, ok, acc);
-          tmem_ld_wait();
-          tmem_ld16(ta + 32, va);
-          stats_chunk<16>(vb, dst, ok, acc);
-          tmem_ld_wait();
-          tmem_ld16(ta + 48, vb);
-          stats_chunk<32>(va, dst, ok, acc);
-          tmem_ld_wait();
-          stats_chunk<48>(vb, dst, ok, acc);
-        }
+        __nv_bfloat16* dst = p.out + off;
+        uint32_t va[16], vb[16];
+        tmem_ld16(taddr, va);
+        tmem_ld_wait();
+        tmem_ld16(taddr + 16, vb);
+        stats_chunk<0>(va, dst, valid, acc);
+        tmem_ld_wait();
+        tmem_ld16(taddr + 32, va);
+        stats_chunk<16>(vb, dst, valid, acc);
+        tmem_ld_wait();
+        tmem_ld16(taddr + 48, vb);
+        stats_chunk<32>(va, dst, valid, acc);
+        tmem_ld_wait();
+        stats_chunk<48>(vb, dst, valid, acc);
       } else if (kSlabOk && p.slab_g) {
-        // slab mode: column block o of the accumulator is output slab o along the slab axis (plain bf16 rows)
-        const long long ostep = p.slab_axis == 1 ? p.osh : p.ost;
-        const int pos = p.slab_axis == 1 ? h : t, lim = p.slab_axis == 1 ? p.Ht : p.Tt;
+        // slab mode: column block o of the accumulator is output row h + o (plain bf16 rows)
         for (int o = 0; o < p.slab_g; ++o) {
-          const bool ok = valid && pos + o < lim;
+          const bool ok = valid && h + o < p.Ht;
           const uint32_t ta = taddr + static_cast<uint32_t>(o * p.slab_cols);
-          if (p.accumulate) epilogue_row_bf16<true>(ta, p.slab_cols, p.out + off + o * ostep, ok);
-          else epilogue_row_bf16<false>(ta, p.slab_cols, p.out + off + o * ostep, ok);
+          if (p.accumulate) epilogue_row_bf16<true>(ta, p.slab_cols, p.out + off + o * p.osh, ok);
+          else epilogue_row_bf16<false>(ta, p.slab_cols, p.out + off + o * p.osh, ok);
         }
       } else if (p.fast_store) {
         // plain bf16 output (optionally accumulated into what is there): pipelined, one 32-byte store per 16 columns.
@@ -629,14 +615,16 @@ extern "C" int cstp_conv_halo_plan_create(const cstp_conv_halo_desc* d, cstp_con
   const bool xform = d->pro.scale != nullptr;
   const int G = d->slabs.n_slabs > 1 ? d->slabs.n_slabs : 0;
   if (G) {
-    // slab mode: taps[] lists, for every w tap j, the nslots stacked weight blocks (tap offset along the slab axis
-    // DEscending); groups[0] is the origin of the first input slab; one tile = 128 positions x G output slabs
+    // slab mode: taps[] lists, for every w tap j, the nslots stacked weight blocks (tap offset along h DEscending);
+    // groups[0] is the origin of the first input slab; one tile = 128 positions x G output rows
     const cstp_halo_slabs& sl = d->slabs;
-    CSTP_REQUIRE((sl.axis == 1 || sl.axis == 2) && sl.nslots >= 1 && sl.nslots <= 4 && d->n_taps % sl.nslots == 0);
+    if (sl.axis != 1 || xform || d->stats_partials != nullptr)
+      return fail_inval("slab mode runs along h (axis 1) without an operand prologue or fused statistics");
+    CSTP_REQUIRE(sl.nslots >= 1 && sl.nslots <= 4 && d->n_taps % sl.nslots == 0);
     CSTP_REQUIRE(G + sl.nslots - 1 <= kHcMaxSlabs && d->n_groups == 1 && d->groups[0].n_taps == d->n_taps);
     CSTP_REQUIRE(d->Np % 16 == 0 && d->n_tile == G * d->Np && d->n_tile <= 256 && sl.nslots * d->Np <= 256);
-    CSTP_REQUIRE((sl.axis == 1 ? d->bh : d->bt) == 1 && (sl.axis == 1 ? d->halo_h : d->halo_t) == 0);
-    CSTP_REQUIRE((!xform || d->stats_partials != nullptr) && d->allow_resident && d->bias == nullptr && d->out_f32 == nullptr);
+    CSTP_REQUIRE(d->bh == 1 && d->halo_h == 0);
+    CSTP_REQUIRE(d->allow_resident && d->bias == nullptr && d->out_f32 == nullptr);
   }
   if (xform) {
     // the prologue picks its coefficient row per tile: one sample per tile, the statistics groups split the N axis evenly
@@ -693,11 +681,10 @@ extern "C" int cstp_conv_halo_plan_create(const cstp_conv_halo_desc* d, cstp_con
       return rc;
     }
   }
-  k.step_h = (G && d->slabs.axis == 1) ? G : d->bh;
-  k.step_t = (G && d->slabs.axis == 2) ? G : d->bt;
+  k.step_h = G ? G : d->bh;
   k.tiles_w = ceil_div(d->Wt, d->bw);
   k.tiles_h = ceil_div(d->Ht, k.step_h);
-  k.tiles_t = ceil_div(d->Tt, k.step_t);
+  k.tiles_t = ceil_div(d->Tt, d->bt);
   k.tiles_n = ceil_div(d->Nt, d->bn);
   k.bw = d->bw; k.bh = d->bh; k.bt = d->bt; k.bn = d->bn;
   k.Wt = d->Wt; k.Ht = d->Ht; k.Tt = d->Tt; k.Nt = d->Nt;
@@ -736,7 +723,6 @@ extern "C" int cstp_conv_halo_plan_create(const cstp_conv_halo_desc* d, cstp_con
     const cstp_halo_slabs& sl = d->slabs;
     const int span = sl.nslots - 1, n_in = G + span;
     k.slab_g = G;
-    k.slab_axis = sl.axis;
     k.slab_in = n_in;
     k.slab_nslots = sl.nslots;
     k.slab_cols = d->Np;
@@ -786,12 +772,12 @@ extern "C" int cstp_conv_halo_plan_create(const cstp_conv_halo_desc* d, cstp_con
   k.pro_groups = d->pro.groups;
   k.pro_cp = d->pro.Cp;
   if (d->stats_partials != nullptr &&
-      !(k.fast_store && !d->accumulate && d->Np == 64 && d->n_tile == (G ? G * 64 : 64) &&
+      !(k.fast_store && !d->accumulate && d->Np == 64 && d->n_tile == 64 &&
         (d->stats_groups == 1 || d->stats_groups == 2) && d->Nt % d->stats_groups == 0 &&
         (d->Nt / d->stats_groups) % d->bn == 0)) {
     delete plan;
-    return fail_inval("fused statistics need Np == 64 (one 64-column tile, or slab mode), a plain aligned bf16 output and 1 or 2 "
-                      "groups dividing N into multiples of bn");
+    return fail_inval("fused statistics need Np == 64 (one 64-column tile), a plain aligned bf16 output and 1 or 2 groups "
+                      "dividing N into multiples of bn");
   }
   const int stats_bytes = d->stats_partials != nullptr ? 3072 : 0;
   const int xtab_bytes = xform ? static_cast<int>(xform_table_bytes(d->pro.groups, d->pro.Cp)) : 0;
@@ -869,7 +855,7 @@ extern "C" int cstp_conv_halo_plan_create(const cstp_conv_halo_desc* d, cstp_con
   // shared-memory plan: resident weights when every K-block of this N tile fits beside >= 3 activation stages
   const int bar_bytes = 256;
   const long long res_all = 1LL * d->n_taps * k.tap_bytes;
-  const long long budget = smem_budget() - 1024 - bar_bytes - stats_bytes - xtab_bytes;
+  const long long budget = kSmemBudget - 1024 - bar_bytes - stats_bytes - xtab_bytes;
   k.xtab_off = static_cast<uint32_t>(bar_bytes + stats_bytes);
   if (d->allow_resident && res_all + (pitch == 8 ? 3LL : 2LL) * k.a_stride <= budget) {
     k.resident = 1;

@@ -1,4 +1,4 @@
-// HBM-bound kernels of the hot path: weight packing, stem im2col, training-mode BatchNorm (statistics,
+// HBM-bound kernels of the hot path: weight packing, stem row packing, training-mode BatchNorm (statistics,
 // finalize, apply + ReLU + residual, backward reduce / apply), average pooling, column sums and casts.
 // All activations are bf16 [rows][Cp] (NDHWC flattened), processed as 16-byte vectors of 8 channels.
 // Replaces ATen/cuDNN batch_norm, relu, add, adaptive_avg_pool3d behind models/pace/r21d_byol.py:83-97,141-148,210-223.
@@ -107,76 +107,6 @@ __global__ void __launch_bounds__(256) pack_weights_batched_kernel(const long lo
   }
 }
 
-// ------------------------------------------------------------------------------------------- stem im2col
-// One CTA per (n, t, ho): the 3 x 7 input rows this output row needs are staged in shared memory with coalesced
-// float4 loads (zero rows / columns for the padding), then every thread assembles 16-byte vectors of 8 consecutive
-// K columns (k = ci*49 + kh*7 + kw) for the 56 output positions.  The first version gathered straight from global
-// memory and ran at 0.85 TB/s.
-constexpr int kStemMaxW = 256;
-__global__ void __launch_bounds__(256) stem_im2col_kernel(const float* __restrict__ x, int N, int T, int H, int W,
-                                                          __nv_bfloat16* __restrict__ col, int ldk) {
-  __shared__ float rows[3 * 7][kStemMaxW + 8];       // [ci*7 + kh][3 + wi], 3 zero columns of left padding
-  const int Ho = H / 2, Wo = W / 2;
-  int b = blockIdx.x;
-  const int ho = b % Ho;
-  b /= Ho;
-  const int t = b % T;
-  const int n = b / T;
-  const int wpad = W + 8;
-  // 21 input rows as independent float4 loads (W % 4 == 0): one L2 round trip per CTA instead of ~10 dependent scalar ones
-  const int w4 = W / 4;
-  if ((W & 3) != 0 || (reinterpret_cast<uintptr_t>(x) & 15) != 0) {       // odd widths: scalar gather
-    for (int i = threadIdx.x; i < 21 * wpad; i += blockDim.x) {
-      const int r = i / wpad, c = i % wpad;
-      const int ci = r / 7, kh = r % 7;
-      const int hi = 2 * ho + kh - 3, wi = c - 3;
-      float v = 0.f;
-      if (hi >= 0 && hi < H && wi >= 0 && wi < W)
-        v = __ldg(x + (((static_cast<long long>(n) * 3 + ci) * T + t) * H + hi) * W + wi);
-      rows[r][c] = v;
-    }
-  } else {
-  for (int i = threadIdx.x; i < 21 * w4; i += blockDim.x) {
-    const int r = i / w4, c4 = i - r * w4;
-    const int ci = r / 7, kh = r - ci * 7;
-    const int hi = 2 * ho + kh - 3;
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (hi >= 0 && hi < H)
-      v = __ldg(reinterpret_cast<const float4*>(x + (((static_cast<long long>(n) * 3 + ci) * T + t) * H + hi) * W) + c4);
-    float* d = &rows[r][3 + 4 * c4];
-    d[0] = v.x;
-    d[1] = v.y;
-    d[2] = v.z;
-    d[3] = v.w;
-  }
-  for (int i = threadIdx.x; i < 21 * 8; i += blockDim.x) {        // 3 zero columns left, 5 right
-    const int r = i >> 3, c = i & 7;
-    rows[r][c < 3 ? c : W + c] = 0.f;
-  }
-  }
-  __syncthreads();
-  // every thread keeps ONE vector column v (8 consecutive K columns): its 8 shared-memory offsets are computed once,
-  // the loop over the output positions of the row is 8 LDS + pack + one 16-byte store
-  const int nvec = ldk / 8;
-  const int v = threadIdx.x % nvec, wo0 = threadIdx.x / nvec, wstep = blockDim.x / nvec;
-  int offs[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const int k = v * 8 + j;
-    offs[j] = k < 147 ? (k / 7) * (kStemMaxW + 8) + (k % 7) : -1;        // rows[k / 7][2 * wo + k % 7]
-  }
-  const float* flat = &rows[0][0];
-  uint4* dst = reinterpret_cast<uint4*>(col) + ((static_cast<long long>(n) * T + t) * Ho + ho) * Wo * nvec;
-  if (wo0 < wstep) {
-    for (int wo = wo0; wo < Wo; wo += wstep) {
-      float f[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = offs[j] >= 0 ? flat[offs[j] + 2 * wo] : 0.f;
-      dst[wo * nvec + v] = pack8(f);
-    }
-  }
-}
-
 // ------------------------------------------------------------------------------------------- stem row packing
 // The 1x7x7 s(1,2,2) p(0,3,3) stem (r21d_byol.py:198) as a FOUR-tap stride-1 convolution over row pairs: the seven kw taps
 // and the three input channels of every output column are packed into a 32-channel vector, and the two frame rows
@@ -187,6 +117,7 @@ __global__ void __launch_bounds__(256) stem_im2col_kernel(const float* __restric
 // w[co][ci][0][kh = 2*j + hpar - 1][kw] (zero for kh = -1).  P holds 64 bytes per (frame row, output column): 0.77 GB per
 // batch of 60 against 1.93 GB for the materialised im2col rows (K = 147 -> 160) it replaces; K grows to 256, which the
 // tensor pipe does not notice on this HBM-bound layer.  One CTA per (n, t, h2): six input rows staged in shared memory.
+constexpr int kStemMaxW = 256;
 constexpr int kStemRowPairs = 4;     // row pairs per CTA: 24 input rows staged with float4 loads, 28 KB written per CTA
 __global__ void __launch_bounds__(256) stem_pack_kernel(const float* __restrict__ x, int T, int H, int W,
                                                         uint4* __restrict__ P) {
@@ -508,8 +439,8 @@ __device__ __forceinline__ void load8(const float* __restrict__ p, float (&f)[8]
 // out = act(raw*scale + shift + residual).  Two rows per trip with every load issued before the first use (one 16-byte
 // load in flight per thread and four CTAs per SM keep 16 KB per SM in the air: 4.7 TB/s; the HBM pipe wants ~3x that).
 // kCoef2: the residual carries its own BatchNorm coefficients (res_mode 2 / 3): 32 more registers, three CTAs per SM.
-template <bool kCoef2, int kRows>
-__global__ void __launch_bounds__(256, (kCoef2 || kRows > 2) ? 3 : 4) bn_apply_kernel(const uint4* __restrict__ raw, int Cp, long long rows_per_group,
+template <bool kCoef2>
+__global__ void __launch_bounds__(256, kCoef2 ? 3 : 4) bn_apply_kernel(const uint4* __restrict__ raw, int Cp, long long rows_per_group,
                                                           const float* __restrict__ scale, const float* __restrict__ shift,
                                                           int relu, int res_mode, const uint4* __restrict__ res,
                                                           const float* __restrict__ scale2, const float* __restrict__ shift2,
@@ -555,6 +486,7 @@ __global__ void __launch_bounds__(256, (kCoef2 || kRows > 2) ? 3 : 4) bn_apply_k
   const long long base = static_cast<long long>(t.g) * rows_per_group;
   const long long rstep = static_cast<long long>(gridDim.x) * t.rows_per_pass;
   long long r = static_cast<long long>(blockIdx.x) * t.rows_per_pass + t.rl;
+  constexpr int kRows = 2;       // (four rows per trip measured neutral, profiles/r02f_bn_rows_ab.txt)
   for (; r + (kRows - 1) * rstep < rows_per_group; r += kRows * rstep) {
     long long i[kRows];
     uint4 a[kRows], q[kRows];
@@ -616,7 +548,6 @@ __global__ void __launch_bounds__(kRedThreads) bn_bwd_finalize_kernel(const floa
 //   act != NULL            mask = act > 0            (block outputs: the pre-activation includes the residual)
 //   mscale != NULL         mask = raw*mscale + mshift > 0, the same fmaf the forward apply evaluated (saves the act read)
 //   neither                no ReLU behind this BatchNorm
-template <int kRows>
 __global__ void __launch_bounds__(256, 2) bn_bwd_apply_kernel(const uint4* __restrict__ d, const uint4* __restrict__ act,
                                                            const uint4* __restrict__ raw, int Cp, long long rows_per_group,
                                                            const float* __restrict__ mean, const float* __restrict__ invstd,
@@ -672,6 +603,7 @@ __global__ void __launch_bounds__(256, 2) bn_bwd_apply_kernel(const uint4* __res
   // kRows rows per trip with every load issued before the first use: 2 (3 with act) independent 16-byte loads per row.
   // Four rows (120 registers, two CTAs per SM: 64 KB in flight per SM) against two: 144-channel pass 5.5 -> 6.4 TB/s,
   // batch-60 step -0.4 ms (profiles/r02f_bn_rows_ab.txt)
+  constexpr int kRows = 4;
   for (; r + (kRows - 1) * rstep < rows_per_group; r += kRows * rstep) {
     long long i[kRows];
     uint4 vd[kRows], vx[kRows], vy[kRows];
@@ -768,7 +700,7 @@ static inline dim3 bn_grid(long long rows_per_group, int Cp, int groups) {
   const int segs = ceil_div(nvec, kSegVecs);
   const int seg_vecs = nvec < kSegVecs ? nvec : kSegVecs;
   const int rows_per_pass = 256 / seg_vecs;
-  long long want = (static_cast<long long>(num_sms()) * stream_ctas_per_sm() + groups * segs - 1) / (groups * segs);
+  long long want = (static_cast<long long>(num_sms()) * kStreamCtasPerSm + groups * segs - 1) / (groups * segs);
   long long have = (rows_per_group + rows_per_pass - 1) / rows_per_pass;
   if (want > have) want = have;
   if (want < 1) want = 1;
@@ -806,19 +738,6 @@ extern "C" int cstp_pack_weights_batched(const int64_t* jobs_dev, const int64_t*
   static_assert(sizeof(long long) == sizeof(int64_t), "job table is int64");
   pack_weights_batched_kernel<<<grid_for((total + 15) / 16, 256), 256, 0, ST(stream)>>>(
       reinterpret_cast<const long long*>(jobs_dev), reinterpret_cast<const long long*>(prefix_dev), n_jobs, total);
-  CSTP_LAUNCHED();
-  return CSTP_OK;
-}
-
-extern "C" int cstp_stem_im2col(const float* x, int N, int T, int H, int W, void* col, int ldk, void* stream) {
-  CSTP_REQUIRE(x && col && N > 0 && T > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0);
-  CSTP_REQUIRE(ldk >= 152 && ldk % 8 == 0 && W <= kStemMaxW);
-  const long long blocks = static_cast<long long>(N) * T * (H / 2);
-  CSTP_REQUIRE(blocks < (1LL << 31));
-  const int nvec = ldk / 8;
-  const int threads = (256 / nvec) * nvec >= 64 ? (256 / nvec) * nvec : 256;   // a whole number of vector columns
-  stem_im2col_kernel<<<static_cast<unsigned>(blocks), threads, 0, ST(stream)>>>(x, N, T, H, W,
-                                                                           reinterpret_cast<__nv_bfloat16*>(col), ldk);
   CSTP_LAUNCHED();
   return CSTP_OK;
 }
@@ -867,7 +786,7 @@ extern "C" int cstp_bn_apply(const void* raw, int64_t rows, int Cp, int groups, 
   CSTP_REQUIRE(raw && out && scale && shift && rows > 0 && groups > 0 && rows % groups == 0 && Cp % 16 == 0);
   CSTP_REQUIRE(res_mode >= 0 && res_mode <= 3 && (res_mode == 0 || res != nullptr));
   CSTP_REQUIRE(res_mode < 2 || (scale2 && shift2));
-  auto kernel = res_mode >= 2 ? bn_apply_kernel<true, 2> : (bn_apply_rows() == 4 ? bn_apply_kernel<false, 4> : bn_apply_kernel<false, 2>);
+  auto kernel = res_mode >= 2 ? bn_apply_kernel<true> : bn_apply_kernel<false>;
   kernel<<<bn_grid(rows / groups, Cp, groups), 256, 0, ST(stream)>>>(
       reinterpret_cast<const uint4*>(raw), Cp, rows / groups, scale, shift, relu, res_mode,
       reinterpret_cast<const uint4*>(res), scale2, shift2, reinterpret_cast<uint4*>(out));
@@ -907,8 +826,7 @@ extern "C" int cstp_bn_bwd_apply(const void* d, const void* act, const void* raw
   CSTP_REQUIRE((mask_scale == nullptr) == (mask_shift == nullptr));
   CSTP_REQUIRE(act == nullptr || mask_scale == nullptr);
   // (64 registers / 4 CTAs per SM was measured: it spills and is 7 % slower than 80 registers / 3 CTAs)
-  auto kernel = bn_bwd_rows() == 4 ? bn_bwd_apply_kernel<4> : bn_bwd_apply_kernel<2>;
-  kernel<<<bn_grid(rows / groups, Cp, groups), 256, 0, ST(stream)>>>(
+  bn_bwd_apply_kernel<<<bn_grid(rows / groups, Cp, groups), 256, 0, ST(stream)>>>(
       reinterpret_cast<const uint4*>(d), reinterpret_cast<const uint4*>(act), reinterpret_cast<const uint4*>(raw), Cp,
       rows / groups, mean, invstd, coef, mask_scale, mask_shift, reinterpret_cast<uint4*>(g),
       reinterpret_cast<uint4*>(dz));

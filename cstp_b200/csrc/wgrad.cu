@@ -362,7 +362,7 @@ extern "C" int cstp_wgrad_plan_create(const cstp_wgrad_desc* d, cstp_wgrad_plan*
   const uint32_t stage_bytes = (2u * static_cast<uint32_t>(n_mt) + static_cast<uint32_t>(k.n_gboxes)) * kBoxBytes;
   const int bar_bytes = 256;
   const int xtab_bytes = xform ? static_cast<int>(xform_table_bytes(d->pro.groups, d->pro.Cp)) : 0;      // prologue coefficient table
-  int stages = (smem_budget() - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(stage_bytes);
+  int stages = (kSmemBudget - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(stage_bytes);
   if (stages > kWgMaxStages) stages = kWgMaxStages;
   if (stages < 2) {
     delete plan;

@@ -53,7 +53,6 @@ struct WgradHaloKParams {
   int n_xboxes, n_mtiles, n_chunks, Np, n_tile, n_gboxes;
   int total_kblocks;
   int n_ntiles, mt_per_class, n_mclasses, pro_on_b;
-  int dbg;                 // development probes (CSTP_WG_DBG): 1 = transform warps skip the arithmetic, 2 = skip the proxy fence
   int class_splits[kWhMaxClasses], class_kps[kWhMaxClasses];   // split-K CTAs and K-blocks per CTA of every M class
   int stages, tmem_cols;
   uint32_t xbox_bytes, stage_bytes, idesc;
@@ -135,7 +134,7 @@ __global__ void __launch_bounds__(kXform ? kWhThreads + kWhXformThreads : kWhThr
     const int cj = xform_unit_channel(smem_addr0 + tid * 16u, 7u);
     // Up to three boxes of at most two units per thread (the N-side boxes of the flipped form): the coefficients of the
     // thread's vector in every box stay in registers (reloaded when the statistics group changes, once per launch) and the
-    // loads of a box are issued before the previous box is finished.  Measured (tools/prologue_probe.py, CSTP_WG_DBG): the
+    // loads of a box are issued before the previous box is finished.  Measured (tools/prologue_probe.py): the
     // cost of the prologue is the arithmetic of the transform warps (ALU pipe), not the proxy fence or the second barrier
     // hop; sixteen warps instead of eight made it worse.
     const bool small = n_boxes <= 3 && box_units <= 2u * kWhXformThreads;
@@ -144,7 +143,7 @@ __global__ void __launch_bounds__(kXform ? kWhThreads + kWhXformThreads : kWhThr
     // N-side boxes on an exact tiling are never out of range and the MMA never reads channels beyond n_tile: the cheaper
     // ReLU-in-the-conversion form applies (its NaN stays NaN)
     const bool exact = on_b && p.tiles_w * p.bw == p.Wt && p.tiles_h * p.bh == p.Ht && p.tiles_t * p.bt == p.Tt &&
-                       p.tiles_n * p.bn == p.Nt && !(p.dbg & 4);
+                       p.tiles_n * p.bn == p.Nt;
     XformCoef kc[3];
     int cur_grp = -1;
     int stage = 0;
@@ -154,9 +153,7 @@ __global__ void __launch_bounds__(kXform ? kWhThreads + kWhXformThreads : kWhThr
     for (int kb = kb_begin; kb < kb_end; ++kb) {
       const int grp = kb >= kb_grp1 ? 1 : 0;
       const uint32_t s_addr = smem_addr0 + static_cast<uint32_t>(stage) * p.stage_bytes + box0;
-      if (p.dbg & 1) {
-        mbar_wait(&full[stage], phase);
-      } else if (small) {
+      if (small) {
         if (grp != cur_grp) {
           cur_grp = grp;
 #pragma unroll
@@ -204,7 +201,7 @@ __global__ void __launch_bounds__(kXform ? kWhThreads + kWhXformThreads : kWhThr
             const WhXBox xb = p.xboxes[b];
             const int bw0 = w0 + xb.dw, bh0 = h0 + xb.dh, bt0 = t0 + xb.dt;
             inside = bw0 >= 0 && bw0 + p.box_w <= p.a_w && bh0 >= 0 && bh0 + p.box_h <= p.a_h && bt0 >= 0 &&
-                     bt0 + p.box_t <= p.a_t && xb.c_off + 64 <= p.pro_cp && !(p.dbg & 4);
+                     bt0 + p.box_t <= p.a_t && xb.c_off + 64 <= p.pro_cp;
           }
           if (inside)
             xform_span<kWhXformThreads, true>(s_addr + static_cast<uint32_t>(b) * box_pitch, tid, box_units, k);
@@ -213,7 +210,7 @@ __global__ void __launch_bounds__(kXform ? kWhThreads + kWhXformThreads : kWhThr
           if (b + 1 < n_boxes) xform_load_smem(k, xtab_addr, tchunks, grp, on_b ? chunk0 + b + 1 : p.xboxes[b + 1].c_off >> 6, cj);
         }
       }
-      if (!(p.dbg & 2)) fence_proxy_async();
+      fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(&xfull[stage]);
       if (++stage == stages) {
@@ -411,10 +408,6 @@ extern "C" int cstp_wgrad_halo_plan_create(const cstp_wgrad_halo_desc* d, cstp_w
   k.mt_per_class = mt_per_class;
   k.n_mclasses = n_mclasses;
   k.pro_on_b = xform && d->pro_on_b;
-  {
-    const char* e = getenv("CSTP_WG_DBG");
-    k.dbg = e ? atoi(e) : 0;
-  }
   // d->splits split-K CTAs per N tile, dealt to the M classes in proportion to their M tiles (at least one each)
   int max_splits = 0, left = d->splits, tiles_left = n_mtiles;
   for (int c = 0; c < n_mclasses; ++c) {
@@ -468,7 +461,7 @@ extern "C" int cstp_wgrad_halo_plan_create(const cstp_wgrad_halo_desc* d, cstp_w
   }
   const int bar_bytes = 256;
   const int xtab_bytes = xform ? static_cast<int>(xform_table_bytes(d->pro.groups, d->pro.Cp)) : 0;      // prologue coefficient table
-  int stages = (smem_budget() - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(k.stage_bytes);
+  int stages = (kSmemBudget - 1024 - bar_bytes - xtab_bytes) / static_cast<int>(k.stage_bytes);
   if (stages > kWhMaxStages) stages = kWhMaxStages;
   if (stages < 2) {
     delete plan;

@@ -9,7 +9,6 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-import os
 from dataclasses import dataclass, field
 from itertools import product
 
@@ -264,17 +263,16 @@ class ConvHaloPlan(_Plan):
         L.check(L.load().cstp_conv_halo_plan_run(self.handle, _stream()))
 
 
-# same knob as csrc/common.cu::smem_budget()
-SMEM_LIMIT = min(227, max(64, int(os.environ.get("CSTP_SMEM_KB") or 227))) * 1024
+# same budget as csrc/common.h kSmemBudget
+SMEM_LIMIT = 227 * 1024
 SMEM_BUDGET = SMEM_LIMIT - 1024 - 256
 
 
 def conv_halo_layout(tile_space, taps, a_channels: int, Np: int):
     """The 2-D halo layout when it applies and keeps the full-width weights resident, else the one-axis halo layout."""
-    if USE_HALO_2D:
-        lay = _conv_halo_layout(tile_space, taps, a_channels, Np, True)
-        if lay is not None and lay["pitch"] != 8 and lay["resident"] and lay["n_tile"] == min(Np, 256):
-            return lay
+    lay = _conv_halo_layout(tile_space, taps, a_channels, Np, True)
+    if lay is not None and lay["pitch"] != 8 and lay["resident"] and lay["n_tile"] == min(Np, 256):
+        return lay
     return _conv_halo_layout(tile_space, taps, a_channels, Np, False)
 
 
@@ -342,7 +340,7 @@ def _conv_halo_layout(tile_space, taps, a_channels: int, Np: int, halo_2d: bool)
     a_bytes = (rows * 128 + 1023) // 1024 * 1024          # stage pitch (csrc/conv_halo.cu a_stride)
     chunks = pad64(a_channels) // 64
     # a channel tail of exactly 16 / 32 beyond a multiple of 64 is staged with 32 / 64-byte rows (csrc/conv_halo.cu)
-    tail = a_channels % 64 if (USE_TAIL_BOXES and a_channels > 64 and a_channels % 64 in (16, 32)) else 0
+    tail = a_channels % 64 if (a_channels > 64 and a_channels % 64 in (16, 32)) else 0
     k_bytes_per_row = ((chunks - 1) * 128 + tail * 2) if tail else chunks * 128      # resident weight bytes per (tap, n)
     # N tile: keep all weight K-blocks resident when they fit beside 3 activation stages, splitting N in two if needed
     n_tile, resident = (Np if Np <= 256 else _default_n_tile(Np)), False
@@ -357,15 +355,6 @@ def _conv_halo_layout(tile_space, taps, a_channels: int, Np: int, halo_2d: bool)
             return None
     return dict(box=box, halo=halo, groups=groups, taps=out_taps, n_tile=n_tile, a_bytes=a_bytes, resident=resident,
                 tail=tail, pitch=pitch)
-
-
-USE_SLABS = os.environ.get("CSTP_SLABS", "1") == "1"
-SLAB_G = int(os.environ.get("CSTP_SLAB_G", "4"))
-# slab mode for the forward 64-column layers (conv1.temporal, conv2.*.temporal) as well: built and tested (prologue + fused
-# statistics run in slab mode), but OFF by default -- behind the operand prologue those launches are bound by the staging
-# pipeline, not by the MMA issue rate, and slab mode stages 6 input frames per 4 output frames instead of 18 per 16
-# (measured at batch 60: 0.82 - 0.86 ms against 0.775 ms per launch)
-SLABS_FWD = os.environ.get("CSTP_SLABS_FWD", "0") == "1"
 
 
 def slab_tables(G: int, nslots: int, Np: int):
@@ -387,58 +376,44 @@ def slab_tables(G: int, nslots: int, Np: int):
     return out
 
 
-def conv_slab_layout(tile_space, taps, a_channels: int, Np: int, G: int | None = None, n_div: int = 0):
-    """Slab-mode geometry of csrc/conv_halo.cu (include/cstp_b200.h cstp_halo_slabs) for a stride-1 tap list
-    [(dw, dh, dt, k_off)] of a layer with Np == 64 output columns, or None.  1 x k x k taps: G output rows per tile (slab
-    axis h), every input row staged as ONE box with a halo along w (the w taps are row shifts of it); k x 1 x 1 taps: G
-    output frames per tile (slab axis t), plain boxes.  Same dict as conv_halo_layout plus `slabs` = (G, axis, nslots);
-    taps are listed w tap by w tap, the taps along the slab axis in DEscending offset order."""
+def conv_slab_layout(tile_space, taps, a_channels: int, Np: int, G: int = 4):
+    """Slab-mode geometry of csrc/conv_halo.cu (include/cstp_b200.h cstp_halo_slabs) for a stride-1 1 x k x k tap list
+    [(dw, dh, dt, k_off)] of a layer with Np == 64 output columns, or None: G output rows per tile (slab axis h), every
+    input row staged as ONE box with a halo along w (the w taps are row shifts of it).  Same dict as conv_halo_layout plus
+    `slabs` = (G, 1, nslots); taps are listed w tap by w tap, the h taps in DEscending offset order."""
     Wt, Ht, Tt, Nt = tile_space
-    G = G or SLAB_G
-    if not USE_SLABS or Np != 64 or G < 2 or G * Np > 256 or len(taps) < 2 or len(taps) > 16:
+    if Np != 64 or G < 2 or G * Np > 256 or len(taps) < 2 or len(taps) > 16:
         return None
     dws, dhs, dts = sorted({t[0] for t in taps}), sorted({t[1] for t in taps}), sorted({t[2] for t in taps})
     consecutive = lambda v: v == list(range(v[0], v[-1] + 1))      # noqa: E731
-    if len(dts) == 1 and len(dhs) > 1 and consecutive(dws) and consecutive(dhs) and len(taps) == len(dws) * len(dhs):
-        axis, along, wspan, extent = 1, dhs, dws[-1] - dws[0], Ht
-    elif len(dws) == 1 and len(dhs) == 1 and len(dts) > 1 and consecutive(dts) and dws[0] == 0 and dhs[0] == 0:
-        axis, along, wspan, extent = 2, dts, 0, Tt
-    else:
+    if not (len(dts) == 1 and len(dhs) > 1 and consecutive(dws) and consecutive(dhs) and len(taps) == len(dws) * len(dhs)):
         return None
-    nslots = len(along)
-    if nslots > 4 or nslots * Np > 256 or extent < G:
+    wspan = dws[-1] - dws[0]
+    nslots = len(dhs)
+    if nslots > 4 or nslots * Np > 256 or Ht < G:
         return None
-    # 128 positions with extent 1 along the slab axis, 8 along w (one swizzle atom per run when the box has a w halo)
+    # 128 positions with extent 1 along h, 8 along w (one swizzle atom per run when the box has a w halo)
     best = None
-    for b1 in (16, 8, 4, 2, 1):                  # extent along the other spatial / temporal axis, the rest along n
-        bn = 16 // b1
-        if n_div and n_div % bn:                 # the samples of a tile must share one BatchNorm statistics group
-            continue
-        other = Tt if axis == 1 else Ht
-        key = (math.ceil(other / b1) * math.ceil(Nt / bn), bn)
+    for bt in (16, 8, 4, 2, 1):                  # extent along t, the rest along n
+        bn = 16 // bt
+        key = (math.ceil(Tt / bt) * math.ceil(Nt / bn), bn)
         if best is None or key < best[0]:
-            best = (key, b1, bn)
-    if best is None:
-        return None
-    _, b1, bn = best
-    box = (8, 1, b1, bn) if axis == 1 else (8, b1, 1, bn)
-    rows = (8 + wspan) * b1 * bn
+            best = (key, bt, bn)
+    _, bt, bn = best
+    box = (8, 1, bt, bn)
+    rows = (8 + wspan) * bt * bn
     pitch = 8 + wspan if wspan else 8
     a_bytes = (rows * 128 + 1023) // 1024 * 1024
     chunks = pad64(a_channels) // 64
-    tail = a_channels % 64 if (USE_TAIL_BOXES and a_channels > 64 and a_channels % 64 in (16, 32)) else 0
+    tail = a_channels % 64 if (a_channels > 64 and a_channels % 64 in (16, 32)) else 0
     k_bytes_per_row = ((chunks - 1) * 128 + tail * 2) if tail else chunks * 128
     if len(taps) * k_bytes_per_row * Np + 2 * a_bytes > SMEM_BUDGET:
         return None
     by_off = {(t[0], t[1], t[2]): t[3] for t in taps}
-    out_taps = []
-    for dw in dws:
-        for da in reversed(along):
-            key = (dw, da, dts[0]) if axis == 1 else (dw, dhs[0], da)
-            out_taps.append(((dw - dws[0]) * 128, by_off[key]))
+    out_taps = [((dw - dws[0]) * 128, by_off[(dw, dh, dts[0])]) for dw in dws for dh in reversed(dhs)]
     groups = [(dws[0], dhs[0], dts[0], 0, len(taps))]
     return dict(box=box, halo=(wspan, 0, 0), groups=groups, taps=out_taps, n_tile=G * Np, a_bytes=a_bytes, resident=True,
-                tail=tail, pitch=pitch, slabs=(G, axis, nslots))
+                tail=tail, pitch=pitch, slabs=(G, 1, nslots))
 
 
 def _make_conv_halo_plan(view, lay, a_channels, w_packed, Np, tile_space, out, out_f32, out_off, ostrides, bias,
@@ -476,7 +451,6 @@ def _make_conv_halo_plan(view, lay, a_channels, w_packed, Np, tile_space, out, o
     L.check(lib.cstp_conv_halo_plan_create(C.byref(d), C.byref(h)))
     plan = ConvHaloPlan(h, lib.cstp_conv_halo_plan_destroy, keep + ((stats.partials,) if stats is not None else ()))
     plan.resident = bool(lib.cstp_conv_halo_plan_resident(h))
-    plan.slab = bool(lay.get("slabs"))
     if stats is not None:
         plan.stat_blocks = lib.cstp_conv_halo_plan_stat_blocks(h)
         if plan.stat_blocks * stats.groups * 2 * stats.Cp > stats.partials.numel():
@@ -484,17 +458,6 @@ def _make_conv_halo_plan(view, lay, a_channels, w_packed, Np, tile_space, out, o
     return plan
 
 
-# BatchNorm statistics fused into the halo-conv epilogue (csrc/conv_halo.cu): only for single 64-column N tiles, where every
-# epilogue thread can keep the running sum / sum of squares of its row's 64 columns in registers (no shuffles per tile).
-# The first attempt (shuffle butterfly per 16-column chunk, all tile widths) removed 2.3 ms of bn_reduce passes at batch 60
-# but cost 3-5 ms in the conv kernels and was taken out (profiles/README.md).
-FUSE_BN_STATS = os.environ.get("CSTP_FUSE_BN_STATS", "1") == "1"
-DGRAD_ONE_LAUNCH = os.environ.get("CSTP_DGRAD_ONE_LAUNCH", "1") == "1"
-# (measured at batch 60: conv3.block1.conv1.spatial dgrad 0.89 ms as one conv_gemm launch, 0.99 ms with its 2- and 4-tap
-# classes on the halo kernel -- kept as a knob, off)
-DGRAD_STRIDED_HALO = os.environ.get("CSTP_DGRAD_STRIDED_HALO", "0") == "1"
-USE_TAIL_BOXES = os.environ.get("CSTP_TAIL_BOXES", "1") == "1"
-USE_HALO_2D = os.environ.get("CSTP_HALO_2D", "1") == "1"
 HALO_MIN_POSITIONS = 28 * 28      # per (t, n) slab: smaller extents cannot fill 128-row single-slab tiles
 
 
@@ -518,19 +481,13 @@ def conv_fwd_plan(x, w_packed, out, geom: ConvGeom, *, out_f32=None, bias=None, 
     taps = [(m, dw, dh, dt, ti * Kc) for (m, dw, dh, dt, ti) in taps]
     ostr = (Np, Wo * Np, Ho * Wo * Np, To * Ho * Wo * Np)
     if allow_halo and box is None and n_tile is None and len(views) == 1 and Ho * Wo >= HALO_MIN_POSITIONS:
-        if SLABS_FWD and out is not None and out_f32 is None and bias is None:
-            # 64-column layers (conv1.temporal, conv2.*.temporal): G output frames per tile on the accumulator's N axis
-            groups = stats.groups if stats is not None else (prologue.groups if prologue is not None else 1)
-            lay = conv_slab_layout((Wo, Ho, To, N), [t[1:] for t in taps], Ca, Np, n_div=N // groups) if N % groups == 0 else None
-            if lay is not None:
-                fuse = FUSE_BN_STATS and stats is not None and stats.groups in (1, 2) and not accumulate
-                if fuse or prologue is None:        # (the kernel has no prologue-without-statistics slab instantiation)
-                    return _make_conv_halo_plan(views[0], lay, Ca, w_packed, Np, (Wo, Ho, To, N), out, None, 0, ostr, None,
-                                                accumulate, (x, w_packed, out), stats=stats if fuse else None,
-                                                prologue=prologue)
         lay = conv_halo_layout((Wo, Ho, To, N), [t[1:] for t in taps], Ca, Np)
         if lay is not None:
-            fuse = (FUSE_BN_STATS and stats is not None and stats.groups in (1, 2) and N % stats.groups == 0
+            # BatchNorm statistics fused into the epilogue: only for single 64-column N tiles, where every epilogue thread
+            # can keep the running sum / sum of squares of its row's 64 columns in registers (no shuffles per tile).  The
+            # first attempt (shuffle butterfly per 16-column chunk, all tile widths) removed 2.3 ms of bn_reduce passes at
+            # batch 60 but cost 3-5 ms in the conv kernels and was taken out (profiles/README.md).
+            fuse = (stats is not None and stats.groups in (1, 2) and N % stats.groups == 0
                     and out is not None and out_f32 is None and bias is None and not accumulate
                     and Np == 64 and lay["n_tile"] == 64 and lay["box"][3] == 1)
             return _make_conv_halo_plan(views[0], lay, Ca, w_packed, Np, (Wo, Ho, To, N), out, out_f32, 0, ostr, bias,
@@ -559,13 +516,11 @@ def conv_dgrad_plans(g, wt_packed, dx, geom: ConvGeom, *, accumulate=False, allo
     rest = []
     for cl in live:
         taps = [(0, dw_, dh_, dt_, ti * Kc) for (dw_, dh_, dt_, ti) in cl["taps"]]
-        # every class is a stride-1 convolution over g with its own taps and a strided output: the halo kernel applies to
-        # the classes whose taps form a 1-D / 2-D neighbourhood (stride-2 1x3x3: the 2- and 4-tap classes)
-        if allow_halo and cl["space"][0] * cl["space"][1] >= HALO_MIN_POSITIONS and (
-                tuple(geom.stride) == (1, 1, 1) or DGRAD_STRIDED_HALO):
-            lay = None
-            if tuple(geom.stride) == (1, 1, 1):
-                lay = conv_slab_layout(cl["space"], [t[1:] for t in taps], Co, Ci)
+        # the halo kernel takes the dgrad of stride-1 convolutions only: the stride-parity classes of a strided one run on
+        # conv_gemm (measured at batch 60: conv3.block1.conv1.spatial dgrad 0.89 ms as one conv_gemm launch, 0.99 ms with
+        # its 2- and 4-tap classes on the halo kernel)
+        if allow_halo and tuple(geom.stride) == (1, 1, 1) and cl["space"][0] * cl["space"][1] >= HALO_MIN_POSITIONS:
+            lay = conv_slab_layout(cl["space"], [t[1:] for t in taps], Co, Ci)
             if lay is None:
                 lay = conv_halo_layout(cl["space"], [t[1:] for t in taps], Co, Ci)
             if lay is not None:
@@ -573,7 +528,7 @@ def conv_dgrad_plans(g, wt_packed, dx, geom: ConvGeom, *, accumulate=False, allo
                                                   cl["ostrides"], None, accumulate, (g, wt_packed, dx)))
                 continue
         rest.append((cl, taps))
-    if (DGRAD_ONE_LAUNCH and 1 < len(rest) <= 8
+    if (1 < len(rest) <= 8
             and all(cl["space"] == rest[0][0]["space"] and cl["ostrides"] == rest[0][0]["ostrides"] for cl, _ in rest)
             and sum(len(t) for _, t in rest) <= L.CSTP_MAX_TAPS):
         # stride-parity classes that share their tile space (even extents): ONE launch, class-minor tile order -- the
@@ -635,10 +590,6 @@ class WgradHaloPlan(_Plan):
         L.check(L.load().cstp_wgrad_halo_plan_run(self.handle, _stream()))
 
 
-WGRAD_TRANSPOSE = os.environ.get("CSTP_WGRAD_TRANSPOSE", "1") == "1"
-WGRAD_MCLASSES = os.environ.get("CSTP_WGRAD_MCLASSES", "1") == "1"
-
-
 def _wgrad_halo_side(m_channels: int, n_channels: int, dims, geom: ConvGeom, flip: bool, sms: int, xform: bool = False):
     """One orientation of the all-taps-per-CTA weight-gradient kernel: the operand with `m_channels` carries the taps (staged
     with a halo, M = (tap, 64-channel chunk)), the other one (`n_channels`, N axis) is staged as plain boxes.  flip: the M
@@ -652,23 +603,17 @@ def _wgrad_halo_side(m_channels: int, n_channels: int, dims, geom: ConvGeom, fli
         return None
     n_mtiles = (n_chunks + 1) // 2
     Np = n_channels
-    if WGRAD_MCLASSES:
-        # full-width N tiles (every MMA as wide as the layer allows); the M tiles are dealt to CTA classes that fit TMEM
-        n_ntiles = math.ceil(Np / 256)
-        n_tile = pad16(math.ceil(Np / n_ntiles))
-        if flip and xform and n_ntiles > 1:      # the prologue on the N-side boxes wants N-tile origins on 64-channel chunks
-            n_tile = pad64(n_tile)
-            n_ntiles = math.ceil(Np / n_tile)
-        mt_per_class = min(n_mtiles, 512 // n_tile)
-        n_mclasses = math.ceil(n_mtiles / mt_per_class)
-        mt_per_class = math.ceil(n_mtiles / n_mclasses)          # balanced classes (5 tiles, cap 3 -> 3 + 2)
-        if n_mclasses > 8:
-            return None
-    else:
-        n_tile = min(Np, 256, (512 // n_mtiles) // 16 * 16)
-        if n_tile < 16 or (flip and xform and n_tile < Np and n_tile % 64):
-            return None
-        n_ntiles, mt_per_class, n_mclasses = math.ceil(Np / n_tile), n_mtiles, 1
+    # full-width N tiles (every MMA as wide as the layer allows); the M tiles are dealt to CTA classes that fit TMEM
+    n_ntiles = math.ceil(Np / 256)
+    n_tile = pad16(math.ceil(Np / n_ntiles))
+    if flip and xform and n_ntiles > 1:      # the prologue on the N-side boxes wants N-tile origins on 64-channel chunks
+        n_tile = pad64(n_tile)
+        n_ntiles = math.ceil(Np / n_tile)
+    mt_per_class = min(n_mtiles, 512 // n_tile)
+    n_mclasses = math.ceil(n_mtiles / mt_per_class)
+    mt_per_class = math.ceil(n_mtiles / n_mclasses)          # balanced classes (5 tiles, cap 3 -> 3 + 2)
+    if n_mclasses > 8:
+        return None
     temporal = kt > 1
     # tap a reads the M-side operand at offset (a - pad) from the K-block origin -- or, flipped, at -(a - pad)
     off = (lambda a, k, p_: (k - 1 - a) if flip else a)
@@ -676,7 +621,7 @@ def _wgrad_halo_side(m_channels: int, n_channels: int, dims, geom: ConvGeom, fli
     # 1 x k x k filters, 2-D halo: ONE staged (8 + kw - 1) x (8 + kh - 1) box per 64-channel chunk serves every tap (a tap
     # is a whole-row shift of it; the 8 positions of a w run are one swizzle atom, atoms one box row apart).  The box is
     # then cheap enough to be re-staged by several CTA classes.
-    halo_2d = (USE_HALO_2D and not temporal and kw > 1 and kh > 1 and n_ntiles * n_mclasses <= 6
+    halo_2d = (not temporal and kw > 1 and kh > 1 and n_ntiles * n_mclasses <= 6
                and math.ceil(Wo / 8) * math.ceil(Ho / 8) * 64 <= 1.35 * Wo * Ho)
     if n_ntiles * n_mclasses > 2 and not halo_2d:          # the M-side boxes are re-staged once per class
         return None
@@ -755,7 +700,7 @@ def wgrad_halo_layout(x_shape, g_shape, geom: ConvGeom, sms: int = 148, xform: b
     N, T, H, W, Ca = x_shape
     _, To, Ho, Wo, Np = g_shape
     lay = _wgrad_halo_side(Ca, Np, (N, To, Ho, Wo), geom, False, sms, xform)
-    if WGRAD_TRANSPOSE and (T, H, W) == (To, Ho, Wo) and geom.pad_hi is None:
+    if (T, H, W) == (To, Ho, Wo) and geom.pad_hi is None:
         alt = _wgrad_halo_side(Np, Ca, (N, To, Ho, Wo), geom, True, sms, xform)
         if alt is not None and (lay is None or alt["cost"] < lay["cost"]):
             lay = alt
@@ -775,9 +720,6 @@ def wgrad_partials_need(x_shape, g_shape, geom: ConvGeom, sms: int = 148) -> int
     return max(_wgrad_gemm_shape(nch, Np, kblocks, sms, xf)[2] for xf in (False, True)) * nch * 64 * Np
 
 
-WGRAD_MT = int(os.environ.get("CSTP_WGRAD_MT", "4"))      # upper bound of M tiles per CTA in csrc/wgrad.cu (1: round-1 shape)
-
-
 def _wgrad_gemm_shape(nch: int, Np: int, kblocks: int, sms: int = 148, xform: bool = False) -> tuple[int, int, int]:
     """(n_tile, mt_per_cta, splits) of csrc/wgrad.cu for `nch` 64-row M chunks, Np columns and `kblocks` 64-position K-blocks.
     The kernel is bound by the L2 -> SM feed: a CTA stages 2 * mt X boxes and n_tile / 64 G boxes of 8 KB per K-block, so
@@ -787,17 +729,13 @@ def _wgrad_gemm_shape(nch: int, Np: int, kblocks: int, sms: int = 148, xform: bo
         share one staged G tile (the prologue variant takes one: its transform keeps the coefficients of two boxes in
         registers);
       * the split-K factor minimises waves x K-blocks per split + the cost of writing and re-reading one more partial."""
-    if WGRAD_MT <= 1:
-        n_tile = Np if Np <= 256 else 256
-        base = math.ceil(nch / 2) * math.ceil(Np / n_tile)
-        return n_tile, 1, max(1, min(math.ceil(2 * sms / base), max(1, kblocks // 4)))
     if Np <= 256:
         n_tile = Np
     else:
         n_tile = min((256, 192, 128), key=lambda c: (math.ceil(Np / c), math.ceil(Np / c) * c, -c))
     ngb = math.ceil(n_tile / 64)
     mt = 1
-    for m in range(2, min(WGRAD_MT, 4) + 1):
+    for m in range(2, 5):                                        # csrc/wgrad.cu takes up to four M tiles per CTA
         if m * n_tile <= 512 and 3 * (2 * m + ngb) * 8192 <= SMEM_BUDGET and m <= math.ceil(nch / 2):
             mt = m
     # (the split-K factor is the plain kernel's also behind the prologue, which runs one M tile per CTA: the same K ranges
@@ -968,14 +906,7 @@ def stem_pack(x: torch.Tensor, P: torch.Tensor) -> None:
     L.check(L.load().cstp_stem_pack(_ptr(x), N, T, H, W, _ptr(P), _stream()))
 
 
-def stem_im2col(x: torch.Tensor, col: torch.Tensor) -> None:
-    _require_cuda(x, col)
-    N, Cc, T, H, W = x.shape
-    assert Cc == 3 and x.dtype == torch.float32 and x.is_contiguous()
-    L.check(L.load().cstp_stem_im2col(_ptr(x), N, T, H, W, _ptr(col), col.shape[-1], _stream()))
-
-
-BN_REDUCE_CTAS_PER_SM = max(1, int(os.environ.get("CSTP_BN_REDUCE_CTAS_PER_SM") or 2))   # per statistics group
+BN_REDUCE_CTAS_PER_SM = 2         # per statistics group (co-residency sweep: profiles/r01_overlap_sweep.txt)
 
 
 def bn_nblocks(rows_per_group: int, Cp: int, sms: int = 148) -> int:

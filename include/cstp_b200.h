@@ -104,7 +104,7 @@ typedef struct cstp_conv_plan cstp_conv_plan;
 int cstp_conv_plan_create(const cstp_conv_desc* desc, cstp_conv_plan** plan);
 int cstp_conv_plan_run(const cstp_conv_plan* plan, void* stream);
 /* CTAs per thread-block cluster the plan launches with: 1, or 2 (CTA pairs, each weight tile multicast into both shared
- * memories; chosen when the persistent grid is full and CSTP_CONV_CLUSTER != 0). */
+ * memories; chosen when the persistent grid is full). */
 int cstp_conv_plan_cluster(const cstp_conv_plan* plan);
 void cstp_conv_plan_destroy(cstp_conv_plan* plan);
 
@@ -122,16 +122,16 @@ typedef struct {
   int32_t k_off;
 } cstp_halo_tap;
 
-/* "Slab mode" for layers with few output channels (Np <= 64): n_slabs = G > 1 consecutive output slabs along `axis`
- * (1: h, 2: t) share one accumulator of n_tile = G * Np columns.  Every input slab of the tile (G + nslots - 1 of them, the
- * first at the origin groups[0]) is staged once and multiplied, per w tap, with the stacked weight blocks of the output
- * slabs it feeds: a 128 x 64 x 16 tcgen05.mma is bound by the shared-memory read of its A slice, an MMA of 2 - 3 x 64
- * columns is not.  taps[] then lists, w tap by w tap, the nslots taps along `axis` in DEscending offset order; the tile
- * covers bw*bh*bt*bn == 128 positions with extent 1 along `axis`.  Needs resident weights, a plain bf16 output, no
- * prologue / statistics. */
+/* "Slab mode" for layers with few output channels (Np <= 64): n_slabs = G > 1 consecutive output slabs along h
+ * (`axis` must be 1) share one accumulator of n_tile = G * Np columns.  Every input slab of the tile (G + nslots - 1 of
+ * them, the first at the origin groups[0]) is staged once and multiplied, per w tap, with the stacked weight blocks of the
+ * output slabs it feeds: a 128 x 64 x 16 tcgen05.mma is bound by the shared-memory read of its A slice, an MMA of 2 - 3 x 64
+ * columns is not.  taps[] then lists, w tap by w tap, the nslots taps along h in DEscending offset order; the tile covers
+ * bw*bh*bt*bn == 128 positions with bh == 1.  Needs resident weights, a plain bf16 output, no prologue, no fused
+ * statistics. */
 typedef struct {
   int32_t n_slabs;              /* 0 / 1: off */
-  int32_t axis;
+  int32_t axis;                 /* 1 (h) */
   int32_t nslots;
 } cstp_halo_slabs;
 
@@ -289,9 +289,6 @@ int cstp_pack_weights_batched(const int64_t* jobs_dev, const int64_t* prefix_dev
  * implicit GEMM over P (row pairs ho-2 .. ho+1) whose packed weights come from cstp_pack_weight(s) with transpose = 2
  * and whose weight gradient is scattered by cstp_wgrad_finalize layout 1. */
 int cstp_stem_pack(const float* x, int N, int T, int H, int W, void* P, void* stream);
-/* Stem (older form, kept for callers that want the GEMM view): fp32 NCDHW clip (N,3,T,H,W) -> bf16 im2col rows [N*T*Ho*Wo][ldk] for the 1x7x7 s(1,2,2) p(0,3,3) conv
- * (r21d_byol.py:198); column = ci*49 + kh*7 + kw, columns >= 147 are zero. */
-int cstp_stem_im2col(const float* x, int N, int T, int H, int W, void* col, int ldk, void* stream);
 
 /* ---- BatchNorm (training mode), fused with ReLU / residual ---------------------------------------------
  * Replaces nn.BatchNorm3d / BatchNorm1d forward+backward and the ReLU / residual adds around them

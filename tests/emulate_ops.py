@@ -204,17 +204,6 @@ def stem_pack(x, P):
     P.view(N, T, H // 2, Wo, 2, 32)[..., :21] = rows.permute(0, 1, 2, 4, 3, 5).to(P.dtype)
 
 
-def stem_im2col(x, col):
-    _count()
-    N, C, T, H, W = x.shape
-    Ho, Wo = H // 2, W // 2
-    xp = F.pad(x, (3, 3, 3, 3))
-    patches = xp.unfold(3, 7, 2).unfold(4, 7, 2)            # (N, 3, T, Ho, Wo, 7, 7)
-    rows = patches.permute(0, 2, 3, 4, 1, 5, 6).reshape(N * T * Ho * Wo, 147)
-    col.zero_()
-    col[:, :147] = rows.to(col.dtype)
-
-
 def _group_view(t, groups):
     rows = t.numel() // t.shape[-1]
     return t.reshape(groups, rows // groups, t.shape[-1])

@@ -230,9 +230,9 @@ def test_conv_halo_layout_semantics(k, p, shape, cin, cout, dgrad):
 @pytest.mark.parametrize("k,p,shape,cin,cout,dgrad,G", [
     ((1, 3, 3), (0, 1, 1), (1, 2, 12, 12), 64, 144, True, 4),      # dgrad of the 64 -> 144 1x3x3 layers (conv2.*.spatial): slab axis h
     ((1, 3, 3), (0, 1, 1), (2, 3, 10, 20), 64, 144, True, 4),      # partial slab group along h, partial tiles along w / t
-    ((3, 1, 1), (1, 0, 0), (1, 8, 16, 8), 144, 64, False, 4),      # temporal forward 144 -> 64: slab axis t
-    ((3, 1, 1), (1, 0, 0), (2, 6, 8, 8), 80, 64, False, 2),        # two output frames per tile, ragged T
-    ((1, 3, 3), (0, 1, 1), (1, 1, 9, 8), 64, 64, False, 3),
+    ((1, 3, 3), (0, 1, 1), (2, 3, 7, 20), 64, 80, True, 2),        # two rows per tile, 16-channel tail of the operand, odd H
+    ((1, 3, 3), (0, 1, 1), (1, 2, 11, 12), 64, 96, True, 3),       # three rows per tile (ragged last group), 32-channel tail
+    ((1, 3, 3), (0, 1, 1), (1, 1, 9, 8), 64, 64, False, 3),        # forward-shaped tap list (the kernel takes either)
 ])
 def test_conv_slab_layout_semantics(k, p, shape, cin, cout, dgrad, G):
     """Interprets ops.conv_slab_layout + ops.slab_tables exactly as csrc/conv_halo.cu's slab mode does: every input slab
@@ -265,7 +265,7 @@ def test_conv_slab_layout_semantics(k, p, shape, cin, cout, dgrad, G):
     bw, bh, bt, bn = lay["box"]
     hw = lay["halo"][0]
     pitch = lay["pitch"]
-    assert bw * bh * bt * bn == 128 and (bh if axis == 1 else bt) == 1 and lay["n_tile"] == G * Np
+    assert axis == 1 and bw * bh * bt * bn == 128 and bh == 1 and lay["n_tile"] == G * Np
     (gdw, gdh, gdt, _, _), = lay["groups"]
     tap_of_koff = {ti * pad64(Ca): ti for (_, _, _, ti) in taps}
     nw = len(lay["taps"]) // nslots
@@ -287,14 +287,13 @@ def test_conv_slab_layout_semantics(k, p, shape, cin, cout, dgrad, G):
         return box.reshape(-1, Ca)
 
     out = torch.zeros(N, T, H, W, n_c)
-    step_h, step_t = (G if axis == 1 else bh), (G if axis == 2 else bt)
     for n0 in range(0, N, bn):
-        for t0 in range(0, T, step_t):
-            for h0 in range(0, H, step_h):
+        for t0 in range(0, T, bt):
+            for h0 in range(0, H, G):
                 for w0 in range(0, W, bw):
                     acc = torch.full((128, G * Np), float("nan"))        # stale accumulator: the init slabs must overwrite
                     for (s, init, doff, brow, width) in table:
-                        staged = fetch(w0 + gdw, h0 + gdh + (s if axis == 1 else 0), t0 + gdt + (s if axis == 2 else 0), n0)
+                        staged = fetch(w0 + gdw, h0 + gdh + s, t0 + gdt, n0)
                         first = init
                         for j in range(nw):
                             rows = staged[[j + a_ * pitch + r for a_ in range(16) for r in range(8)]]
@@ -305,12 +304,8 @@ def test_conv_slab_layout_semantics(k, p, shape, cin, cout, dgrad, G):
                     for r in range(128):
                         ww, hh_, tt, n_ = w0 + r % bw, h0 + (r // bw) % bh, t0 + (r // (bw * bh)) % bt, n0 + r // (bw * bh * bt)
                         for o in range(G):
-                            pos = (hh_ if axis == 1 else tt) + o
-                            if ww < W and n_ < N and (pos < H if axis == 1 else pos < T) and hh_ < H and tt < T:
-                                if axis == 1:
-                                    out[n_, tt, pos, ww] = acc[r, o * Np:o * Np + n_c]
-                                else:
-                                    out[n_, pos, hh_, ww] = acc[r, o * Np:o * Np + n_c]
+                            if ww < W and n_ < N and hh_ + o < H and tt < T:
+                                out[n_, tt, hh_ + o, ww] = acc[r, o * Np:o * Np + n_c]
     x5 = a[..., :a_c].permute(0, 4, 1, 2, 3)
     if not dgrad:
         ref = F.conv3d(x5, w, None, 1, p)

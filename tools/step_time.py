@@ -1,7 +1,7 @@
 """Step time of the pretraining step with its forward / backward / update split (CUDA events on the main stream).
-Development tool for schedule experiments; knobs come from the environment (CSTP_SMEM_KB, CSTP_STREAM_CTAS_PER_SM,
-CSTP_BN_REDUCE_CTAS_PER_SM).
-    python tools/step_time.py [B] [--no-overlap] [--steps K]"""
+Development tool for schedule experiments; the engine options of the DESIGN.md appendix come from the environment
+(CSTP_FUSE_POLICY, CSTP_FUSE_MIN_POSITIONS, ...) and are echoed in the result line.
+    python tools/step_time.py [B] [--no-overlap] [--no-graph] [--steps K]"""
 import json
 import os
 import sys
