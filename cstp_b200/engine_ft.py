@@ -27,6 +27,7 @@ def finetune_param_specs(num_classes: int, cls_bn: bool):
 
 class FinetuneEngine(StepEngine):
     VIEWS = 1
+    FORWARD_ONLY = False             # InferenceEngine: no backward program, no gradient / momentum store
 
     def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", num_classes: int = 101,
                  cls_bn: bool = True, record: bool = False, overlap: bool = True, backbone_grads: bool = True,
@@ -37,10 +38,13 @@ class FinetuneEngine(StepEngine):
                          fuse_min_positions=fuse_min_positions, fuse_policy=fuse_policy)
 
     def _make_stores(self):
-        specs = finetune_param_specs(self.num_classes, self.cls_bn)
-        self.train = FlatStore(specs, self.device)
+        self._make_param_stores()
         self.grad = self.train.like()
         self.mom = self.train.like()
+
+    def _make_param_stores(self):
+        specs = finetune_param_specs(self.num_classes, self.cls_bn)
+        self.train = FlatStore(specs, self.device)
         self.target = None
         self.bufs = FlatStore(bn_buffer_specs(specs), self.device)
         for name in self.bufs.slots:
@@ -59,14 +63,15 @@ class FinetuneEngine(StepEngine):
         self.norms = torch.zeros(B, **f32)
         self.nfeat = self._act(B, 512)                     # F.normalize(feat) as bf16 rows
         self.hfeat = self._act(B, 512) if self.cls_bn else self.nfeat
+        head_grads = not self.FORWARD_ONLY
         self.logits = torch.zeros(B, Cp, **f32)
-        self.dlogits = torch.zeros(B, Cp, **f32)
+        self.dlogits = torch.zeros(B, Cp, **f32) if head_grads else None
         self.loss = torch.zeros(1, **f32)
         self.ce_ws = torch.zeros(max(B, 16), **f32)
-        wc, wct = self._packed(self.train, "classify.weight", True)
+        wc, wct = self._packed(self.train, "classify.weight", head_grads)
         bias = self.train.slot("classify.bias")
         p_cls = ops.linear_plan(self.hfeat, wc, None, out_f32=self.logits, bias=bias)
-        site = self._site(self.train, True, "cls_bn", 512, 1, B) if self.cls_bn else None
+        site = self._site(self.train, head_grads, "cls_bn", 512, 1, B) if self.cls_bn else None
         self._rec("head.feat", self.feat)
         self._rec("head.nfeat", self.nfeat)
         self._rec("head.hfeat", self.hfeat)
@@ -84,6 +89,9 @@ class FinetuneEngine(StepEngine):
                 ops.bn_apply(self.nfeat, site.st, self.hfeat, relu=False)
             p_cls.run()
         self.fwd_online.append(head_fwd)
+        if not head_grads:
+            self._finish_build()
+            return
 
         # ---------------- backward program: head -> pool -> backbone
         g_out = self._act(B, Cp)
@@ -188,3 +196,72 @@ class FinetuneEngine(StepEngine):
                                 0.0, False, self.first_step, self.norm_out, self.sgd_ws)
         self.first_step = False
         self.pack_online()
+
+
+def inference_capacity(n: int) -> int:
+    """Batch capacity of the inference engine that runs an eval forward of n clips: the smallest power of two >= n up to
+    64, then the next multiple of 64 -- a handful of engines covers every clip count of a test set."""
+    if n < 1:
+        raise ValueError(f"an eval forward needs at least one clip, got {n}")
+    return 1 << (n - 1).bit_length() if n <= 64 else (n + 63) // 64 * 64
+
+
+class InferenceEngine(FinetuneEngine):
+    """Forward-only eval engine (model.eval(): every BatchNorm is the affine map of its running statistics) of a fixed
+    batch `capacity` that evaluates any n <= capacity clips: `run(n)` computes rows [0, n) of `x_static` and leaves the
+    other rows unread.  Eval BatchNorm couples no samples and the forward convolutions have no split-K, so a clip's
+    logits do not depend on the batch it runs in: they are bit-identical to FinetuneEngine(n).forward_eval's.
+
+    share: an engine whose parameter and BatchNorm running-statistics stores this one reads (the module's bound training
+    engine); None allocates them here.  Either way the packed bf16 weights are this engine's own (pack_online)."""
+
+    FORWARD_ONLY = True
+
+    def __init__(self, capacity: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", num_classes: int = 101,
+                 cls_bn: bool = True, share: FinetuneEngine | None = None, **options):
+        self._share = share
+        options["overlap"] = False              # one stream: there is no target network and no backward pass
+        super().__init__(capacity, T, H, W, device=device, num_classes=num_classes, cls_bn=cls_bn, backbone_grads=False,
+                         **options)
+        self.capacity = capacity
+        self.eval_mode = True
+        self.x_static = torch.zeros(capacity, 3, T, H, W, device=self.device, dtype=torch.float32)
+
+    def _make_stores(self):
+        if self._share is None:
+            self._make_param_stores()
+        else:
+            self.train, self.bufs, self.target = self._share.train, self._share.bufs, None
+        self.grad = self.mom = None
+
+    def run(self, n: int) -> torch.Tensor:
+        """Eval forward of rows [0, n) of x_static; returns self.logits, whose rows [0, n) are valid.  The program behind
+        the input pass is replayed from a CUDA graph captured on the first call."""
+        if not 1 <= n <= self.capacity:
+            raise ValueError(f"{n} clips do not fit an inference engine of capacity {self.capacity}")
+        E.ops.stem_pack(self.x_static[:n], self.stem_rows[:n])
+        if not self.use_graph:
+            for op in self.fwd_online:
+                op()
+            return self.logits
+        if self._graph is None:
+            for op in self.fwd_online:           # eager warm-up: one-time kernel attribute calls happen here
+                op()
+            torch.cuda.synchronize(self.device)
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                for op in self.fwd_online:
+                    op()
+            self._graph = g
+        self._graph.replay()
+        return self.logits
+
+    def forward_batch(self, x: torch.Tensor) -> torch.Tensor:
+        """Copies the clips x (n, 3, T, H, W) into x_static and runs them (see run)."""
+        self.x_static[:x.shape[0]].copy_(x)
+        return self.run(x.shape[0])
+
+    def cross_entropy(self, labels):
+        """nn.CrossEntropyLoss() over the rows of the last run (labels has one entry per row); fills self.loss."""
+        n = labels.shape[0]
+        E.ops.ce_loss(self.logits[:n], labels, self.num_classes, self.loss, None, self.ce_ws)

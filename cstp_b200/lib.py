@@ -220,6 +220,8 @@ SIGNATURES = {
     "cstp_sgd_clip_step": (_i, [_vp, _vp, _vp, _i64, _f, _f, _f, _f, _i, _i, _vp, _vp, _vp]),
     "cstp_sgd_clip_step_dev": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "cstp_clip_assemble": (_i, [_vp, _i, _i, _i, _i, _vp]),
+    "cstp_video_accumulate": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _i, _vp]),
+    "cstp_video_finalize": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "cstp_bn_sync_buffer_bytes": (C.c_longlong, [_i, _i, _i]),
     "cstp_bn_sync_exchange": (_i, [_vp, _i, _vp, _i, _i, _i, _i, C.c_uint32, _vp, _vp, _vp, _vp]),
 }

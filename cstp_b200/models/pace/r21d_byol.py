@@ -213,6 +213,10 @@ class R21DBYOL(nn.Module):
                     w.uniform_(-bound, bound)
         self._engine = None
         self._engine_key = None
+        self._infer = {}              # (capacity, T, H, W, device) -> engine_ft.InferenceEngine (eval forwards)
+        self._infer_owner = None      # the inference engine that owns the stores while no engine is bound
+        self._last_engine = None      # the engine that ran the last forward
+        self._wgen = 0                # weight generation (see _repack_if_changed)
         if pretrain:
             self._trainable_names = [n for n, _ in _engine_mod.trainable_param_specs()]
         else:
@@ -263,6 +267,11 @@ class R21DBYOL(nn.Module):
             self._dirty = True
         return eng
 
+    def _ft_key(self, x):
+        B, _, T, H, W = x.shape
+        bgrads = any(p.requires_grad for n, p in self.named_parameters() if n.startswith("online_net."))
+        return (B, T, H, W, x.device, bgrads)
+
     def _bind_ft(self, x):
         """Finetune / test flavour of _bind: a FinetuneEngine per (batch geometry, frozen-backbone) configuration."""
         from ... import engine_ft
@@ -270,18 +279,23 @@ class R21DBYOL(nn.Module):
         if not isinstance(self.cls_bn, nn.Module):
             raise TypeError("'bool' object is not callable")      # the reference calls self.cls_bn(feat) unconditionally
         B, _, T, H, W = x.shape
-        bgrads = any(p.requires_grad for n, p in self.named_parameters() if n.startswith("online_net."))
-        key = (B, T, H, W, x.device, bgrads)
+        key = self._ft_key(x)
         eng = self._engine
         if eng is None or self._engine_key != key:
             new = engine_ft.FinetuneEngine(B, T, H, W, device=x.device, num_classes=self.num_classes, cls_bn=True,
-                                           backbone_grads=bgrads, **getattr(self, "engine_options", {}))
+                                           backbone_grads=key[-1], **getattr(self, "engine_options", {}))
             if eng is not None:
                 new.mom.copy_(eng.mom)
                 new.first_step = eng.first_step
+            self.free_inference_engines()        # they read the stores the parameters are about to leave
             eng = self._engine = new
             self._engine_key = key
             self._alias_ptr = None
+        self._alias_ft(eng)
+        return eng
+
+    def _alias_ft(self, eng):
+        """Points every parameter / BatchNorm buffer at eng's flat stores (again after .cuda() / .to() moved them)."""
         sentinel = self.online_net.conv1.spatial_conv.weight
         if getattr(self, "_alias_ptr", None) != sentinel.data_ptr():
             with torch.no_grad():
@@ -297,40 +311,103 @@ class R21DBYOL(nn.Module):
                             v.copy_(mod._buffers[b])
                             mod._buffers[b] = v
                         nbt.append(mod)
-                flat = torch.stack([m._buffers["num_batches_tracked"].to(x.device) for m in nbt])
+                flat = torch.stack([m._buffers["num_batches_tracked"].to(eng.device) for m in nbt])
                 for i, m in enumerate(nbt):
                     m._buffers["num_batches_tracked"] = flat[i]
                 self._nbt, self._nbt_inc = flat, torch.ones_like(flat)
             self._alias_ptr = sentinel.data_ptr()
             self._dirty = True
+
+    def inference_engine(self, capacity: int, T: int, H: int, W: int, device):
+        """The cached forward-only eval engine (engine_ft.InferenceEngine) of this batch capacity and clip size.  It reads
+        the parameters and BatchNorm running statistics of the bound engine; while no engine is bound, the first one
+        created owns them and the parameters are aliased onto it, as _bind_ft does."""
+        from ... import engine_ft
+        if not isinstance(self.cls_bn, nn.Module):
+            raise TypeError("'bool' object is not callable")
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        owner = self._engine
+        if owner is None:
+            owner = self._infer_owner
+            if owner is not None and owner.device != device:
+                self.free_inference_engines()
+                owner = None
+        elif owner.device != device:
+            raise _engine_mod.ops.L.CstpError(f"the bound engine lives on {owner.device}, not {device}")
+        key = (capacity, T, H, W, device)
+        eng = self._infer.get(key)
+        if eng is None:
+            eng = engine_ft.InferenceEngine(capacity, T, H, W, device=device, num_classes=self.num_classes, cls_bn=True,
+                                            share=owner, **getattr(self, "engine_options", {}))
+            self._infer[key] = eng
+            if owner is None:
+                self._infer_owner = owner = eng
+                self._alias_ptr = None
+        self._alias_ft(owner)
         return eng
 
+    def free_inference_engines(self):
+        """Frees the cached eval engines of other batch sizes (activations, packed weights, CUDA graphs); the next eval
+        forward builds what it needs again.  The bound training engine is not affected."""
+        self._infer.clear()
+        if self._infer_owner is not None:
+            self._infer_owner = None
+            if self._engine is None:
+                self._alias_ptr = None          # the parameters move to the next engine that is built
+        if self._last_engine is not self._engine:
+            self._last_engine = None
+
     def _repack_if_changed(self, eng):
-        """Re-packs the bf16 tensor-core weights when the fp32 parameters changed behind the engine's back.  The
-        parameters are views of the engine's flat buffer, so every in-place update (optimizer.step, load_state_dict)
-        bumps the version counter of that buffer."""
-        v = eng.train.data._version
-        if self._dirty or getattr(self, "_packed_version", None) != (id(eng), v):
-            eng.pack_online()
-            self._packed_version = (id(eng), v)
+        """Re-packs eng's bf16 tensor-core weights when the fp32 parameters changed since it last packed them.  The
+        parameters are views of the engines' shared flat buffer, so every in-place update (optimizer.step,
+        load_state_dict) bumps the version counter of that buffer; every other change (the fused finetune step, edits
+        announced through _dirty) starts a new weight generation."""
+        if self._dirty:
+            self._wgen += 1
             self._dirty = False
+        key = (eng.train.data._version, self._wgen)
+        if getattr(eng, "_packed_key", None) != key:
+            eng.pack_online()
+            eng._packed_key = key
 
     def _forward_ft(self, x1):
+        if not self.training:
+            return self._forward_eval_ft(x1)
         eng = self._bind_ft(x1)
+        self._last_engine = eng
         x1 = x1.contiguous()
-        if self.training and torch.is_grad_enabled():
+        if torch.is_grad_enabled():
             out = _FinetuneFn.apply(self, x1, *self._trainable())
             self._nbt += self._nbt_inc
             self._dirty = True
             return out
         self._repack_if_changed(eng)
-        if self.training:
-            eng.eval_mode = False
-            eng.forward(x1)
-            self._nbt += self._nbt_inc
-        else:
-            eng.forward_eval(x1)
+        eng.eval_mode = False
+        eng.forward(x1)
+        self._nbt += self._nbt_inc
         return eng.logits[:, :self.num_classes].clone()
+
+    def _forward_eval_ft(self, x):
+        """model.eval() forward.  A batch of the bound engine's geometry runs on that engine; any other batch size runs on
+        the cached inference engine of its capacity bucket (engine_ft.inference_capacity), which leaves the bound engine,
+        its momentum and its captured step untouched.  Logits are bit-identical either way."""
+        from ... import engine_ft
+        _engine_mod.ops.require_device(x)
+        eng = self._engine
+        n = x.shape[0]
+        if eng is not None and (self._engine_key == self._ft_key(x) or eng.device != x.device):
+            eng = self._bind_ft(x)
+            self._repack_if_changed(eng)
+            eng.forward_eval(x.contiguous())
+        else:
+            _, _, T, H, W = x.shape
+            eng = self.inference_engine(engine_ft.inference_capacity(n), T, H, W, x.device)
+            self._repack_if_changed(eng)
+            eng.forward_batch(x)
+        self._last_engine = eng
+        return eng.logits[:n, :self.num_classes].clone()
 
     @torch.no_grad()
     def finetune_step(self, x, labels, lr=0.025, momentum=0.9, weight_decay=1e-3, grad_sync=None):
@@ -352,6 +429,9 @@ class R21DBYOL(nn.Module):
             self._ft_ranges = eng.trainable_ranges(frozen) if frozen else None
         eng.optimizer_step(lr, momentum, weight_decay, ranges=self._ft_ranges)
         self._nbt += self._nbt_inc
+        self._wgen += 1                          # the kernel updated the weights: other engines must re-pack
+        eng._packed_key = (eng.train.data._version, self._wgen)       # optimizer_step re-packed this one
+        self._last_engine = eng
         return eng.loss
 
     def _bump_nbt(self):

@@ -1075,6 +1075,25 @@ def bn_eval_coeffs(st: BNState, gamma, beta, running_mean, running_var, eps: flo
                                          st.groups, float(eps), _ptr(st.scale), _ptr(st.shift), _stream()))
 
 
+def video_accumulate(logits, n_cls: int, seg, sums, rows: int | None = None) -> None:
+    """sums[slot] += logits[first:first + count, :n_cls] in row order for every {slot, first, count} row of the int32
+    device table seg [n][3] (count <= 0: skipped).  rows: how many leading rows of logits entries may name."""
+    _require_cuda(logits, seg, sums)
+    L.check(L.load().cstp_video_accumulate(_ptr(logits), rows or logits.shape[0], logits.shape[1], n_cls, _ptr(seg),
+                                           seg.shape[0], _ptr(sums), sums.shape[0], _stream()))
+
+
+def video_finalize(sums, fin, topk_out, labels=None, mean_out=None, hits=None) -> None:
+    """For every {slot, count, video} row of the int32 device table fin [n][3]: mean = sums[slot] / count ->
+    mean_out[video] (optional), topk_out[video] (int64 [videos][k]: descending, ties to the lower class), hits[0] / hits[1]
+    += top-1 / top-5 hits against labels[video] (int64, optional); the slot is zeroed."""
+    _require_cuda(sums, fin, topk_out, labels, mean_out, hits)
+    n_slots, n_cls = sums.shape
+    L.check(L.load().cstp_video_finalize(_ptr(sums), n_slots, n_cls, _ptr(fin), fin.shape[0], topk_out.shape[0],
+                                         topk_out.shape[1], _ptr(labels), _ptr(mean_out), _ptr(topk_out), _ptr(hits),
+                                         _stream()))
+
+
 def ema_update(k, q, m: float) -> None:
     import numpy as np
     L.check(L.load().cstp_ema_update(_ptr(k), _ptr(q), k.numel(), float(np.float32(m)), float(np.float32(1.0 - m)),

@@ -205,9 +205,9 @@ def finetune_epochs(model, train_batches, val_batches, opts, begin_epoch: int = 
         with torch.no_grad():
             for x, labels in val_batches(epoch):
                 model(x, None, o_type=task)                          # eval-mode forward (running statistics)
-                eng = model._engine
+                eng = model._last_engine                             # an inference engine when x.shape[0] is not the training batch
                 eng.cross_entropy(labels)
-                hits = (eng.logits[:, :model.num_classes].argmax(1) == labels).sum()
+                hits = (eng.logits[:x.shape[0], :model.num_classes].argmax(1) == labels).sum()
                 z = torch.zeros(1, device=eng.loss.device)
                 acc = fold(acc or (z, z.clone(), 0), eng.loss.clone(), hits, x.shape[0])
         if acc is None:

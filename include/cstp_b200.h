@@ -374,6 +374,20 @@ int cstp_ce_loss(const float* logits, const int64_t* labels, int B, int n_cls, i
  * shift = beta - running_mean*scale, replicated for `groups` groups. */
 int cstp_bn_eval_coeffs(const float* gamma, const float* beta, const float* running_mean, const float* running_var, int C,
                         int Cp, int groups, float eps, float* scale, float* shift, void* stream);
+/* Video-level scoring of test.py:76-93 (csrc/video_eval.cu).  A video's clip logits are summed into an fp32 slot
+ * sums[slot][n_cls] that keeps accumulating across launches, in clip order (no float atomics: bit-reproducible, equal to a
+ * sequential fp32 loop).  Work lists are DEVICE int32 tables the host may rewrite in place between graph replays; an entry
+ * whose count is <= 0 (or that points outside the buffers) is skipped.
+ * accumulate: seg[n_seg][3] = {slot, first row, row count}; adds rows [first, first + count) of logits (fp32 [rows][ld],
+ *   first n_cls columns) to sums[slot].  Rows no entry names are never read. */
+int cstp_video_accumulate(const float* logits, int rows, int ld, int n_cls, const int32_t* seg, int n_seg, float* sums,
+                          int n_slots, void* stream);
+/* finalize: fin[n_fin][3] = {slot, clip count, video}; mean = sums[slot] / count (fp32), optionally written to
+ * mean_out[video][n_cls]; topk_out[video][k] (1 <= k <= 8) = class indices by mean, descending, ties to the lower index;
+ * with hits: hits[0] += (top-1 == labels[video]), hits[1] += (labels[video] among the top 5) (int64 counters).  The slot
+ * is left zero. */
+int cstp_video_finalize(float* sums, int n_slots, int n_cls, const int32_t* fin, int n_fin, int n_videos, int k,
+                        const int64_t* labels, float* mean_out, int64_t* topk_out, int64_t* hits, void* stream);
 
 /* ---- optimiser side -------------------------------------------------------------------------------------
  * EMA target update (r21d_byol.py:331-337): k = k*m + q*(1-m), bit-exact fp32 (two rounded products, one add). */
