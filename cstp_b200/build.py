@@ -19,7 +19,7 @@ LIB_PATH = PKG_DIR / "libcstp_b200.so"
 OBJ_DIR = PKG_DIR / "_build"
 
 SOURCES = ["common.cu", "conv_gemm.cu", "conv_halo.cu", "wgrad.cu", "wgrad_halo.cu", "elementwise.cu", "loss_optim.cu", "ntxent_tc.cu",
-           "clip_pipeline.cu", "p2p_sync.cu", "video_eval.cu"]
+           "clip_pipeline.cu", "p2p_sync.cu", "video_eval.cu", "retrieval.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

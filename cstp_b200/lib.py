@@ -222,6 +222,9 @@ SIGNATURES = {
     "cstp_clip_assemble": (_i, [_vp, _i, _i, _i, _i, _vp]),
     "cstp_video_accumulate": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _i, _vp]),
     "cstp_video_finalize": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "cstp_l2_normalize_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),
+    "cstp_knn_partial": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "cstp_knn_merge": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
     "cstp_bn_sync_buffer_bytes": (C.c_longlong, [_i, _i, _i]),
     "cstp_bn_sync_exchange": (_i, [_vp, _i, _vp, _i, _i, _i, _i, C.c_uint32, _vp, _vp, _vp, _vp]),
 }

@@ -1094,6 +1094,63 @@ def video_finalize(sums, fin, topk_out, labels=None, mean_out=None, hits=None) -
                                          _stream()))
 
 
+KNN_MAX_K, KNN_MAX_SPLITS, KNN_QUERY_TILE, KNN_CTAS_PER_SM = 64, 32, 64, 3
+
+
+def knn_splits(nq: int, ng: int, sms: int = 148) -> int:
+    """Gallery splits of cstp_knn_partial for nq queries against ng gallery rows: the count (at most 32, at least 512
+    gallery rows each) whose grid of query tiles x splits leaves the least of its last wave of 148 x 3 resident CTAs
+    idle; ties go to fewer splits (less merge work).  Results do not depend on it."""
+    tiles, slots = -(-nq // KNN_QUERY_TILE), sms * KNN_CTAS_PER_SM
+    best, best_eff = 1, 0.0
+    for s in range(1, max(1, min(KNN_MAX_SPLITS, ng // 512)) + 1):
+        ctas = tiles * s
+        eff = ctas / (-(-ctas // slots) * slots)
+        if eff > best_eff + 1e-9:
+            best, best_eff = s, eff
+    return best
+
+
+def l2_normalize_rows(x, y) -> None:
+    """y[n][d] = x[:, :d] / max(||x[:, :d]||, 1e-12) (F.normalize) for x fp32 [n][ld], y fp32 [n][d] contiguous."""
+    _require_cuda(x, y)
+    if x.dtype != torch.float32 or y.dtype != torch.float32 or x.stride(1) != 1 or not y.is_contiguous() \
+            or x.shape[0] != y.shape[0] or x.shape[1] < y.shape[1]:
+        raise L.CstpError("l2_normalize_rows: x fp32 [n][>= d] with unit column stride, y contiguous fp32 [n][d]")
+    L.check(L.load().cstp_l2_normalize_rows(_ptr(x), x.shape[0], y.shape[1], x.stride(0), _ptr(y), _stream()))
+
+
+def knn_partial(q, g, k: int, splits: int, part_val, part_idx) -> None:
+    """Each gallery split's top-k of s(q, g) for normalised rows q [nq][d], g [ng][d] into part_val fp32 /
+    part_idx int32 [splits][nq][k] (similarity descending, then the lower gallery index; -inf / -1 past the split)."""
+    _require_cuda(q, g, part_val, part_idx)
+    if q.dtype != torch.float32 or g.dtype != torch.float32 or not (q.is_contiguous() and g.is_contiguous()) \
+            or q.shape[1] != g.shape[1] or part_val.dtype != torch.float32 or part_idx.dtype != torch.int32 \
+            or part_val.shape != (splits, q.shape[0], k) or part_idx.shape != part_val.shape:
+        raise L.CstpError("knn_partial: contiguous fp32 q [nq][d], g [ng][d]; part_val fp32 / part_idx int32 "
+                          "[splits][nq][k]")
+    L.check(L.load().cstp_knn_partial(_ptr(q), q.shape[0], _ptr(g), g.shape[0], q.shape[1], k, splits, _ptr(part_val),
+                                      _ptr(part_idx), _stream()))
+
+
+def knn_merge(part_val, part_idx, idx_out, sim_out, q_labels=None, g_labels=None, cutoffs=None, hits=None) -> None:
+    """Merges knn_partial's lists into idx_out int64 / sim_out fp32 [nq][k]; with hits (int64 [len(cutoffs)]):
+    hits[c] += queries with a label match among their first cutoffs[c] neighbours.  g_labels (int64) must hold one label
+    per gallery row knn_partial searched."""
+    _require_cuda(part_val, part_idx, idx_out, sim_out, q_labels, g_labels, cutoffs, hits)
+    splits, nq, k = part_val.shape
+    if part_idx.shape != part_val.shape or idx_out.dtype != torch.int64 or sim_out.dtype != torch.float32 \
+            or idx_out.shape != (nq, k) or sim_out.shape != (nq, k) or not (idx_out.is_contiguous() and sim_out.is_contiguous()):
+        raise L.CstpError("knn_merge: idx_out int64 / sim_out fp32 contiguous [nq][k] for the partial lists' nq, k")
+    if hits is not None and (q_labels is None or g_labels is None or cutoffs is None or q_labels.dtype != torch.int64
+                             or q_labels.numel() != nq or g_labels.dtype != torch.int64 or cutoffs.dtype != torch.int32
+                             or hits.dtype != torch.int64 or hits.numel() != cutoffs.numel()):
+        raise L.CstpError("knn_merge: int64 q_labels [nq] and g_labels, int32 cutoffs, int64 hits [len(cutoffs)]")
+    L.check(L.load().cstp_knn_merge(_ptr(part_val), _ptr(part_idx), nq, k, splits, _ptr(idx_out), _ptr(sim_out),
+                                    _ptr(q_labels), _ptr(g_labels), _ptr(cutoffs), 0 if cutoffs is None else cutoffs.numel(),
+                                    _ptr(hits), _stream()))
+
+
 def ema_update(k, q, m: float) -> None:
     import numpy as np
     L.check(L.load().cstp_ema_update(_ptr(k), _ptr(q), k.numel(), float(np.float32(m)), float(np.float32(1.0 - m)),

@@ -389,6 +389,26 @@ int cstp_video_accumulate(const float* logits, int rows, int ld, int n_cls, cons
 int cstp_video_finalize(float* sums, int n_slots, int n_cls, const int32_t* fin, int n_fin, int n_videos, int k,
                         const int64_t* labels, float* mean_out, int64_t* topk_out, int64_t* hits, void* stream);
 
+/* Nearest-neighbour retrieval (csrc/retrieval.cu).  Defined fp32 arithmetic, no contraction: results are bit-identical
+ * for every tiling and split.
+ * l2_normalize_rows: y[n][d] = x / max(||x||_2, 1e-12) (F.normalize), x fp32 [n][ld].  The sum of squares is lane-strided
+ *   over a warp (lane l adds x[l]^2, x[l+32]^2, ... in order) and then reduced by an xor butterfly over offsets 16, 8, 4,
+ *   2, 1; sqrt and the division are correctly rounded. */
+int cstp_l2_normalize_rows(const float* x, int n, int d, int ld, float* y, void* stream);
+/* knn_partial: q fp32 [nq][d], g fp32 [ng][d] (rows normalised, 16-byte aligned, d % 4 == 0).  s(q, g) is the sequential
+ * chain acc = acc + q[j] * g[j], j = 0 .. d-1, each product and sum rounded.  Gallery split s = rows
+ * [ng*s/splits, ng*(s+1)/splits); part_val / part_idx [splits][nq][k] receive each split's top-k (similarity descending,
+ * then the lower gallery index), empty entries -inf / -1.  1 <= k <= 64, 1 <= splits <= 32; the similarity matrix is
+ * never written. */
+int cstp_knn_partial(const float* q, int nq, const float* g, int ng, int d, int k, int splits, float* part_val,
+                     int32_t* part_idx, void* stream);
+/* knn_merge: the splits' lists -> idx_out int64 [nq][k], sim_out fp32 [nq][k] in the same order (-1 / -inf past ng).
+ * With hits (then q_labels int64 [nq], g_labels int64 [ng], cutoffs int32 [n_cut], all device): for every cutoff c,
+ * hits[c] += (one of the first c neighbours has g_labels == q_labels[i]), int64 counters. */
+int cstp_knn_merge(const float* part_val, const int32_t* part_idx, int nq, int k, int splits, int64_t* idx_out,
+                   float* sim_out, const int64_t* q_labels, const int64_t* g_labels, const int32_t* cutoffs, int n_cut,
+                   int64_t* hits, void* stream);
+
 /* ---- optimiser side -------------------------------------------------------------------------------------
  * EMA target update (r21d_byol.py:331-337): k = k*m + q*(1-m), bit-exact fp32 (two rounded products, one add). */
 int cstp_ema_update(float* k, const float* q, int64_t n, float m, float one_minus_m, void* stream);
