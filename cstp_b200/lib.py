@@ -168,6 +168,14 @@ class ClipView(C.Structure):
     ]
 
 
+class JpegImage(C.Structure):
+    """cstp_jpeg_image: one stream of a `cstp_jpeg_decode` batch (include/cstp_b200.h)."""
+    _fields_ = [("src_offset", C.c_int64), ("src_bytes", C.c_int64), ("out", C.c_void_p),
+                ("width", C.c_int32), ("height", C.c_int32), ("ws_offset", C.c_int64)]
+
+
+CSTP_JPEG_UNSUPPORTED, CSTP_JPEG_MALFORMED, CSTP_JPEG_SIZE = 1, 2, 3
+
 _vp, _i, _i64, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
 
 # name -> (restype, argtypes); the single source of truth for the symbols include/cstp_b200.h declares.
@@ -225,6 +233,8 @@ SIGNATURES = {
     "cstp_l2_normalize_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "cstp_knn_partial": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "cstp_knn_merge": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "cstp_jpeg_workspace_bytes": (C.c_longlong, [_i, _i]),
+    "cstp_jpeg_decode": (_i, [_vp, _vp, _i, _vp, _vp, C.c_longlong, _vp]),
     "cstp_bn_sync_buffer_bytes": (C.c_longlong, [_i, _i, _i]),
     "cstp_bn_sync_exchange": (_i, [_vp, _i, _vp, _i, _i, _i, _i, C.c_uint32, _vp, _vp, _vp, _vp]),
 }

@@ -1189,3 +1189,24 @@ def note_replayed(n: int) -> None:
 def launch_count() -> int:
     """Kernels of this library launched so far: direct launches through the C ABI plus launches replayed from CUDA graphs."""
     return int(L.load().cstp_launch_count()) + _replayed_launches
+
+
+def jpeg_workspace_bytes(width: int, height: int) -> int:
+    """Workspace bytes cstp_jpeg_decode needs for one image of this size (any supported sampling)."""
+    v = L.load().cstp_jpeg_workspace_bytes(int(width), int(height))
+    if v < 0:
+        raise ValueError(f"JPEG frame size {width}x{height} outside 1 .. 65535")
+    return v
+
+
+def jpeg_decode(staged, data_offset: int, n_images: int, status, workspace) -> None:
+    """Decodes a batch staged in one uint8 device buffer: n_images cstp_jpeg_image descriptors at its start, the
+    concatenated streams from data_offset.  status: int32 [n_images]; workspace: uint8, each image's slice at its
+    descriptor's ws_offset."""
+    _require_cuda(staged, status, workspace)
+    if staged.dtype != torch.uint8 or status.dtype != torch.int32 or status.numel() < n_images \
+            or workspace.dtype != torch.uint8 or not (staged.is_contiguous() and workspace.is_contiguous()):
+        raise L.CstpError("jpeg_decode: contiguous uint8 staging and workspace buffers, int32 status [n_images]")
+    base = staged.data_ptr()
+    L.check(L.load().cstp_jpeg_decode(C.c_void_p(base + data_offset), C.c_void_p(base), n_images, _ptr(status),
+                                      _ptr(workspace), workspace.numel(), _stream()))

@@ -461,6 +461,32 @@ typedef struct {
  * staging of the horizontal pass; CSTP_EINVAL when it does not fit).  One CTA per (frame, view). */
 int cstp_clip_assemble(const cstp_clip_view* views, int n_views, int T, int S, int max_crop_h, void* stream);
 
+/* ---- JPEG decoding (csrc/jpeg_decode.cu) -------------------------------------------------------------------
+ * Baseline / extended-sequential Huffman JPEG (SOF0 / SOF1, 8-bit samples, one interleaved scan; grayscale or YCbCr
+ * 4:4:4, 4:2:2 (h2v1), 4:2:0 (h2v2); restart intervals; any size) decoded to RGB uint8 [height][width][3], byte for
+ * byte what Pillow on libjpeg-turbo returns for Image.open(...).convert("RGB") (ISLOW IDCT, fancy upsampling).  One call
+ * decodes a batch on `stream`: stage A parses and entropy-decodes (one warp per image, one lane per restart interval),
+ * stage B runs the IDCT per block, stage C upsamples and converts colour per pixel.  status[i] becomes 0 or one of the
+ * codes below; a rejected image leaves its `out` unspecified and touches nothing outside its own stream, output and
+ * workspace slice.  Where libjpeg would warn and fill in zeros (corrupt or truncated entropy data), this decoder
+ * reports CSTP_JPEG_MALFORMED. */
+#define CSTP_JPEG_UNSUPPORTED 1 /* progressive / arithmetic / lossless / hierarchical, 12-bit, CMYK or RGB, other
+                                   sampling, several scans, no Huffman table (Motion-JPEG) */
+#define CSTP_JPEG_MALFORMED 2   /* truncated or corrupt stream, a missing quantisation table */
+#define CSTP_JPEG_SIZE 3        /* SOF size differs from (width, height), or an invalid size / workspace slice */
+typedef struct {
+  int64_t src_offset, src_bytes; /* this image's stream inside `data` */
+  uint8_t* out;                  /* device: RGB uint8 [height][width][3] */
+  int32_t width, height;         /* expected size: a stream of another size is rejected */
+  int64_t ws_offset;             /* this image's slice of the workspace (a multiple of 256, workspace_bytes long) */
+} cstp_jpeg_image;
+/* Workspace bytes one image of this size needs, whatever its sampling; -1 outside 1 .. 65535. */
+long long cstp_jpeg_workspace_bytes(int width, int height);
+/* data: DEVICE, the concatenated streams; images: DEVICE array of n_images descriptors; status: DEVICE int32
+ * [n_images]; workspace: DEVICE, 256-byte aligned, workspace_bytes long. */
+int cstp_jpeg_decode(const uint8_t* data, const cstp_jpeg_image* images, int n_images, int32_t* status,
+                     void* workspace, long long workspace_bytes, void* stream);
+
 /* ---- SyncBN statistics exchange over NVLink peer memory ----------------------------------------------------
  * The all-reduce(SUM) of the [groups][2][Cp] row a world-synchronised BatchNorm call exchanges (the north star's SyncBN;
  * no counterpart in the reference, whose --sync_bn group holds one rank: models/model.py:95-96), as ONE kernel that
