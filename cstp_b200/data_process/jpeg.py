@@ -5,13 +5,15 @@ host, and neither a resident store of decoded frames nor host cores for decoding
   * `jpeg_size(b)`       (width, height) from the SOF segment, read on the host without touching entropy data.
   * `GpuJpegDecoder`     `decode(streams, sizes, outs)`: one upload and one `cstp_jpeg_decode` call per batch on the
                          current stream; `check(status, names)` raises ValueError for the rejected images.
+  * `JpegSlabs`          what every JPEG-fed batch source shares: `read_frames`, the frame-size cache, one decode call per
+                         batch into an arena of per-video slabs, and the status of that decode checked at the next request.
   * `FrameDirReader`     `read_frames(video, frame_numbers) -> [bytes]` for videos extracted to frame directories.
 """
 from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Dict, List, Sequence, Tuple
+from typing import Callable, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -136,6 +138,62 @@ def raise_for_status(status: np.ndarray, names: Sequence = None) -> None:
         what = names[i] if names is not None else f"image {i}"
         more = f" ({bad.size - 1} more rejected in this batch)" if bad.size > 1 else ""
         raise ValueError(f"{what}: {REASONS.get(int(status[i]), f'status {int(status[i])}')}{more}")
+
+
+class JpegSlabs:
+    """Per-batch decoding of the frames a batch reads: `decode(videos, frames)` reads frames[k] of videos[k] with
+    read_frames(video, frame_numbers) -> [bytes], uploads them once and decodes them in one call on the current stream
+    into a fresh arena, one [len(frames[k])][H][W][3] slab per video.  Nothing is resident beyond one batch's frames.
+
+    Frame sizes come from each video's first frame (frame number `first_frame`, read once and cached), or from
+    `sizes[video] = (w, h)` when given.  `check()` waits for the last decode and raises ValueError naming the video and
+    the frame of the first rejected stream; `decode` calls it for the previous batch, by which time that decode has
+    usually finished."""
+
+    def __init__(self, read_frames: Callable[[int, Sequence[int]], List[bytes]], first_frame: int,
+                 sizes: Optional[Sequence[Tuple[int, int]]] = None, device="cuda"):
+        self.read_frames, self.first_frame = read_frames, first_frame
+        self.decoder = GpuJpegDecoder(device)
+        self._sizes: Dict[int, Tuple[int, int]] = {i: tuple(s) for i, s in enumerate(sizes)} if sizes is not None else {}
+        self._pending = None                       # (pinned status, event, frame names) of the last decode
+
+    def frame_size(self, video: int) -> Tuple[int, int]:
+        if video not in self._sizes:
+            self._sizes[video] = jpeg_size(self.read_frames(video, [self.first_frame])[0])
+        return self._sizes[video]
+
+    def check(self) -> None:
+        if self._pending is not None:
+            host, ev, names = self._pending
+            self._pending = None
+            ev.synchronize()
+            raise_for_status(host.numpy(), names)
+
+    def decode(self, videos: Sequence[int], frames: Sequence[Sequence[int]]) -> List[torch.Tensor]:
+        self.check()
+        sizes = [self.frame_size(i) for i in videos]
+        arena = torch.empty(sum(len(fr) * w * h * 3 for fr, (w, h) in zip(frames, sizes)), dtype=torch.uint8,
+                            device=self.decoder.device)
+        streams, exp, outs, names, slabs = [], [], [], [], []
+        off = 0
+        for i, fr, (w, h) in zip(videos, frames, sizes):
+            slab = arena[off:off + len(fr) * h * w * 3].view(len(fr), h, w, 3)
+            off += slab.numel()
+            data = self.read_frames(i, fr)
+            if len(data) != len(fr):
+                raise ValueError(f"read_frames returned {len(data)} streams for {len(fr)} frames of video {i}")
+            streams += data
+            exp += [(w, h)] * len(fr)
+            outs += list(slab)
+            names += [f"video {i} frame {f}" for f in fr]
+            slabs.append(slab)
+        status = self.decoder.decode(streams, exp, outs)
+        host = torch.empty(len(streams), dtype=torch.int32).pin_memory()
+        host.copy_(status, non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record()
+        self._pending = (host, ev, names)
+        return slabs
 
 
 class FrameDirReader:

@@ -8,19 +8,24 @@ averaging, top-k and hit counting run in two small kernels (csrc/video_eval.cu).
 
 The same packing loop extracts per-video backbone features (video_features: the mean of the pooled 512-d feature in
 front of the classification head), which retrieve_videos searches for nearest neighbours (csrc/retrieval.cu).
+
+test_videos_jpeg / video_features_jpeg run the same loop from JPEG frames instead of a resident store: each batch
+decodes only the frames its clips read, on the GPU, and the results are the store-fed call's bits.
 """
 from __future__ import annotations
 
+import itertools
 import math
-from typing import Callable, Optional, Sequence
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 
 from . import engine as _engine_mod
 from .data_process.clip_plan import FinetuneClipSampler
-from .data_process.datasets import GpuVideoStore
+from .data_process.datasets import GpuVideoStore, clip_frames
 from .data_process.gpu_clips import GpuClipPipeline
+from .data_process.jpeg import JpegSlabs
 
 TOPK = 5
 
@@ -53,24 +58,75 @@ def batch_tables(counts: Sequence[int], capacity: int) -> np.ndarray:
     return tab
 
 
-def _plan_clips(store: GpuVideoStore, total_frames: Sequence[int], videos: range, sampler: FinetuneClipSampler):
+class _StoreFrames:
+    """Test windows read from a resident GpuVideoStore."""
+
+    def __init__(self, store: GpuVideoStore):
+        self.store, self.device = store, store.device
+
+    def frame_size(self, v: int):
+        vid = self.store[v]
+        return vid.shape[2], vid.shape[1]
+
+    def batch(self, clips, owners):
+        return clips, [self.store[v] for v in owners]
+
+    def finish(self) -> None:
+        pass
+
+
+def batch_slabs(clips, owners):
+    """What one packed batch decodes when it is fed from JPEG frames: the batch's clips grouped by video (the packing
+    keeps a video's clips together), the distinct frames of each video's clips, and the clips remapped onto one slab per
+    video (datasets.clip_frames).  Returns (videos, frame numbers per video, remapped clips, slab index per clip)."""
+    videos, frames, remapped, slab = [], [], [], []
+    for v, group in itertools.groupby(zip(owners, clips), key=lambda oc: oc[0]):
+        fr, rc = clip_frames([c for _, c in group])
+        slab += [len(videos)] * len(rc)
+        videos.append(v)
+        frames.append(fr)
+        remapped += rc
+    return videos, frames, remapped, slab
+
+
+class _JpegFrames:
+    """Test windows read from JPEG frames: per packed batch, only the frames its clips read are decoded, into a
+    per-batch arena (jpeg.JpegSlabs); a rejected frame raises at the next batch or at the end of the call."""
+
+    def __init__(self, read_frames, sizes, device):
+        self.jpeg = JpegSlabs(read_frames, 1, sizes, device)
+        self.device = self.jpeg.decoder.device
+
+    def frame_size(self, v: int):
+        return self.jpeg.frame_size(v)
+
+    def batch(self, clips, owners):
+        videos, frames, remapped, slab = batch_slabs(clips, owners)
+        slabs = self.jpeg.decode(videos, frames)
+        return remapped, [slabs[k] for k in slab]
+
+    def finish(self) -> None:
+        self.jpeg.check()
+
+
+def _plan_clips(frames, total_frames: Sequence[int], videos: range, sampler: FinetuneClipSampler):
     """test.py's sliding windows of every video in `videos`: (per-video plans, flat clip list, owning video per clip)."""
     plans, owners = [], []
     for v in videos:
-        vid = store[v]
-        p = sampler.plan_test(int(total_frames[v]), vid.shape[2], vid.shape[1])
+        w, h = frames.frame_size(v)
+        p = sampler.plan_test(int(total_frames[v]), w, h)
         plans.append(p)
         owners += [v] * len(p)
     return plans, [c for p in plans for c in p], owners
 
 
-def _pack_videos(model, store: GpuVideoStore, plans, clips, owners, *, T: int, S: int, capacity: int, source: str,
+def _pack_videos(model, frames, plans, clips, owners, *, T: int, S: int, capacity: int, source: str,
                  width: int, finalize: Callable, assemble: Optional[Callable] = None) -> None:
     """Runs the clips of consecutive videos through one inference engine in full batches of `capacity` and averages,
     per video, the first `width` columns of the engine's `source` rows ("logits" or "feat") in clip order.
     `finalize(sums, fin)` consumes the sums of the videos whose last clip is in the batch (cstp_video_finalize)."""
     ops = _engine_mod.ops
-    device = store.device
+    device = frames.device
     eng = model.inference_engine(capacity, T, S, S, device)
     model._repack_if_changed(eng)
     assemble = assemble or GpuClipPipeline(T, S, device).assemble_clips
@@ -78,10 +134,12 @@ def _pack_videos(model, store: GpuVideoStore, plans, clips, owners, *, T: int, S
     sums = torch.zeros(len(plans), width, dtype=torch.float32, device=device)
     for b in range(tables.shape[0]):
         rows = range(b * capacity, min(len(clips), (b + 1) * capacity))
-        assemble([clips[i] for i in rows], [store[owners[i]] for i in rows], eng.x_static[:len(rows)])
+        batch, videos = frames.batch([clips[i] for i in rows], [owners[i] for i in rows])
+        assemble(batch, videos, eng.x_static[:len(rows)])
         eng.run(len(rows))
         ops.video_accumulate(getattr(eng, source), width, tables[b, 0], sums, rows=len(rows))
         finalize(sums, tables[b, 1])
+    frames.finish()
 
 
 @torch.no_grad()
@@ -99,19 +157,41 @@ def test_videos(model, store: GpuVideoStore, total_frames: Sequence[int], labels
     Returns {"top1", "top5": accuracies over all ranks' videos, "hits": (top-1, top-5) hit counts, "videos", "clips":
     totals over all ranks, "predictions": int64 [shard videos][5] top-5 classes of this rank's videos, "logits": fp32
     [shard videos][num_classes] mean logits (keep_logits) or None}."""
+    return _test_videos(model, _StoreFrames(store), total_frames, labels, sample_duration, sample_size, pb_rate, capacity,
+                        rank, world, keep_logits, assemble)
+
+
+@torch.no_grad()
+def test_videos_jpeg(model, read_frames: Callable[[int, Sequence[int]], List[bytes]], total_frames: Sequence[int],
+                     labels: Sequence[int], *, sizes: Optional[Sequence[Tuple[int, int]]] = None, device="cuda",
+                     sample_duration: int = 16, sample_size: int = 112, pb_rate: int = 4, capacity: int = 60,
+                     rank: int = 0, world: int = 1, keep_logits: bool = False) -> dict:
+    """`test_videos` fed from JPEG frames instead of a store: the same windows, packing, results and bits.
+
+    read_frames(video, frame_numbers) -> [bytes] returns the JPEG streams of those frames (1-based file numbers, as
+    `FrameDirReader` reads them).  Each batch of `capacity` clips reads and decodes only the frames its clips use, in one
+    call into a per-batch arena, so device memory holds one batch's frames, not the split's.  Frame sizes come from each
+    video's first frame (read once) or from `sizes[video] = (w, h)`.  A rejected frame raises ValueError naming the video
+    and the frame before the call returns."""
+    return _test_videos(model, _JpegFrames(read_frames, sizes, device), total_frames, labels, sample_duration,
+                        sample_size, pb_rate, capacity, rank, world, keep_logits, None)
+
+
+def _test_videos(model, frames, total_frames, labels, sample_duration, sample_size, pb_rate, capacity, rank, world,
+                 keep_logits, assemble) -> dict:
     model = getattr(model, "module", model)
     ops = _engine_mod.ops
     T, S, C = int(sample_duration), int(sample_size), model.num_classes
-    device = store.device
+    device = frames.device
     mine = shard(len(total_frames), rank, world)
-    plans, clips, owners = _plan_clips(store, total_frames, mine, FinetuneClipSampler(T, S, pb_rate))
+    plans, clips, owners = _plan_clips(frames, total_frames, mine, FinetuneClipSampler(T, S, pb_rate))
     nv = len(mine)
     topk = torch.zeros(nv, TOPK, dtype=torch.int64, device=device)
     mean = torch.zeros(nv, C, dtype=torch.float32, device=device) if keep_logits else None
     counts = torch.tensor([0, 0, nv, len(clips)], dtype=torch.int64, device=device)   # top-1 hits, top-5 hits, videos, clips
     if clips:
         y = torch.as_tensor([int(labels[v]) for v in mine], dtype=torch.int64).to(device)
-        _pack_videos(model, store, plans, clips, owners, T=T, S=S, capacity=capacity, source="logits", width=C,
+        _pack_videos(model, frames, plans, clips, owners, T=T, S=S, capacity=capacity, source="logits", width=C,
                      finalize=lambda sums, fin: ops.video_finalize(sums, fin, topk, y, mean, counts[:2]),
                      assemble=assemble)
     if world > 1:
@@ -136,18 +216,37 @@ def video_features(model, store: GpuVideoStore, total_frames: Sequence[int], *, 
 
     With world > 1 this rank extracts its contiguous shard and the shards are all-gathered over the default process
     group, so every rank returns all rows.  Returns fp32 [videos][512] on the store's device.  A split that does not fit
-    in device memory is extracted chunk by chunk (one call per range of videos) and concatenated."""
+    in device memory is extracted chunk by chunk (one call per range of videos) and concatenated, or with
+    video_features_jpeg."""
+    return _video_features(model, _StoreFrames(store), total_frames, sample_duration, sample_size, pb_rate, capacity,
+                           rank, world, assemble)
+
+
+@torch.no_grad()
+def video_features_jpeg(model, read_frames: Callable[[int, Sequence[int]], List[bytes]], total_frames: Sequence[int], *,
+                        sizes: Optional[Sequence[Tuple[int, int]]] = None, device="cuda", sample_duration: int = 16,
+                        sample_size: int = 112, pb_rate: int = 4, capacity: int = 60, rank: int = 0,
+                        world: int = 1) -> torch.Tensor:
+    """`video_features` fed from JPEG frames instead of a store, bit for bit the same features; `read_frames`, `sizes`
+    and the per-batch decoding are those of test_videos_jpeg.  Device memory holds one batch's frames, so a split of
+    any size is extracted in one call."""
+    return _video_features(model, _JpegFrames(read_frames, sizes, device), total_frames, sample_duration, sample_size,
+                           pb_rate, capacity, rank, world, None)
+
+
+def _video_features(model, frames, total_frames, sample_duration, sample_size, pb_rate, capacity, rank, world,
+                    assemble) -> torch.Tensor:
     model = getattr(model, "module", model)
     ops = _engine_mod.ops
     T, S = int(sample_duration), int(sample_size)
-    device = store.device
+    device = frames.device
     n = len(total_frames)
     mine = shard(n, rank, world)
-    plans, clips, owners = _plan_clips(store, total_frames, mine, FinetuneClipSampler(T, S, pb_rate))
+    plans, clips, owners = _plan_clips(frames, total_frames, mine, FinetuneClipSampler(T, S, pb_rate))
     feats = torch.zeros(len(mine), FEATURE_DIM, dtype=torch.float32, device=device)
     if clips:
         scratch = torch.zeros(len(mine), 1, dtype=torch.int64, device=device)      # finalize's top-k, unused
-        _pack_videos(model, store, plans, clips, owners, T=T, S=S, capacity=capacity, source="feat", width=FEATURE_DIM,
+        _pack_videos(model, frames, plans, clips, owners, T=T, S=S, capacity=capacity, source="feat", width=FEATURE_DIM,
                      finalize=lambda sums, fin: ops.video_finalize(sums, fin, scratch, None, feats, None),
                      assemble=assemble)
     if world == 1:
