@@ -161,6 +161,15 @@ def compile_view(view: ViewPlan, frame_base: int, W: int, H: int, S: int, video_
     return d, coef, y1 - y0
 
 
+def clip_layout(S: int, max_crop_h: int):
+    """(CTAs per (frame, view), shared-memory bytes per CTA) that `cstp_clip_assemble` launches for clips of side S whose
+    tallest crop has max_crop_h rows: 1 CTA while the crop rows and two S x S images fit, else a cluster pair.  Raises
+    CstpError, naming the crop height, when neither fits.  Host arithmetic only; needs no GPU."""
+    cluster, smem = C.c_int(), C.c_int()
+    L.check(L.load().cstp_clip_layout(int(S), int(max_crop_h), C.byref(cluster), C.byref(smem)))
+    return cluster.value, smem.value
+
+
 def collate_labels(plans: Sequence[SamplePlan], device=None):
     """default_collate of the per-sample label lists: [spa (B,), tem (B,), pb (B,), [rot1 (B,), rot2 (B,)]] int64
     (datasets.py:856-857, consumed at main_byol.py:45-49)."""

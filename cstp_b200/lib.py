@@ -142,7 +142,8 @@ class WgradHaloDesc(C.Structure):
     ]
 
 
-CSTP_CLIP_T = 16
+CSTP_CLIP_T = 64
+CSTP_CLIP_S = 224
 CSTP_CLIP_KMAX = 24
 
 
@@ -228,6 +229,7 @@ SIGNATURES = {
     "cstp_sgd_clip_step": (_i, [_vp, _vp, _vp, _i64, _f, _f, _f, _f, _i, _i, _vp, _vp, _vp]),
     "cstp_sgd_clip_step_dev": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "cstp_clip_assemble": (_i, [_vp, _i, _i, _i, _i, _vp]),
+    "cstp_clip_layout": (_i, [_i, _i, C.POINTER(_i), C.POINTER(_i)]),
     "cstp_video_accumulate": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _i, _vp]),
     "cstp_video_finalize": (_i, [_vp, _i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "cstp_l2_normalize_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),

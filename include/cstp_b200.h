@@ -434,7 +434,8 @@ int cstp_sgd_clip_step_dev(float* p, const float* g, float* mom, int64_t n, cons
  * frames resident in HBM into the two fp32 NCDHW clips the model consumes.  The arithmetic is Pillow's, restated in
  * integers (Q22 resampling taps, 16.16 affine walk, Q24 box blur, uint8 HSV), so the output equals the reference's
  * clips bit for bit. */
-#define CSTP_CLIP_T 16     /* frames per clip (opts.sample_duration) upper bound */
+#define CSTP_CLIP_T 64     /* frames per clip (opts.sample_duration) upper bound */
+#define CSTP_CLIP_S 224    /* clip side (opts.sample_size) upper bound */
 #define CSTP_CLIP_KMAX 24  /* resampling taps per output pixel upper bound (crop side <= 616 for a 112 output) */
 typedef struct {
   const uint8_t* video;  /* device: frame 0 of this sample's decoded video, uint8 [F][H][W][3] */
@@ -458,8 +459,15 @@ typedef struct {
   uint32_t blur_ww, blur_fw;
 } cstp_clip_view;
 /* views: DEVICE array of n_views descriptors; max_crop_h: largest (box[3]-box[1]) among them (sizes the shared-memory
- * staging of the horizontal pass; CSTP_EINVAL when it does not fit).  One CTA per (frame, view). */
+ * staging of the horizontal pass; CSTP_EINVAL when it does not fit).  8 <= S <= CSTP_CLIP_S, T <= CSTP_CLIP_T.
+ * One CTA per (frame, view) when the crop rows and two S x S images fit its shared memory, else a thread-block cluster
+ * of two CTAs per (frame, view) that splits every staged buffer by rows (see cstp_clip_layout). */
 int cstp_clip_assemble(const cstp_clip_view* views, int n_views, int T, int S, int max_crop_h, void* stream);
+/* The launch layout cstp_clip_assemble picks for (S, max_crop_h): *cluster = 1 (one CTA holds
+ * align16(max_crop_h * S * 3) + 2 * align16(S * S * 3) bytes) or 2 (each CTA of the pair holds
+ * align16(max(ceil(max_crop_h / 2), ceil(S / 2)) * S * 3) + align16(ceil(S / 2) * S * 3) bytes); *smem_bytes per CTA.
+ * CSTP_EINVAL, naming the crop height, when neither fits 226 KB.  Host only: needs no GPU. */
+int cstp_clip_layout(int S, int max_crop_h, int* cluster, int* smem_bytes);
 
 /* ---- JPEG decoding (csrc/jpeg_decode.cu) -------------------------------------------------------------------
  * Baseline / extended-sequential Huffman JPEG (SOF0 / SOF1, 8-bit samples, one interleaved scan; grayscale or YCbCr
