@@ -496,6 +496,76 @@ __global__ void __launch_bounds__(256) sgd_step_kernel(float* __restrict__ p, co
   }
 }
 
+// ------------------------------------------------------------------------------------------- clip + Adam / AdamW
+// clip_grad_norm_ (main_byol.py:88-90): every block reduces the kNormBlocks partial sums of squares in the same fixed
+// order (in double) and derives the clip coefficient max_norm / (norm + 1e-6), capped at 1; block 0 reports both.
+// Kept operation for operation equal to the prologue of sgd_step_kernel: both optimisers clip by the same norm.
+__device__ __forceinline__ float clip_coefficient(const float* __restrict__ partials, int do_clip, float max_norm,
+                                                  float* __restrict__ norm_out) {
+  __shared__ double red[256];
+  double acc = 0.0;
+  for (int i = threadIdx.x; i < kNormBlocks; i += blockDim.x) acc += static_cast<double>(partials[i]);
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int s = 128; s > 0; s >>= 1) {
+    if (threadIdx.x < s) red[threadIdx.x] += red[threadIdx.x + s];
+    __syncthreads();
+  }
+  const float total_norm = static_cast<float>(sqrt(red[0]));
+  float coef = 1.f;
+  if (do_clip) {
+    coef = max_norm / (total_norm + 1e-6f);
+    coef = coef > 1.f ? 1.f : coef;
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0 && norm_out != nullptr) {
+    norm_out[0] = total_norm;
+    norm_out[1] = coef;
+  }
+  return coef;
+}
+
+// torch.optim.Adam / AdamW (_single_tensor_adam) per element, each operation rounded on its own so that a float32
+// restatement reproduces the bits (include/cstp_b200.h has the formula).
+__device__ __forceinline__ void adam_element(float& w, float gr, float& m, float& v, const cstp_adam_hyper& h,
+                                             float coef) {
+  gr = __fmul_rn(gr, coef);
+  w = __fmul_rn(w, h.decay);
+  gr = __fadd_rn(gr, __fmul_rn(h.l2, w));
+  m = __fadd_rn(m, __fmul_rn(__fsub_rn(gr, m), h.one_minus_beta1));
+  v = __fadd_rn(__fmul_rn(v, h.beta2), __fmul_rn(__fmul_rn(h.one_minus_beta2, gr), gr));
+  const float den = __fadd_rn(__fdiv_rn(__fsqrt_rn(v), h.bc2_sqrt), h.eps);
+  w = __fsub_rn(w, __fdiv_rn(__fmul_rn(h.step_size, m), den));
+}
+
+// One float4 of each buffer per thread and iteration (4 loads, 3 stores); block 0 also takes the n % 4 tail.
+__global__ void __launch_bounds__(256) adam_step_kernel(float4* __restrict__ p, const float4* __restrict__ g,
+                                                        float4* __restrict__ m, float4* __restrict__ v, long long n4,
+                                                        int tail, cstp_adam_hyper h, const float* __restrict__ partials,
+                                                        float* __restrict__ norm_out,
+                                                        const cstp_adam_hyper* __restrict__ hyper) {
+  if (hyper != nullptr) h = *hyper;
+  const float coef = clip_coefficient(partials, h.do_clip != 0.f, h.max_norm, norm_out);
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n4;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    float4 w = p[i], a = m[i], b = v[i];
+    const float4 gr = g[i];
+    adam_element(w.x, gr.x, a.x, b.x, h, coef);
+    adam_element(w.y, gr.y, a.y, b.y, h, coef);
+    adam_element(w.z, gr.z, a.z, b.z, h, coef);
+    adam_element(w.w, gr.w, a.w, b.w, h, coef);
+    p[i] = w;
+    m[i] = a;
+    v[i] = b;
+  }
+  if (blockIdx.x == 0 && static_cast<int>(threadIdx.x) < tail) {
+    const long long i = n4 * 4 + threadIdx.x;
+    float* pt = reinterpret_cast<float*>(p);
+    float* mt = reinterpret_cast<float*>(m);
+    float* vt = reinterpret_cast<float*>(v);
+    adam_element(pt[i], reinterpret_cast<const float*>(g)[i], mt[i], vt[i], h, coef);
+  }
+}
+
 int ntxent_tensor_path(const float* zn, int rows, int d, float temperature, bool backward, float* row_loss, float* ws,
                        float** dzn_out, cudaStream_t stream);
 
@@ -657,4 +727,31 @@ extern "C" int cstp_sgd_clip_step_dev(float* p, const float* g, float* mom, int6
   sgd_step_kernel<<<grid_cap(n, 256), 256, 0, ST(stream)>>>(p, g, mom, n, 0.f, 0.f, 0.f, 0.f, 0, 0, workspace, norm_out, hyper);
   CSTP_LAUNCHED();
   return CSTP_OK;
+}
+
+static int adam_launch(float* p, const float* g, float* m, float* v, int64_t n, const cstp_adam_hyper& h,
+                       const cstp_adam_hyper* hyper_dev, float* norm_out, float* workspace, void* stream) {
+  CSTP_REQUIRE(p && g && m && v && workspace && n > 0);
+  for (const void* ptr : {static_cast<const void*>(p), static_cast<const void*>(g), static_cast<const void*>(m),
+                          static_cast<const void*>(v)})
+    CSTP_REQUIRE(reinterpret_cast<uintptr_t>(ptr) % 16 == 0);
+  sumsq_partial_kernel<<<kNormBlocks, 256, 0, ST(stream)>>>(g, n, workspace);
+  CSTP_LAUNCHED();
+  const long long n4 = n / 4;
+  adam_step_kernel<<<grid_cap(n4 > 0 ? n4 : 1, 256), 256, 0, ST(stream)>>>(
+      reinterpret_cast<float4*>(p), reinterpret_cast<const float4*>(g), reinterpret_cast<float4*>(m),
+      reinterpret_cast<float4*>(v), n4, static_cast<int>(n % 4), h, workspace, norm_out, hyper_dev);
+  CSTP_LAUNCHED();
+  return CSTP_OK;
+}
+
+extern "C" int cstp_adam_clip_step(float* p, const float* g, float* m, float* v, int64_t n, cstp_adam_hyper hyper,
+                                   float* norm_out, float* workspace, void* stream) {
+  return adam_launch(p, g, m, v, n, hyper, nullptr, norm_out, workspace, stream);
+}
+
+extern "C" int cstp_adam_clip_step_dev(float* p, const float* g, float* m, float* v, int64_t n,
+                                       const cstp_adam_hyper* hyper, float* norm_out, float* workspace, void* stream) {
+  CSTP_REQUIRE(hyper != nullptr);
+  return adam_launch(p, g, m, v, n, cstp_adam_hyper{}, hyper, norm_out, workspace, stream);
 }

@@ -6,11 +6,12 @@ models/pace/r21d_byol.py:357-382) into three launch programs of hand-written sm_
 
   forward   online_net(view1|view2) -> predictor -> EMA -> target_net(view1|view2) -> BYOL loss -> pretext heads
   backward  heads / predictor / projector / backbone (BN-bwd, wgrad, dgrad per layer) into ONE flat fp32 grad buffer
-  update    (grad all-reduce) -> global-norm clip + SGD momentum on the flat buffers -> bf16 weight re-pack
+  update    (grad all-reduce) -> global-norm clip + SGD momentum (or Adam / AdamW) on the flat buffers -> bf16 weight re-pack
 
 Data layout in HBM
   * parameters: two flat fp32 buffers (trainable = online_net + predictor + 4 pretext heads; target_net), every
-    tensor in a 16-float aligned slot; gradients and SGD momentum mirror the trainable buffer.  The nn.Parameters of
+    tensor in a 16-float aligned slot; gradients and SGD momentum mirror the trainable buffer (and so do Adam's exp_avg /
+    exp_avg_sq, allocated when Adam first runs).  The nn.Parameters of
     the drop-in module are views into these buffers (reference shapes, state_dict compatible).
   * activations: bf16 NDHWC, channels padded to 16, the two views concatenated along N (2B samples) and kept as two
     BatchNorm statistics groups (the reference runs the views one after the other, SURVEY.md 0.3).
@@ -62,6 +63,17 @@ USE_GRAPH = os.environ.get("CSTP_GRAPH", "1") == "1"
 # Storage type of activations, activation gradients and packed weights.  The CUDA kernels only implement bf16; the
 # CPU emulator in tests/ also runs the orchestration in fp32 to separate wiring errors from rounding.
 ACT_DTYPE = torch.bfloat16
+
+
+OPTIMIZERS = ("sgd", "adam", "adamw")
+
+
+def adam_scalars(step: int, lr, betas, eps, weight_decay, decoupled: bool, max_norm=0.0, clip=False) -> tuple:
+    """The cstp_adam_hyper scalars (include/cstp_b200.h, in field order) of Adam / AdamW step `step` (1-based), computed in
+    double as torch.optim.Adam(W) computes them (_single_tensor_adam); the kernel receives them rounded to fp32."""
+    b1, b2, lr, wd = float(betas[0]), float(betas[1]), float(lr), float(weight_decay)
+    return (lr / (1 - b1 ** step), (1 - b2 ** step) ** 0.5, 1 - b1, b2, 1 - b2, float(eps), 0.0 if decoupled else wd,
+            1 - lr * wd if decoupled else 1.0, float(max_norm), 1.0 if clip else 0.0)
 
 
 def intermed_channels(cin: int, cout: int, k: tuple[int, int, int]) -> int:
@@ -249,7 +261,10 @@ class StepEngine:
         f32 = dict(device=self.device, dtype=torch.float32)
 
         self._make_stores()
-        self.first_step = True
+        self.first_step = True       # no optimiser state yet (SGD momentum / Adam moments)
+        self.optim_kind = "sgd"      # the optimiser the state belongs to (OPTIMIZERS)
+        self.adam_step = 0           # Adam / AdamW steps taken (torch's per-parameter `step`)
+        self.exp_avg = self.exp_avg_sq = self.adam_hyper = None
 
         # ---- scratch shared by all layers
         self._g_numel = 0            # bf16 d(raw) scratch, sized while building
@@ -855,11 +870,49 @@ class StepEngine:
                     main.wait_event(e)
         return bucketed
 
-    def optimizer_step(self, lr, momentum=0.9, wd=5e-4, max_norm=18.0, clip=True):
-        """clip_grad_norm_ + SGD.step (main_byol.py:88-91,229-232) on the flat buffers, then re-pack the bf16 weights."""
+    def select_optimizer(self, kind: str) -> None:
+        """Binds the optimiser `kind` (OPTIMIZERS) for the next step.  Adam's state buffers (exp_avg / exp_avg_sq mirrors
+        of the trainable buffer) are allocated when Adam first runs, so an SGD run holds nothing extra.  Optimiser state
+        belongs to one kind: asking for another while it exists raises ValueError."""
+        if kind not in OPTIMIZERS:
+            raise ValueError(f"optimizer {kind!r}: expected one of {OPTIMIZERS}")
+        if kind != self.optim_kind and not self.first_step:
+            raise ValueError(f"the engine holds {self.optim_kind} optimiser state; it cannot continue as {kind}")
+        self.optim_kind = kind
+        if kind == "sgd":
+            return
+        if self.exp_avg is None:
+            self.exp_avg, self.exp_avg_sq = self.train.like(), self.train.like()
+            self.adam_hyper = torch.zeros(len(ops.L.AdamHyper._fields_), device=self.device, dtype=torch.float32)
+        elif self.first_step:
+            self.exp_avg.zero_()
+            self.exp_avg_sq.zero_()
+        if self.first_step:
+            self.adam_step = 0
+
+    def _next_adam(self, lr, betas, eps, wd, max_norm, clip) -> tuple:
+        self.adam_step += 1
+        return adam_scalars(self.adam_step, lr, betas, eps, wd, self.optim_kind == "adamw", max_norm, clip)
+
+    def take_optimizer_state(self, other: "StepEngine") -> None:
+        """Continues the optimiser of `other`, an engine of another batch geometry over the same parameter layout that is
+        about to be dropped (its Adam moments are taken over, not copied)."""
+        self.mom.copy_(other.mom)
+        self.first_step, self.optim_kind, self.adam_step = other.first_step, other.optim_kind, other.adam_step
+        self.exp_avg, self.exp_avg_sq, self.adam_hyper = other.exp_avg, other.exp_avg_sq, other.adam_hyper
+
+    def optimizer_step(self, lr, momentum=0.9, wd=5e-4, max_norm=18.0, clip=True, optimizer="sgd", betas=(0.9, 0.999),
+                       eps=1e-8):
+        """clip_grad_norm_ + SGD.step (main_byol.py:88-91,229-232), or + Adam / AdamW.step (`momentum` unused), on the flat
+        buffers, then re-pack the bf16 weights."""
+        self.select_optimizer(optimizer)
         n = self.train.numel
-        ops.sgd_clip_step(self.train.data[:n], self.grad[:n], self.mom[:n], lr, momentum, wd, max_norm, clip,
-                          self.first_step, self.norm_out, self.sgd_ws)
+        if optimizer == "sgd":
+            ops.sgd_clip_step(self.train.data[:n], self.grad[:n], self.mom[:n], lr, momentum, wd, max_norm, clip,
+                              self.first_step, self.norm_out, self.sgd_ws)
+        else:
+            ops.adam_clip_step(self.train.data[:n], self.grad[:n], self.exp_avg[:n], self.exp_avg_sq[:n],
+                               self._next_adam(lr, betas, eps, wd, max_norm, clip), self.norm_out, self.sgd_ws)
         self.first_step = False
         self.pack_online()
 
@@ -871,6 +924,12 @@ class StepEngine:
             self.hyper[:6].copy_(torch.tensor(h, dtype=torch.float32), non_blocking=False)
             self._hyper_host = h
 
+    def set_adam_hyper(self, lr, betas, eps, wd, max_norm, clip) -> None:
+        """Writes the scalars of the next Adam / AdamW step into device memory, in stream order ahead of the step (through
+        pinned memory, which torch's host allocator keeps until the copy has run: the host does not wait)."""
+        h = torch.tensor(self._next_adam(lr, betas, eps, wd, max_norm, clip), dtype=torch.float32)
+        self.adam_hyper.copy_(h.pin_memory(), non_blocking=True)
+
     def _step_body(self, grad_sync, after):
         """forward (behind the input pass) -> pretext losses -> backward (+ gradient all-reduce) -> optimiser -> re-pack,
         on engine-owned buffers only: the program graphed_step captures."""
@@ -881,22 +940,32 @@ class StepEngine:
         elif grad_sync is not None:
             grad_sync(self.grad)
         n = self.train.numel
-        ops.sgd_clip_step_dev(self.train.data[:n], self.grad[:n], self.mom[:n], self.hyper, self.norm_out, self.sgd_ws)
+        if self.optim_kind == "sgd":
+            ops.sgd_clip_step_dev(self.train.data[:n], self.grad[:n], self.mom[:n], self.hyper, self.norm_out, self.sgd_ws)
+        else:
+            ops.adam_clip_step_dev(self.train.data[:n], self.grad[:n], self.exp_avg[:n], self.exp_avg_sq[:n],
+                                   self.adam_hyper, self.norm_out, self.sgd_ws)
         self.pack_online()
         if after is not None:
             after()
 
-    def graphed_step(self, x1, x2, labels, lr, momentum, wd, max_norm, clip, grad_sync=None, after=None):
+    def graphed_step(self, x1, x2, labels, lr, momentum, wd, max_norm, clip, grad_sync=None, after=None, optimizer="sgd",
+                     betas=(0.9, 0.999), eps=1e-8):
         """One pretraining step with everything behind the input pass replayed from a CUDA graph.  The first call runs the
         program eagerly (one-time kernel attributes, NCCL / peer-memory channel set-up), the second captures it; inputs
         (clips -> packed stem rows, labels, hyper-parameters) are written into static buffers in front of the graph.
         `after` (device-side bookkeeping of the caller, e.g. num_batches_tracked) is part of the program and must be the
-        same callable for the lifetime of a capture; drop_graph() forgets the capture."""
+        same callable for the lifetime of a capture; drop_graph() forgets the capture.  Each optimiser kind is a capture of
+        its own (Adam / AdamW: the step-dependent scalars are rewritten in device memory before every replay)."""
+        self.select_optimizer(optimizer)
         self.load_clips(x1, x2)
         for dst, src in zip(self.labels_static, labels):
             dst.copy_(src)
-        self.set_hyper(lr, momentum, wd, max_norm, clip)
-        key = id(grad_sync)
+        if optimizer == "sgd":
+            self.set_hyper(lr, momentum, wd, max_norm, clip)
+        else:
+            self.set_adam_hyper(lr, betas, eps, wd, max_norm, clip)
+        key = (id(grad_sync), optimizer)
         if self._graph is not None and self._graph_key == key:
             self._graph.replay()
             ops.note_replayed(self._graph_launches)

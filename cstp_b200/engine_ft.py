@@ -184,16 +184,25 @@ class FinetuneEngine(StepEngine):
                 runs.append([off, n])
         return [(o, n) for o, n in runs]
 
-    def optimizer_step(self, lr, momentum=0.9, wd=1e-3, max_norm=0.0, clip=False, ranges=None):
-        """SGD.step of main_ft_mp.py:117-121,212 (no gradient clipping in the finetune driver).  `ranges` restricts the
-        update to the trainable runs of the flat buffer (see trainable_ranges); None updates every parameter."""
+    def optimizer_step(self, lr, momentum=0.9, wd=1e-3, max_norm=0.0, clip=False, ranges=None, optimizer="sgd",
+                       betas=(0.9, 0.999), eps=1e-8):
+        """SGD.step of main_ft_mp.py:117-121,212 (no gradient clipping in the finetune driver), or Adam / AdamW.step.
+        `ranges` restricts the update to the trainable runs of the flat buffer (see trainable_ranges): the other
+        parameters get no update, and their optimiser state stays zero; None updates every parameter."""
         if ranges is None:
-            return super().optimizer_step(lr, momentum, wd, max_norm, clip)
+            return super().optimizer_step(lr, momentum, wd, max_norm, clip, optimizer, betas, eps)
         if clip:
             raise E.ops.L.CstpError("gradient clipping over a partial parameter set is not part of the finetune path")
-        for off, n in ranges:
-            E.ops.sgd_clip_step(self.train.data[off:off + n], self.grad[off:off + n], self.mom[off:off + n], lr, momentum, wd,
-                                0.0, False, self.first_step, self.norm_out, self.sgd_ws)
+        self.select_optimizer(optimizer)
+        if optimizer == "sgd":
+            for off, n in ranges:
+                E.ops.sgd_clip_step(self.train.data[off:off + n], self.grad[off:off + n], self.mom[off:off + n], lr,
+                                    momentum, wd, 0.0, False, self.first_step, self.norm_out, self.sgd_ws)
+        else:
+            h = self._next_adam(lr, betas, eps, wd, 0.0, False)
+            for off, n in ranges:
+                E.ops.adam_clip_step(self.train.data[off:off + n], self.grad[off:off + n], self.exp_avg[off:off + n],
+                                     self.exp_avg_sq[off:off + n], h, self.norm_out, self.sgd_ws)
         self.first_step = False
         self.pack_online()
 

@@ -177,6 +177,12 @@ class JpegImage(C.Structure):
 
 CSTP_JPEG_UNSUPPORTED, CSTP_JPEG_MALFORMED, CSTP_JPEG_SIZE = 1, 2, 3
 
+
+class AdamHyper(C.Structure):
+    """cstp_adam_hyper: the scalars of one Adam / AdamW step (include/cstp_b200.h); ten floats, also as a device vector."""
+    _fields_ = [(n, C.c_float) for n in ("step_size", "bc2_sqrt", "one_minus_beta1", "beta2", "one_minus_beta2", "eps",
+                                         "l2", "decay", "max_norm", "do_clip")]
+
 _vp, _i, _i64, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
 
 # name -> (restype, argtypes); the single source of truth for the symbols include/cstp_b200.h declares.
@@ -228,6 +234,8 @@ SIGNATURES = {
     "cstp_ema_update": (_i, [_vp, _vp, _i64, _f, _f, _vp]),
     "cstp_sgd_clip_step": (_i, [_vp, _vp, _vp, _i64, _f, _f, _f, _f, _i, _i, _vp, _vp, _vp]),
     "cstp_sgd_clip_step_dev": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "cstp_adam_clip_step": (_i, [_vp, _vp, _vp, _vp, _i64, AdamHyper, _vp, _vp, _vp]),
+    "cstp_adam_clip_step_dev": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "cstp_clip_assemble": (_i, [_vp, _i, _i, _i, _i, _vp]),
     "cstp_clip_layout": (_i, [_i, _i, C.POINTER(_i), C.POINTER(_i)]),
     "cstp_video_accumulate": (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _i, _vp]),

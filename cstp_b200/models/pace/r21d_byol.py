@@ -236,8 +236,7 @@ class R21DBYOL(nn.Module):
             new = _engine_mod.StepEngine(B, T, H, W, device=x1.device, momentum_ema=self.momentum,
                                          **getattr(self, "engine_options", {}))
             if eng is not None:      # keep optimiser-side state across a batch-geometry change
-                new.mom.copy_(eng.mom)
-                new.first_step = eng.first_step
+                new.take_optimizer_state(eng)
             eng = self._engine = new
             self._engine_key = key
             self._alias_ptr = None
@@ -285,8 +284,7 @@ class R21DBYOL(nn.Module):
             new = engine_ft.FinetuneEngine(B, T, H, W, device=x.device, num_classes=self.num_classes, cls_bn=True,
                                            backbone_grads=key[-1], **getattr(self, "engine_options", {}))
             if eng is not None:
-                new.mom.copy_(eng.mom)
-                new.first_step = eng.first_step
+                new.take_optimizer_state(eng)
             self.free_inference_engines()        # they read the stores the parameters are about to leave
             eng = self._engine = new
             self._engine_key = key
@@ -410,10 +408,13 @@ class R21DBYOL(nn.Module):
         return eng.logits[:n, :self.num_classes].clone()
 
     @torch.no_grad()
-    def finetune_step(self, x, labels, lr=0.025, momentum=0.9, weight_decay=1e-3, grad_sync=None):
+    def finetune_step(self, x, labels, lr=0.025, momentum=0.9, weight_decay=1e-3, grad_sync=None, optimizer="sgd",
+                      betas=(0.9, 0.999), eps=1e-8):
         """One fused finetune step (main_ft_mp.py:196-214: forward, CrossEntropyLoss, backward, SGD.step -- no gradient
-        clipping in the finetune driver).  Returns the device scalar loss without synchronising."""
+        clipping in the finetune driver).  optimizer="adam" / "adamw" steps torch.optim.Adam / AdamW(lr, betas, eps,
+        weight_decay) instead, and `momentum` is unused.  Returns the device scalar loss without synchronising."""
         eng = self._bind_ft(x)
+        eng.select_optimizer(optimizer)          # an invalid or conflicting kind raises before anything runs
         eng.eval_mode = False
         eng.forward(x.contiguous(), repack=self._dirty)
         self._dirty = False
@@ -427,7 +428,7 @@ class R21DBYOL(nn.Module):
         if frozen != getattr(self, "_ft_frozen", None) or getattr(self, "_ft_ranges_eng", None) is not eng:
             self._ft_frozen, self._ft_ranges_eng = frozen, eng
             self._ft_ranges = eng.trainable_ranges(frozen) if frozen else None
-        eng.optimizer_step(lr, momentum, weight_decay, ranges=self._ft_ranges)
+        eng.optimizer_step(lr, momentum, weight_decay, ranges=self._ft_ranges, optimizer=optimizer, betas=betas, eps=eps)
         self._nbt += self._nbt_inc
         self._wgen += 1                          # the kernel updated the weights: other engines must re-pack
         eng._packed_key = (eng.train.data._version, self._wgen)       # optimizer_step re-packed this one
@@ -471,13 +472,15 @@ class R21DBYOL(nn.Module):
     # ------------------------------------------------------------------------------------------ fused fast path
     @torch.no_grad()
     def train_step(self, x1, x2, labels, loss_weight=(0.1, 1, 1, 1, 1), lr=0.03, momentum=0.9, weight_decay=5e-4,
-                   clip_grad_norm=18.0, grad_sync=None):
-        """One full pretraining step (main_byol.py:60-91) as a single launch program.
+                   clip_grad_norm=18.0, grad_sync=None, optimizer="sgd", betas=(0.9, 0.999), eps=1e-8):
+        """One full pretraining step (main_byol.py:60-91) as a single launch program.  optimizer="adam" / "adamw" steps
+        torch.optim.Adam / AdamW(lr, betas, eps, weight_decay) after the same gradient clipping; `momentum` is then unused.
 
         labels = (spa, tem, pb, rot1, rot2) int64 device tensors.  `grad_sync(flat_grad)` is called between backward
         and the optimiser (data-parallel all-reduce).  Returns the engine's device loss vector
         [ce_spa, ce_tem, ce_pb1, ce_pb2, ce_rot1, ce_rot2, weighted CE sum, loss_byol] without synchronising."""
         eng = self._bind(x1)
+        eng.select_optimizer(optimizer)          # an invalid or conflicting kind raises before anything runs
         if tuple(loss_weight) != getattr(self, "_lw", None):
             eng.set_loss_weight(loss_weight)
             self._lw = tuple(loss_weight)
@@ -487,7 +490,7 @@ class R21DBYOL(nn.Module):
         if eng.use_graph and eng._prof is None:
             # everything behind the input pass replayed from a CUDA graph (engine.graphed_step)
             eng.graphed_step(x1, x2, labels, lr, momentum, weight_decay, clip_grad_norm or 0.0, bool(clip_grad_norm),
-                             grad_sync, self._bump_nbt)
+                             grad_sync, self._bump_nbt, optimizer, betas, eps)
             return eng.losses
         eng.forward(x1, x2)
         eng.pretext_losses(labels)
@@ -495,6 +498,6 @@ class R21DBYOL(nn.Module):
             grad_sync.finish()                   # the all-reduce ran in buckets beside the backward pass
         elif grad_sync is not None:
             grad_sync(eng.grad)
-        eng.optimizer_step(lr, momentum, weight_decay, clip_grad_norm or 0.0, bool(clip_grad_norm))
+        eng.optimizer_step(lr, momentum, weight_decay, clip_grad_norm or 0.0, bool(clip_grad_norm), optimizer, betas, eps)
         self._nbt += self._nbt_inc
         return eng.losses

@@ -1170,6 +1170,38 @@ def sgd_clip_step_dev(p, g, mom, hyper, norm_out, workspace) -> None:
                                             _ptr(workspace), _stream()))
 
 
+ADAM_HYPER_FLOATS = len(L.AdamHyper._fields_)
+NORM_PARTIALS = 1024                 # workspace floats of the clip-norm reduction (kNormBlocks, csrc/loss_optim.cu)
+
+
+def _check_adam(p, g, m, v, norm_out, workspace, hyper=None) -> None:
+    _require_cuda(p, g, m, v, norm_out, workspace, hyper)
+    flat = (p, g, m, v, norm_out, workspace) + (() if hyper is None else (hyper,))
+    if any(t.dtype != torch.float32 or not t.is_contiguous() for t in flat):
+        raise L.CstpError("adam_clip_step: every buffer must be contiguous fp32")
+    if len({p.numel(), g.numel(), m.numel(), v.numel()}) != 1 or p.numel() == 0:
+        raise L.CstpError(f"adam_clip_step: p, g, m, v need one non-zero length, got "
+                          f"{[t.numel() for t in (p, g, m, v)]}")
+    if norm_out.numel() < 2 or workspace.numel() < NORM_PARTIALS or (hyper is not None and hyper.numel() < ADAM_HYPER_FLOATS):
+        raise L.CstpError(f"adam_clip_step: norm_out needs 2 floats, workspace {NORM_PARTIALS}, hyper {ADAM_HYPER_FLOATS}")
+
+
+def adam_clip_step(p, g, m, v, hyper: tuple, norm_out, workspace) -> None:
+    """clip_grad_norm_ + one Adam / AdamW step on flat fp32 buffers (p, g, exp_avg m, exp_avg_sq v); `hyper` holds the
+    ten cstp_adam_hyper scalars in field order (engine.adam_scalars computes them)."""
+    _check_adam(p, g, m, v, norm_out, workspace)
+    L.check(L.load().cstp_adam_clip_step(_ptr(p), _ptr(g), _ptr(m), _ptr(v), p.numel(), L.AdamHyper(*map(float, hyper)),
+                                         _ptr(norm_out), _ptr(workspace), _stream()))
+
+
+def adam_clip_step_dev(p, g, m, v, hyper, norm_out, workspace) -> None:
+    """adam_clip_step with the scalars read from the device vector `hyper` (fp32 [10]) at run time: the form a captured
+    CUDA graph replays while the host rewrites the step-dependent scalars before every replay."""
+    _check_adam(p, g, m, v, norm_out, workspace, hyper)
+    L.check(L.load().cstp_adam_clip_step_dev(_ptr(p), _ptr(g), _ptr(m), _ptr(v), p.numel(), _ptr(hyper), _ptr(norm_out),
+                                             _ptr(workspace), _stream()))
+
+
 def kernel_name(plan) -> str:
     """CUDA kernel a plan object launches (for profiles and the bench roofline)."""
     inner = getattr(plan, "plan", plan)          # WgradSpec wraps its plan

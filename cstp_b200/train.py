@@ -36,14 +36,18 @@ def unwrap(model):
 
 
 def optimizer_state_dict(model, lr: float = 0.03, momentum: float = 0.9, weight_decay: float = 5e-4,
-                         initial_lr: float | None = None) -> dict:
+                         initial_lr: float | None = None, betas=(0.9, 0.999), eps: float = 1e-8) -> dict:
     """torch.optim.SGD state dict of the engine's fused optimiser: momentum buffers addressed by the position of each
     parameter in model.parameters() (frozen target_net entries keep their indices and have no state) and ONE complete
     parameter group -- SGD.load_state_dict replaces the live groups by the saved ones, so every hyper-parameter key of
     torch's SGD has to be there for the reference's `optimizer.load_state_dict(...)` + `optimizer.step()` +
-    `CosineAnnealingWarmupRestarts(optimizer, ...)` to work on it (main_byol.py:138,243-258)."""
+    `CosineAnnealingWarmupRestarts(optimizer, ...)` to work on it (main_byol.py:138,243-258).
+    When the engine runs Adam / AdamW, the state dict of torch.optim.Adam / AdamW(lr, betas, eps, weight_decay) instead
+    (see _adam_state_dict); `momentum` is then unused."""
     model = unwrap(model)
     eng = model._engine
+    if eng.optim_kind != "sgd":
+        return _adam_state_dict(model, lr, weight_decay, initial_lr, betas, eps)
     names = [n for n, _ in model.named_parameters()]
     state = {}
     if not eng.first_step:
@@ -56,12 +60,40 @@ def optimizer_state_dict(model, lr: float = 0.03, momentum: float = 0.9, weight_
     return {"state": state, "param_groups": [group]}
 
 
-def load_optimizer_state_dict(model, sd: dict) -> None:
+def _adam_state_dict(model, lr, weight_decay, initial_lr, betas, eps) -> dict:
+    """torch.optim.Adam / AdamW state dict of the engine's fused Adam: {"step", "exp_avg", "exp_avg_sq"} per parameter
+    that takes part in the update, indexed by position in model.parameters() (target_net and parameters frozen with
+    requires_grad = False have no state, as torch gives them none), and ONE parameter group whose keys are those the
+    installed torch writes (taken from a throw-away optimiser, so they follow the torch version) plus `initial_lr`."""
+    eng = model._engine
+    state = {}
+    if not eng.first_step:
+        for i, (n, p) in enumerate(model.named_parameters()):
+            if n in eng.train.slots and p.requires_grad:
+                state[i] = {"step": torch.tensor(float(eng.adam_step)),
+                            "exp_avg": eng.train.view(n, eng.exp_avg).detach().clone().cpu(),
+                            "exp_avg_sq": eng.train.view(n, eng.exp_avg_sq).detach().clone().cpu()}
+    cls = torch.optim.AdamW if eng.optim_kind == "adamw" else torch.optim.Adam
+    group = cls([torch.zeros(1)], lr=float(lr), betas=tuple(float(b) for b in betas), eps=float(eps),
+                weight_decay=float(weight_decay)).state_dict()["param_groups"][0]
+    group.update(initial_lr=float(lr if initial_lr is None else initial_lr),
+                 params=list(range(sum(1 for _ in model.parameters()))))
+    return {"state": state, "param_groups": [group]}
+
+
+def load_optimizer_state_dict(model, sd: dict, optimizer: str | None = None) -> None:
     """Momentum buffers of an `optim.SGD.state_dict()` (ours or one the reference wrote, main_byol.py:138) -> the
     engine's flat momentum buffer.  Hyper-parameters are not taken from the file: the reference re-creates them from
-    `opts` on resume as well (main_byol.py:229-232 builds the optimizer before :243-244 loads the state)."""
+    `opts` on resume as well (main_byol.py:229-232 builds the optimizer before :243-244 loads the state).
+    An `optim.Adam` / `AdamW` state dict (entries with exp_avg / exp_avg_sq / step) restores the engine's Adam moments and
+    step count instead.  Whether it continues as "adam" or "adamw" is `optimizer` when given, else the group's
+    `decoupled_weight_decay` flag (written by the torch versions that have it), else "adam"."""
     model = unwrap(model)
     eng = model._engine
+    if any("exp_avg" in st for st in sd.get("state", {}).values()):
+        return _load_adam_state(model, sd, optimizer)
+    if optimizer not in (None, "sgd") and any("momentum_buffer" in st for st in sd.get("state", {}).values()):
+        raise ValueError(f"an SGD state dict cannot continue as {optimizer}")
     names = [n for n, _ in model.named_parameters()]
     loaded = False
     for i, st in sd.get("state", {}).items():
@@ -70,38 +102,66 @@ def load_optimizer_state_dict(model, sd: dict) -> None:
             eng.train.view(names[int(i)], eng.mom).copy_(buf)
             loaded = True
     eng.first_step = not loaded
+    if loaded:
+        eng.optim_kind = "sgd"
+
+
+def _load_adam_state(model, sd: dict, optimizer: str | None) -> None:
+    eng = model._engine
+    if optimizer is None:
+        optimizer = "adamw" if sd["param_groups"][0].get("decoupled_weight_decay") else "adam"
+    if optimizer not in ("adam", "adamw"):
+        raise ValueError(f"an Adam state dict cannot continue as {optimizer}")
+    entries = {int(i): st for i, st in sd["state"].items() if "exp_avg" in st}
+    steps = {float(st["step"]) for st in entries.values()}
+    if len(steps) != 1:
+        raise ValueError(f"the fused Adam step keeps one step count for every parameter; the state dict has {sorted(steps)}")
+    eng.first_step = True                        # fresh, zeroed moments of the requested kind, then the file's
+    eng.select_optimizer(optimizer)
+    names = [n for n, _ in model.named_parameters()]
+    for i, st in entries.items():
+        if names[i] in eng.train.slots:
+            eng.train.view(names[i], eng.exp_avg).copy_(st["exp_avg"])
+            eng.train.view(names[i], eng.exp_avg_sq).copy_(st["exp_avg_sq"])
+    eng.adam_step = int(steps.pop())
+    eng.first_step = False
 
 
 def save_checkpoint(path: str, model, epoch: int, arch: str, ddp_prefix: bool = True, lr: float = 0.03,
-                    momentum: float = 0.9, weight_decay: float = 5e-4, initial_lr: float | None = None) -> None:
+                    momentum: float = 0.9, weight_decay: float = 5e-4, initial_lr: float | None = None,
+                    betas=(0.9, 0.999), eps: float = 1e-8) -> None:
     """main_byol.py:132-140.  Keys carry the `module.` prefix of the DDP-wrapped model the reference saves (once: a model
-    that is already wrapped contributes it itself)."""
+    that is already wrapped contributes it itself).  The optimizer entry is the SGD or Adam / AdamW state dict of
+    whichever optimiser the engine runs (optimizer_state_dict)."""
     sd = {}
     for k, v in model.state_dict().items():
         k = k if (k.startswith("module.") or not ddp_prefix) else "module." + k
         sd[k] = v.detach().cpu()
     torch.save({"epoch": epoch + 1, "arch": arch, "state_dict": sd,
-                "optimizer": optimizer_state_dict(model, lr, momentum, weight_decay, initial_lr)}, path)
+                "optimizer": optimizer_state_dict(model, lr, momentum, weight_decay, initial_lr, betas, eps)}, path)
 
 
-def load_checkpoint(path: str, model, example_clip: torch.Tensor | None = None) -> int:
-    """Restores weights, BatchNorm buffers and SGD momentum; returns the epoch to continue with (the number in the file
-    name, main_byol.py:214-215).  `example_clip` (a device tensor of the training shape) binds the engine first so that
-    the momentum buffers have a home."""
+def load_checkpoint(path: str, model, example_clip: torch.Tensor | None = None, optimizer: str | None = None) -> int:
+    """Restores weights, BatchNorm buffers and the optimiser state (SGD momentum, or Adam / AdamW moments and step count;
+    `optimizer` as in load_optimizer_state_dict); returns the epoch to continue with (the number in the file name,
+    main_byol.py:214-215).  `example_clip` (a device tensor of the training shape) binds the engine first so that the
+    optimiser buffers have a home."""
     md = torch.load(path, map_location="cpu", weights_only=False)
     sd = {(k[len("module."):] if k.startswith("module.") else k): v for k, v in md["state_dict"].items()}
     model = unwrap(model)
     model.load_state_dict(sd)
     if example_clip is not None:
         model._bind(example_clip)
-        load_optimizer_state_dict(model, md["optimizer"])
+        load_optimizer_state_dict(model, md["optimizer"], optimizer)
     return int(os.path.basename(path).split("_")[1].split(".")[0])
 
 
 def pretrain_epochs(model, batches, opts, begin_epoch: int = 1, result_path: str | None = None, arch: str = "r21d_byol-1",
-                    grad_sync=None, save_every: int = 100, log=None):
+                    grad_sync=None, save_every: int = 100, log=None, optimizer: str = "sgd", betas=(0.9, 0.999),
+                    eps: float = 1e-8):
     """Runs epochs begin_epoch..opts.n_epochs.  `batches(epoch)` yields (clip_1, clip_2, (spa, tem, pb, rot_1, rot_2)) on
-    the device.  Returns one dict of LOG_COLUMNS per epoch."""
+    the device.  Returns one dict of LOG_COLUMNS per epoch.  optimizer="adam" / "adamw" (with betas, eps) trains with
+    torch.optim.Adam / AdamW semantics; learning rate, weight decay and gradient clipping still come from `opts`."""
     rows = []
     wrapped, model = model, unwrap(model)        # the fused step lives on the bare module; checkpoints keep the wrapper's keys
     clip = 18.0 if getattr(opts, "clip_grad_norm", 1) else 0.0
@@ -110,7 +170,8 @@ def pretrain_epochs(model, batches, opts, begin_epoch: int = 1, result_path: str
         per_step = []
         for clip_1, clip_2, labels in batches(epoch):
             losses = model.train_step(clip_1, clip_2, labels, opts.loss_weight, lr=lr, momentum=opts.momentum,
-                                      weight_decay=opts.weight_decay, clip_grad_norm=clip, grad_sync=grad_sync)
+                                      weight_decay=opts.weight_decay, clip_grad_norm=clip, grad_sync=grad_sync,
+                                      optimizer=optimizer, betas=betas, eps=eps)
             per_step.append(losses.clone())                       # device side; no host sync inside the epoch
         L = torch.stack(per_step).mean(0)
         if torch.distributed.is_available() and torch.distributed.is_initialized():
@@ -127,7 +188,8 @@ def pretrain_epochs(model, batches, opts, begin_epoch: int = 1, result_path: str
             log(row)
         if result_path is not None and (epoch % save_every == 0 or epoch == opts.n_epochs):
             save_checkpoint(os.path.join(result_path, f"save_{epoch}.pth"), wrapped, epoch, arch, lr=lr,
-                            momentum=opts.momentum, weight_decay=opts.weight_decay, initial_lr=opts.learning_rate)
+                            momentum=opts.momentum, weight_decay=opts.weight_decay, initial_lr=opts.learning_rate,
+                            betas=betas, eps=eps)
     return rows
 
 
@@ -162,13 +224,15 @@ FT_VAL_COLUMNS = ["epoch", "loss", "acc"]
 
 
 def finetune_epochs(model, train_batches, val_batches, opts, begin_epoch: int = 1, result_path: str | None = None,
-                    arch: str = "r21d_byol-1", grad_sync=None, log_train=None, log_val=None):
+                    arch: str = "r21d_byol-1", grad_sync=None, log_train=None, log_val=None, optimizer: str = "sgd",
+                    betas=(0.9, 0.999), eps: float = 1e-8):
     """The epoch loop of main_ft_mp.py:160-170 on the fused finetune step: `train` (:179-244: CrossEntropyLoss, SGD.step,
     top-1 accuracy, mean loss / accuracy per epoch weighted by batch size) then `validation` (:246-310: model.eval(), mean
     loss / accuracy, ReduceLROnPlateau on the validation loss, `save_<epoch>_max.pth` whenever the validation accuracy
     beats the best so far, the previous best file removed).  `train_batches(epoch)` / `val_batches(epoch)` yield
     (clips, labels) on the device.  Losses and hit counts stay on the device inside an epoch (one read-back per phase
-    instead of two `.item()`s per step).  Returns (train rows, val rows) with the reference's log columns."""
+    instead of two `.item()`s per step).  optimizer="adam" / "adamw" (with betas, eps) replaces SGD.step by
+    Adam / AdamW.step.  Returns (train rows, val rows) with the reference's log columns."""
     model = unwrap(model)
     task = getattr(opts, "task", "ft_all")
     sched = PlateauLR(opts.learning_rate, getattr(opts, "lr_patience", 10))
@@ -184,7 +248,7 @@ def finetune_epochs(model, train_batches, val_batches, opts, begin_epoch: int = 
         acc = None
         for x, labels in train_batches(epoch):
             loss = model.finetune_step(x, labels, lr=sched.lr, momentum=opts.momentum, weight_decay=opts.weight_decay,
-                                       grad_sync=grad_sync)
+                                       grad_sync=grad_sync, optimizer=optimizer, betas=betas, eps=eps)
             eng = model._engine
             hits = (eng.logits[:, :model.num_classes].argmax(1) == labels).sum()          # calculate_accuracy, utils.py:52-65
             z = torch.zeros(1, device=loss.device)
@@ -225,7 +289,7 @@ def finetune_epochs(model, train_batches, val_batches, opts, begin_epoch: int = 
                 os.remove(old)
             best_name, best_acc = f"save_{epoch}_max.pth", vacc
             save_checkpoint(os.path.join(result_path, best_name), model, epoch, arch, lr=sched.lr, momentum=opts.momentum,
-                            weight_decay=opts.weight_decay, initial_lr=opts.learning_rate)
+                            weight_decay=opts.weight_decay, initial_lr=opts.learning_rate, betas=betas, eps=eps)
         elif vacc > best_acc:
             best_name, best_acc = f"save_{epoch}_max.pth", vacc
     if hasattr(opts, "highest_val"):

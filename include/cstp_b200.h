@@ -422,6 +422,24 @@ int cstp_sgd_clip_step(float* p, const float* g, float* mom, int64_t n, float lr
  * learning-rate schedule (scheduler/cosine_anneal.py) by rewriting six floats. */
 int cstp_sgd_clip_step_dev(float* p, const float* g, float* mom, int64_t n, const float* hyper, float* norm_out,
                            float* workspace, void* stream);
+/* Scalars of one Adam / AdamW step, in the form torch.optim.Adam(W) (foreach=False) uses them.  step_size =
+ * lr / (1 - beta1^t) and bc2_sqrt = sqrt(1 - beta2^t) are computed by the caller in double, as torch does; so are
+ * 1 - beta1, 1 - beta2 and decay.  Adam: l2 = weight_decay, decay = 1.  AdamW: l2 = 0, decay = 1 - lr * weight_decay.
+ * Flags: nonzero = set.  Ten floats, so a device copy is a plain float[10]. */
+typedef struct {
+  float step_size, bc2_sqrt, one_minus_beta1, beta2, one_minus_beta2, eps, l2, decay, max_norm, do_clip;
+} cstp_adam_hyper;
+/* clip_grad_norm_ (as cstp_sgd_clip_step) + one Adam / AdamW step over flat fp32 buffers p, g, m (exp_avg), v
+ * (exp_avg_sq), all 16-byte aligned.  Per element, every operation rounded on its own (no FMA contraction):
+ *   g *= coef; p *= decay; g += l2 * p; m += (g - m) * (1 - beta1); v = beta2 * v + ((1 - beta2) * g) * g;
+ *   p -= (step_size * m) / (sqrt(v) / bc2_sqrt + eps).
+ * norm_out[0] = total grad norm (before clipping), norm_out[1] = clip coefficient. */
+int cstp_adam_clip_step(float* p, const float* g, float* m, float* v, int64_t n, cstp_adam_hyper hyper, float* norm_out,
+                        float* workspace, void* stream);
+/* The same with the scalars read from DEVICE memory at run time: the launch can sit in a captured CUDA graph while the
+ * host rewrites the step-dependent scalars before every replay. */
+int cstp_adam_clip_step_dev(float* p, const float* g, float* m, float* v, int64_t n, const cstp_adam_hyper* hyper,
+                            float* norm_out, float* workspace, void* stream);
 
 /* ---- pretraining clip pipeline (SURVEY.md 8 f-2) -----------------------------------------------------------
  * Replaces the pixel work of the reference's CPU data pipeline for one batch of pretraining samples:
