@@ -566,6 +566,71 @@ __global__ void __launch_bounds__(256) adam_step_kernel(float4* __restrict__ p, 
   }
 }
 
+// ------------------------------------------------------------------------------------------- representation statistics
+// Collapse indicator of one step (SimSiam's std of the l2-normalised output): per row block k and view v, the mean over
+// the 512 columns of the unbiased standard deviation over the view's B rows of z = x / max(||x||, 1e-12); block 0 also
+// gives the mean row norm ||x||.  One CTA of 512 threads per (block, view).  Every operation is a separately rounded _rn
+// intrinsic in the fixed order include/cstp_b200.h spells out, so a float32 restatement reproduces the bits.
+constexpr int kReprD = 512;
+constexpr int kReprMaxRows = 8192;        // per view: the row norms sit in dynamic shared memory
+
+struct ReprArgs {
+  const float* x[4];
+  long long ld[4];
+};
+
+__global__ void __launch_bounds__(kReprD) repr_stats_kernel(ReprArgs a, int B, float* __restrict__ out) {
+  extern __shared__ float norms[];         // [B] row norms of this view
+  __shared__ float red[kReprD];
+  const int k = blockIdx.x, t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  float* o = out + blockIdx.y * 5;
+  // selected without a dynamic index into the parameter block, which would copy it to local memory
+  const float* xk = k == 0 ? a.x[0] : k == 1 ? a.x[1] : k == 2 ? a.x[2] : a.x[3];
+  const long long ld = k == 0 ? a.ld[0] : k == 1 ? a.ld[1] : k == 2 ? a.ld[2] : a.ld[3];
+  if (xk == nullptr) {                 // block not given: its entries are 0
+    if (t == 0) {
+      o[k] = 0.f;
+      if (k == 0) o[4] = 0.f;
+    }
+    return;
+  }
+  const float* x = xk + static_cast<long long>(blockIdx.y) * B * ld;
+  for (int r = warp; r < B; r += kReprD / 32) {
+    const float* xr = x + r * ld;
+    float ss = 0.f;
+    for (int c = lane; c < kReprD; c += 32) ss = __fadd_rn(ss, __fmul_rn(xr[c], xr[c]));
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) ss = __fadd_rn(ss, __shfl_xor_sync(0xffffffffu, ss, off));
+    if (lane == 0) norms[r] = __fsqrt_rn(ss);
+  }
+  __syncthreads();
+  // column t, two passes over the rows, shifted by the first row: equal rows give exactly 0
+  const float* col = x + t;
+  const float z0 = __fdiv_rn(col[0], fmaxf(norms[0], 1e-12f));
+  float s1 = 0.f;
+  for (int r = 0; r < B; ++r) s1 = __fadd_rn(s1, __fsub_rn(__fdiv_rn(col[r * ld], fmaxf(norms[r], 1e-12f)), z0));
+  const float mean = __fdiv_rn(s1, static_cast<float>(B));
+  float s2 = 0.f;
+  for (int r = 0; r < B; ++r) {
+    const float d = __fsub_rn(__fsub_rn(__fdiv_rn(col[r * ld], fmaxf(norms[r], 1e-12f)), z0), mean);
+    s2 = __fadd_rn(s2, __fmul_rn(d, d));
+  }
+  red[t] = __fsqrt_rn(__fdiv_rn(s2, static_cast<float>(B - 1)));
+  __syncthreads();
+  for (int s = kReprD / 2; s > 0; s >>= 1) {
+    if (t < s) red[t] = __fadd_rn(red[t], red[t + s]);
+    __syncthreads();
+  }
+  if (t == 0) {
+    o[k] = __fdiv_rn(red[0], static_cast<float>(kReprD));
+    if (k == 0) {
+      float n = 0.f;
+      for (int r = 0; r < B; ++r) n = __fadd_rn(n, norms[r]);
+      o[4] = __fdiv_rn(n, static_cast<float>(B));
+    }
+  }
+}
+
 int ntxent_tensor_path(const float* zn, int rows, int d, float temperature, bool backward, float* row_loss, float* ws,
                        float** dzn_out, cudaStream_t stream);
 
@@ -586,6 +651,17 @@ extern "C" int cstp_byol_loss(const float* pred, const float* tproj, int B, int 
                               const float* upstream, float* dpred, void* stream) {
   CSTP_REQUIRE(pred && tproj && loss_out && B > 0 && D > 0 && D <= ld);
   byol_loss_kernel<<<1, 1024, 0, ST(stream)>>>(pred, tproj, B, D, ld, loss_out, upstream, dpred);
+  CSTP_LAUNCHED();
+  return CSTP_OK;
+}
+
+extern "C" int cstp_repr_stats(const float* feat, int ld_feat, const float* proj, int ld_proj, const float* pred,
+                               int ld_pred, const float* tproj, int ld_tproj, int B, float* out, void* stream) {
+  CSTP_REQUIRE(out && B >= 2 && B <= kReprMaxRows && reinterpret_cast<uintptr_t>(out) % sizeof(float) == 0);
+  const ReprArgs a{{feat, proj, pred, tproj}, {ld_feat, ld_proj, ld_pred, ld_tproj}};
+  for (int k = 0; k < 4; ++k)
+    CSTP_REQUIRE(a.x[k] == nullptr || (a.ld[k] >= kReprD && reinterpret_cast<uintptr_t>(a.x[k]) % sizeof(float) == 0));
+  repr_stats_kernel<<<dim3(4, 2), kReprD, B * sizeof(float), ST(stream)>>>(a, B, out);
   CSTP_LAUNCHED();
   return CSTP_OK;
 }

@@ -29,7 +29,7 @@ from dataclasses import dataclass
 import torch
 
 from . import ops
-from .ops import ConvGeom, pad16, pad64
+from .ops import REPR_STATS, ConvGeom, pad16, pad64
 
 import os
 
@@ -214,7 +214,7 @@ class StepEngine:
     def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", momentum_ema: float = 0.996,
                  record: bool = False, overlap: bool = True, bn_sync=None, fuse_apply: bool | None = None,
                  ntxent: dict | None = None, fuse_min_positions: int | None = None, fuse_policy: str | None = None,
-                 graph: bool | None = None):
+                 graph: bool | None = None, collapse_stats: bool = False):
         if H % 2 or W % 4:
             raise ops.L.CstpError("clip height must be even and its width a multiple of 4 (1x7x7 stride-2 stem over packed rows)")
         self.B, self.T, self.H, self.W = B, T, H, W
@@ -284,6 +284,10 @@ class StepEngine:
         self.stem_rows = torch.zeros(self.N, T, H // 2, W // 2, ops.STEM_CHANNELS, device=self.device, dtype=ACT_DTYPE)
         self.weights5 = torch.tensor([0.1, 1.0, 1.0, 1.0, 1.0], **f32)
         self.losses = torch.zeros(8, **f32)       # [0..5] CE, [6] weighted CE sum, [7] BYOL loss
+        # collapse statistics (cstp_repr_stats) of the last forward run with collapse_stats on: [view][REPR_STATS].
+        # Changing the flag changes the step program: drop a captured graph first (R21DBYOL.train_step does).
+        self.collapse_stats = bool(collapse_stats)
+        self.step_stats = torch.zeros(2, len(REPR_STATS), **f32)
         self.norm_out = torch.zeros(2, **f32)
         self.sgd_ws = torch.zeros(2048, **f32)
         # static inputs of the captured step: integer labels (spa, tem, pb, rot1, rot2) and the optimiser's hyper-parameters
@@ -836,6 +840,8 @@ class StepEngine:
             for op in self.fwd_target:
                 op()
         ops.byol_loss(self.pred, self.tproj, self.B, 512, self.losses[7:8], None, self.dpred)
+        if self.collapse_stats:           # reads buffers the step writes anyway: nothing else changes
+            ops.repr_stats(self.feat, self.proj_out, self.pred, self.tproj, self.B, self.step_stats)
         if self.ntxent is not None:
             self._ntxent_forward()
         for op in self.fwd_heads:

@@ -274,3 +274,19 @@ class InferenceEngine(FinetuneEngine):
         """nn.CrossEntropyLoss() over the rows of the last run (labels has one entry per row); fills self.loss."""
         n = labels.shape[0]
         E.ops.ce_loss(self.logits[:n], labels, self.num_classes, self.loss, None, self.ce_ws)
+
+
+class FeatureEngine(InferenceEngine):
+    """Forward-only eval engine of the online network alone: its program ends at the average pool (`feat`, fp32
+    [capacity][512]); there is no F.normalize, cls_bn or classify.  It reads the `online_net.*` weights and BatchNorm
+    running statistics by name from the stores of `share`, a pretraining StepEngine (nothing is copied), and packs its
+    own bf16 weights.  The backbone program is InferenceEngine's, so the features are bit-identical to those of a
+    finetune model holding the same online-network weights and running statistics."""
+
+    def _build(self):
+        x5, _ = self._backbone(self.fwd_online, self.train, "online_net", False, "online")
+        self.feat = torch.zeros(self.B, 512, device=self.device, dtype=torch.float32)
+        self.logits = None                       # no classification head: run() returns None
+        self._rec("head.feat", self.feat)
+        self.fwd_online.append(lambda: E.ops.avgpool_fwd(x5, self.feat, None))
+        self._finish_build()

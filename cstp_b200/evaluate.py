@@ -214,6 +214,11 @@ def video_features(model, store: GpuVideoStore, total_frames: Sequence[int], *, 
     finetune model `model` (R21DBYOL(pretrain=False), DDP-wrapped or not) in eval semantics.  The clips are packed like
     test_videos'; a video's mean is its sequential fp32 sum in clip order divided by its clip count.
 
+    `model` may also be a pretraining model (R21DBYOL(pretrain=True) that has run train_step): the features are then
+    those of its live online network (engine_ft.FeatureEngine over the step engine's weights and BatchNorm running
+    statistics), bit for bit the features of the finetune model loaded from a checkpoint of the same moment.  Nothing
+    of the training state changes: no running statistic, no captured step, no optimiser state, no random generator.
+
     With world > 1 this rank extracts its contiguous shard and the shards are all-gathered over the default process
     group, so every rank returns all rows.  Returns fp32 [videos][512] on the store's device.  A split that does not fit
     in device memory is extracted chunk by chunk (one call per range of videos) and concatenated, or with

@@ -224,6 +224,7 @@ SIGNATURES = {
     "cstp_colsum": (_i, [_vp, _i64, _i, _i, _vp, _i, _vp]),
     "cstp_cast_pad": (_i, [_vp, _i64, _i, _i, _vp, _i, _vp, _vp]),
     "cstp_byol_loss": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "cstp_repr_stats": (_i, [_vp, _i, _vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp]),
     "cstp_pretext_ce": (_i, [C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _i, _i, _i, _vp, _vp, _vp]),
     "cstp_ntxent_workspace_floats": (C.c_longlong, [_i, _i]),
     "cstp_ntxent": (_i, [_vp, _i, _i, _f, _i, _vp, _vp, _vp, C.c_longlong, _vp]),

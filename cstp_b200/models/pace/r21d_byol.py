@@ -237,6 +237,7 @@ class R21DBYOL(nn.Module):
                                          **getattr(self, "engine_options", {}))
             if eng is not None:      # keep optimiser-side state across a batch-geometry change
                 new.take_optimizer_state(eng)
+            self._infer.clear()      # feature engines read the stores of the engine being replaced
             eng = self._engine = new
             self._engine_key = key
             self._alias_ptr = None
@@ -319,8 +320,12 @@ class R21DBYOL(nn.Module):
     def inference_engine(self, capacity: int, T: int, H: int, W: int, device):
         """The cached forward-only eval engine (engine_ft.InferenceEngine) of this batch capacity and clip size.  It reads
         the parameters and BatchNorm running statistics of the bound engine; while no engine is bound, the first one
-        created owns them and the parameters are aliased onto it, as _bind_ft does."""
+        created owns them and the parameters are aliased onto it, as _bind_ft does.
+        A pretraining model gets an engine_ft.FeatureEngine instead: the online network up to its pooled feature, reading
+        the live weights and running statistics of the bound step engine."""
         from ... import engine_ft
+        if self.pretrain:
+            return self._feature_engine(capacity, T, H, W, device)
         if not isinstance(self.cls_bn, nn.Module):
             raise TypeError("'bool' object is not callable")
         device = torch.device(device)
@@ -346,6 +351,26 @@ class R21DBYOL(nn.Module):
         self._alias_ft(owner)
         return eng
 
+    def _feature_engine(self, capacity, T, H, W, device):
+        from ... import engine_ft
+        eng = self._engine
+        if eng is None:
+            raise _engine_mod.ops.L.CstpError(
+                "the features of a pretraining model are those of its live step engine: run train_step (or "
+                "train.load_checkpoint with example_clip) before extracting them")
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        if eng.device != device:
+            raise _engine_mod.ops.L.CstpError(f"the bound engine lives on {eng.device}, not {device}")
+        key = (capacity, T, H, W, device)
+        feat = self._infer.get(key)
+        if feat is None:
+            opts = {k: v for k, v in getattr(self, "engine_options", {}).items()
+                    if k in ("fuse_apply", "fuse_min_positions", "fuse_policy")}
+            feat = self._infer[key] = engine_ft.FeatureEngine(capacity, T, H, W, device=device, share=eng, **opts)
+        return feat
+
     def free_inference_engines(self):
         """Frees the cached eval engines of other batch sizes (activations, packed weights, CUDA graphs); the next eval
         forward builds what it needs again.  The bound training engine is not affected."""
@@ -364,7 +389,7 @@ class R21DBYOL(nn.Module):
         announced through _dirty) starts a new weight generation."""
         if self._dirty:
             self._wgen += 1
-            self._dirty = False
+            self._dirty = self.pretrain          # a pretraining model's step engine re-packs (and clears it) in train_step
         key = (eng.train.data._version, self._wgen)
         if getattr(eng, "_packed_key", None) != key:
             eng.pack_online()
@@ -472,15 +497,23 @@ class R21DBYOL(nn.Module):
     # ------------------------------------------------------------------------------------------ fused fast path
     @torch.no_grad()
     def train_step(self, x1, x2, labels, loss_weight=(0.1, 1, 1, 1, 1), lr=0.03, momentum=0.9, weight_decay=5e-4,
-                   clip_grad_norm=18.0, grad_sync=None, optimizer="sgd", betas=(0.9, 0.999), eps=1e-8):
+                   clip_grad_norm=18.0, grad_sync=None, optimizer="sgd", betas=(0.9, 0.999), eps=1e-8,
+                   collapse_stats=False):
         """One full pretraining step (main_byol.py:60-91) as a single launch program.  optimizer="adam" / "adamw" steps
         torch.optim.Adam / AdamW(lr, betas, eps, weight_decay) after the same gradient clipping; `momentum` is then unused.
+        collapse_stats=True adds one launch right after the BYOL loss that writes the step's representation statistics
+        (see step_stats); losses, gradients, weights and buffers are bit for bit those of a step without it.  A setting
+        that differs from the captured step's drops that graph and captures the step again.
 
         labels = (spa, tem, pb, rot1, rot2) int64 device tensors.  `grad_sync(flat_grad)` is called between backward
         and the optimiser (data-parallel all-reduce).  Returns the engine's device loss vector
         [ce_spa, ce_tem, ce_pb1, ce_pb2, ce_rot1, ce_rot2, weighted CE sum, loss_byol] without synchronising."""
         eng = self._bind(x1)
         eng.select_optimizer(optimizer)          # an invalid or conflicting kind raises before anything runs
+        if eng.collapse_stats != bool(collapse_stats):
+            eng.collapse_stats = bool(collapse_stats)
+            eng.drop_graph()
+        self._wgen += 1                          # the step updates the weights in place: feature engines must re-pack
         if tuple(loss_weight) != getattr(self, "_lw", None):
             eng.set_loss_weight(loss_weight)
             self._lw = tuple(loss_weight)
@@ -501,3 +534,14 @@ class R21DBYOL(nn.Module):
         eng.optimizer_step(lr, momentum, weight_decay, clip_grad_norm or 0.0, bool(clip_grad_norm), optimizer, betas, eps)
         self._nbt += self._nbt_inc
         return eng.losses
+
+    def step_stats(self) -> torch.Tensor:
+        """Representation statistics of the last train_step run with collapse_stats=True, as the bound engine's device
+        tensor fp32 [2 views][5] (no synchronisation; the next such step overwrites it).  Columns, in order
+        (ops.REPR_STATS): std_feat, std_proj, std_pred, std_tproj -- the mean over the 512 columns of the unbiased
+        standard deviation over the view's samples of the l2-normalised online pooled feature, projector output,
+        predictor output and target projector output (about 1/sqrt(512) = 0.0442 for well-spread embeddings, 0 for a
+        collapsed, constant one) -- and feat_norm, the mean norm of the pooled feature."""
+        if self._engine is None or not self.pretrain:
+            raise RuntimeError("step_stats() belongs to a pretraining model that has run train_step")
+        return self._engine.step_stats

@@ -1035,6 +1035,38 @@ def byol_loss(pred, tproj, B: int, D: int, loss_out, upstream=None, dpred=None) 
                                     _ptr(dpred), _stream()))
 
 
+REPR_DIM, REPR_MAX_ROWS = 512, 8192
+REPR_STATS = ("std_feat", "std_proj", "std_pred", "std_tproj", "feat_norm")     # the columns of one view's statistics
+
+
+def _check_repr_stats(blocks, B: int, out) -> None:
+    if not 2 <= B <= REPR_MAX_ROWS:
+        raise L.CstpError(f"repr_stats: B = {B}, expected 2 .. {REPR_MAX_ROWS} (an unbiased std needs two rows per view)")
+    for t in blocks:
+        if t is None:
+            continue
+        if t.dtype != torch.float32 or t.dim() != 2 or t.stride(1) != 1 or t.shape[0] < 2 * B \
+                or t.shape[1] < REPR_DIM or t.stride(0) < REPR_DIM:
+            raise L.CstpError(f"repr_stats: row blocks must be fp32 [2B][ld >= {REPR_DIM}] with unit column stride, got "
+                              f"{t.dtype} {tuple(t.shape)} strides {t.stride()} for B = {B}")
+    if out.dtype != torch.float32 or not out.is_contiguous() or out.numel() < 2 * len(REPR_STATS):
+        raise L.CstpError("repr_stats: out must be contiguous fp32 [2][5]")
+
+
+def repr_stats(feat, proj, pred, tproj, B: int, out) -> None:
+    """Representation (collapse) statistics of one step into out fp32 [2][5]: per view, the mean over 512 columns of the
+    unbiased std over the view's B rows of the l2-normalised online pooled feature / projector / predictor / target
+    projector output (REPR_STATS order), and the feature's mean row norm.  Each block is fp32 [2B][ld] (views stacked
+    along the rows, the first 512 columns valid) or None (skipped: its entry is 0).  Exact arithmetic of
+    include/cstp_b200.h cstp_repr_stats."""
+    blocks = (feat, proj, pred, tproj)
+    _check_repr_stats(blocks, B, out)
+    _require_cuda(*blocks, out)
+    ld = [0 if t is None else t.stride(0) for t in blocks]
+    L.check(L.load().cstp_repr_stats(_ptr(feat), ld[0], _ptr(proj), ld[1], _ptr(pred), ld[2], _ptr(tproj), ld[3], B,
+                                     _ptr(out), _stream()))
+
+
 def pretext_ce(logits, labels, dlogits, B: int, n_cls: int, weights5, losses_out) -> None:
     arr = C.c_void_p * 6
     lg = arr(*[t.data_ptr() for t in logits])

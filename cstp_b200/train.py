@@ -13,6 +13,8 @@ What it keeps from the reference:
   * the log columns of main_byol.py:216-225.
 What it changes: the six `.item()` host syncs per step (main_byol.py:77-84) become one read-back of the per-step loss
 vectors per epoch; the all-reduce of the logged loss (:75) is folded into that read-back.
+What it adds on request: per-epoch representation (collapse) statistics of the fused step, and nearest-neighbour
+retrieval of the live online network every few epochs (RetrievalMonitor), as extra columns of the epoch's row.
 """
 from __future__ import annotations
 
@@ -20,6 +22,7 @@ import os
 
 import torch
 
+from .ops import REPR_STATS
 from .scheduler.cosine_anneal import lr_at
 
 LOG_COLUMNS = ["epoch", "loss", "loss_byol", "loss_pred_spa", "loss_pred_tem", "loss_pred_pb", "loss_pred_rot", "acc", "lr"]
@@ -158,31 +161,57 @@ def load_checkpoint(path: str, model, example_clip: torch.Tensor | None = None, 
 
 def pretrain_epochs(model, batches, opts, begin_epoch: int = 1, result_path: str | None = None, arch: str = "r21d_byol-1",
                     grad_sync=None, save_every: int = 100, log=None, optimizer: str = "sgd", betas=(0.9, 0.999),
-                    eps: float = 1e-8):
+                    eps: float = 1e-8, collapse_stats: bool = False, monitor: "RetrievalMonitor | None" = None,
+                    monitor_every: int = 10):
     """Runs epochs begin_epoch..opts.n_epochs.  `batches(epoch)` yields (clip_1, clip_2, (spa, tem, pb, rot_1, rot_2)) on
     the device.  Returns one dict of LOG_COLUMNS per epoch.  optimizer="adam" / "adamw" (with betas, eps) trains with
-    torch.optim.Adam / AdamW semantics; learning rate, weight decay and gradient clipping still come from `opts`."""
+    torch.optim.Adam / AdamW semantics; learning rate, weight decay and gradient clipping still come from `opts`.
+
+    collapse_stats=True: every step also computes its representation statistics on the device (R21DBYOL.step_stats);
+    their epoch mean comes back with the losses in the same read-back (averaged over ranks like them) and the row gains
+    the columns std_feat, std_proj, std_pred, std_tproj and feat_norm, each the mean of the two views.
+    monitor (a RetrievalMonitor): every `monitor_every` epochs and at the last epoch, the row gains its recall@k columns,
+    computed from the live online network.  Neither changes the training: losses, weights and checkpoints are bit for bit
+    those of a run without them."""
+    if monitor_every < 1:
+        raise ValueError(f"monitor_every must be at least 1, got {monitor_every}")
     rows = []
     wrapped, model = model, unwrap(model)        # the fused step lives on the bare module; checkpoints keep the wrapper's keys
     clip = 18.0 if getattr(opts, "clip_grad_norm", 1) else 0.0
+    dist = torch.distributed.is_available() and torch.distributed.is_initialized()
+    rank, world = (torch.distributed.get_rank(), torch.distributed.get_world_size()) if dist else (0, 1)
     for epoch in range(begin_epoch, opts.n_epochs + 1):
         lr = epoch_lr(epoch, opts.n_epochs, opts.learning_rate)
-        per_step = []
+        per_step, per_stats = [], []
         for clip_1, clip_2, labels in batches(epoch):
             losses = model.train_step(clip_1, clip_2, labels, opts.loss_weight, lr=lr, momentum=opts.momentum,
                                       weight_decay=opts.weight_decay, clip_grad_norm=clip, grad_sync=grad_sync,
-                                      optimizer=optimizer, betas=betas, eps=eps)
+                                      optimizer=optimizer, betas=betas, eps=eps, collapse_stats=collapse_stats)
             per_step.append(losses.clone())                       # device side; no host sync inside the epoch
+            if collapse_stats:
+                per_stats.append(model.step_stats().clone())
         L = torch.stack(per_step).mean(0)
-        if torch.distributed.is_available() and torch.distributed.is_initialized():
+        if dist:
             torch.distributed.all_reduce(L)                       # reduce_mean of main_byol.py:22-26,75
-            L /= torch.distributed.get_world_size()
-        L = L.cpu()
+            L /= world
+        if collapse_stats:
+            S = torch.stack(per_stats).mean(0)
+            if dist:
+                torch.distributed.all_reduce(S)
+                S /= world
+            L, S = torch.cat([L, S.reshape(-1)]).cpu().split([L.numel(), S.numel()])
+            S = S.view(per_stats[0].shape)
+        else:
+            L = L.cpu()
         w = opts.loss_weight
         total = w[0] * L[7] + L[6]
         # main_byol.py:81-84,119-129: pb / rot columns are the MEAN of the two views' terms, acc is None, lr has 5 decimals
         row = dict(zip(LOG_COLUMNS, [epoch, total.item(), L[7].item(), L[0].item(), L[1].item(), ((L[2] + L[3]) / 2).item(),
                                      ((L[4] + L[5]) / 2).item(), None, float("{:.5f}".format(lr))]))
+        if collapse_stats:
+            row.update({name: ((S[0, i] + S[1, i]) / 2).item() for i, name in enumerate(REPR_STATS)})
+        if monitor is not None and (epoch % monitor_every == 0 or epoch == opts.n_epochs):
+            row.update(monitor(wrapped, rank, world))
         rows.append(row)
         if log is not None:
             log(row)
@@ -191,6 +220,44 @@ def pretrain_epochs(model, batches, opts, begin_epoch: int = 1, result_path: str
                             momentum=opts.momentum, weight_decay=opts.weight_decay, initial_lr=opts.learning_rate,
                             betas=betas, eps=eps)
     return rows
+
+
+class RetrievalMonitor:
+    """Nearest-neighbour retrieval of the live online network during pretraining (the VCOP / Pace protocol): a call
+    extracts per-video features of the gallery (the train split) and of the queries (the test split) from the pretraining
+    model itself (evaluate.video_features / video_features_jpeg on R21DBYOL(pretrain=True)), ranks the gallery for every
+    query (evaluate.retrieve_videos) and returns {"recall@k": fraction of queries} for every k in `ks`.
+
+    gallery, query: (source, total_frames, labels), source a GpuVideoStore or a read_frames(video, frame_numbers)
+    callable returning the JPEG bytes of those frames (frame sizes are read from each video's first frame).  clip_kwargs
+    (sample_duration, sample_size, pb_rate, capacity) go to the feature extraction.  The model's training state is left
+    as it was, and nothing is written to disk."""
+
+    def __init__(self, gallery, query, ks=(1, 5, 10, 20, 50), **clip_kwargs):
+        self.ks = tuple(int(k) for k in ks)
+        if not self.ks or min(self.ks) < 1 or max(self.ks) > 64:
+            raise ValueError(f"retrieval cutoffs must lie in [1, 64], got {ks}")
+        for name, side in (("gallery", gallery), ("query", query)):
+            if len(side) != 3 or len(side[1]) != len(side[2]):
+                raise ValueError(f"{name}: expected (store or read_frames, total_frames, labels) with one label per video")
+        self.gallery, self.query, self.clip_kwargs = tuple(gallery), tuple(query), clip_kwargs
+
+    def _features(self, model, side, rank, world):
+        from .data_process.datasets import GpuVideoStore
+        from .evaluate import video_features, video_features_jpeg
+        source, frames, _ = side
+        if isinstance(source, GpuVideoStore):
+            return video_features(model, source, frames, rank=rank, world=world, **self.clip_kwargs)
+        eng = unwrap(model)._engine
+        return video_features_jpeg(model, source, frames, device=eng.device if eng is not None else "cuda", rank=rank,
+                                   world=world, **self.clip_kwargs)
+
+    def __call__(self, model, rank: int = 0, world: int = 1) -> dict:
+        from .evaluate import retrieve_videos
+        g = self._features(model, self.gallery, rank, world)
+        q = self._features(model, self.query, rank, world)
+        r = retrieve_videos(q, self.query[2], g, self.gallery[2], self.ks, rank=rank, world=world)
+        return {f"recall@{k}": r["recall"][k] for k in self.ks}
 
 
 # ---------------------------------------------------------------------------------------------- finetune driver

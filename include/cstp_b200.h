@@ -346,6 +346,17 @@ int cstp_cast_pad(const float* x, int64_t rows, int cols, int ld_in, void* out, 
  * (`upstream` is a device scalar, NULL = 1). */
 int cstp_byol_loss(const float* pred, const float* tproj, int B, int D, int ld, float* loss_out,
                    const float* upstream, float* dpred, void* stream);
+/* Representation (collapse) statistics of one step.  Blocks k = 0..3 are fp32 [2B][ld_k] rows (512 valid columns,
+ * ld_k >= 512; NULL = not given, its entries are 0): the online pooled feature, projector, predictor and target projector
+ * outputs.  Per view v (rows [vB, (v+1)B)) and block, with every operation rounded on its own, in this order:
+ *   n_r = sqrt(ss_r): lane l of a warp adds x[l]^2, x[l+32]^2, ... in order, then an xor butterfly over offsets
+ *         16, 8, 4, 2, 1 sums the lanes;  z_rj = x_rj / max(n_r, 1e-12)  (F.normalize);
+ *   per column j: d_rj = z_rj - z_0j, m_j = (sum_r d_rj, r ascending) / B, std_j = sqrt((sum_r (d_rj - m_j)^2) / (B - 1));
+ *   s = (pairwise tree sum of std_j: a[i] += a[i + h] for h = 256, 128, ..., 1) / 512.
+ * out fp32 [2][5]: out[v][k] = s of block k, out[v][4] = (sum_r n_r of block 0, r ascending) / B.  s is about
+ * 1/sqrt(512) = 0.0442 for well-spread rows and exactly 0 when the view's rows are equal.  2 <= B <= 8192. */
+int cstp_repr_stats(const float* feat, int ld_feat, const float* proj, int ld_proj, const float* pred, int ld_pred,
+                    const float* tproj, int ld_tproj, int B, float* out, void* stream);
 /* Six nn.CrossEntropyLoss() (mean) over [B][ld] logits with 5 classes + the weighted sum of main_byol.py:63-73.
  * logits[h], labels[h] (int64), dlogits[h] for h in spa, tem, pb1, pb2, rot1, rot2; weights[5] = --loss_weight.
  * losses_out[0..5] = the six CE values, losses_out[6] = weighted sum of them (BYOL term excluded). */
