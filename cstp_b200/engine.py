@@ -567,8 +567,11 @@ class StepEngine:
 
         def fwd():
             p0.run()
-            ops.bn_forward_stats(raw, site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS, BN_MOMENTUM,
-                                 sync=self.bn_sync)
+            if self.eval_mode:       # model.eval() of a standalone R2Plus1DNet's projector (engine_backbone)
+                ops.bn_eval_coeffs(site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS)
+            else:
+                ops.bn_forward_stats(raw, site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS, BN_MOMENTUM,
+                                     sync=self.bn_sync)
             ops.bn_apply(raw, site.st, h, relu=True)
             p3.run()
         prog.append(fwd)

@@ -212,6 +212,7 @@ SIGNATURES = {
     "cstp_pack_weight": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _vp]),
     "cstp_pack_weights_batched": (_i, [_vp, _vp, _i, _i64, _vp]),
     "cstp_stem_pack": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
+    "cstp_stem_dgrad": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp]),
     "cstp_bn_stats": (_i, [_vp, _i64, _i, _i, _vp, _i, _vp]),
     "cstp_bn_partials_reduce": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "cstp_bn_finalize": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _vp, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

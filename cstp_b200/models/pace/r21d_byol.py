@@ -19,8 +19,14 @@ import math
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from ... import engine as _engine_mod
+
+
+def _engine_backbone():
+    from ... import engine_backbone
+    return engine_backbone
 
 
 def get_fine_tuning_parameters(model, ft_begin_index):
@@ -109,7 +115,69 @@ class Predictor(_Holder):
         self.net = _mlp(dim, prediction_hidden_size, prediction_size)
 
 
-class R2Plus1DNet(_Holder):
+class _Lease:
+    """An engine lent to one grad-enabled R2Plus1DNet call: it goes back to its pool after the call's backward, or when
+    autograd frees the call's graph without one (the lease lives on the autograd node)."""
+
+    __slots__ = ("pool", "engine")
+
+    def __init__(self, pool, engine):
+        self.pool, self.engine = pool, engine
+
+    def release(self):
+        if self.engine is not None:
+            self.pool.append(self.engine)
+            self.engine = None
+
+    def __del__(self):
+        self.release()
+
+
+class _BackboneFn(torch.autograd.Function):
+    """One autograd node for a standalone train-mode R2Plus1DNet call: (feat[, proj]) forward, and a backward that returns
+    the gradient of every parameter and, when the clip requires it, of the clip."""
+
+    @staticmethod
+    def forward(ctx, names, lease, x, *params):
+        eng = lease.engine
+        eng.forward(x)
+        ctx.names, ctx.lease = names, lease
+        feat = eng.feat.clone()
+        if eng.proj:
+            return feat, eng.proj_out[:, :512].clone()
+        return feat
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dfeat, dproj=None):
+        lease = ctx.lease
+        eng = lease.engine
+        if eng is None:
+            raise RuntimeError("the backward pass of this R2Plus1DNet call has already run (retain_graph is not supported: "
+                               "its activations went back to the module's pool)")
+        need = ctx.needs_input_grad
+        dx = torch.empty((eng.B, 3, eng.T, eng.H, eng.W), device=eng.device, dtype=torch.float32) if need[2] else None
+        eng.backward_from(dfeat, dproj, dx)
+        grads = [eng.train.view(n, eng.grad).clone() if want else None for n, want in zip(ctx.names, need[3:])]
+        lease.release()
+        return (None, None, dx, *grads)
+
+
+class R2Plus1DNet(nn.Module):
+    """The backbone (+ projector with proj_flag) of r21d_byol.py:184-229.  Inside R21DBYOL it only holds parameters of
+    the parent's engine.  Created on its own and moved to CUDA, forward(x) runs it on engine_backbone.BackboneEngine:
+
+      x fp32 (B, 3, T, H, W) on the device (H even, W a multiple of 4) -> feat fp32 [B][512], or (feat, proj) with proj_flag
+      train():  BatchNorm over this call's B clips, running statistics updated (momentum 0.1, unbiased variance) and
+                num_batches_tracked + 1, as torch's BatchNorm3d / BatchNorm1d; with autograd enabled one custom Function
+                whose backward returns every parameter gradient and, when x.requires_grad, d x (no double backward);
+                under torch.no_grad() forward only (statistics still update)
+      eval():   running statistics, forward only, any batch size (engines of engine_ft.inference_capacity buckets)
+
+    Every grad-enabled call holds an engine (its activations) until its backward has run or its graph is freed; engines are
+    pooled per (batch geometry, device, variant) and share one set of flat parameter / BatchNorm-buffer stores, of which
+    the module's parameters and buffers are views (optimizer.step and load_state_dict are seen by the next call)."""
+
     def __init__(self, layer_sizes=(1, 1, 1, 1), block_type=SpatioTemporalResBlock, proj_flag=False):
         super().__init__()
         self.conv1 = SpatioTemporalConv(3, 64, (3, 7, 7), stride=(1, 2, 2), padding=(1, 3, 3))
@@ -121,6 +189,142 @@ class R2Plus1DNet(_Holder):
         self.proj_flag = proj_flag
         if proj_flag:
             self.project = Projector(dim=512, projection_size=512, projection_hidden_size=4096)
+        self._in_parent = False       # set by R21DBYOL: the parameters then belong to the parent's engine
+        self._reset_engines()
+
+    def _reset_engines(self):
+        self._pools = {}              # (B, T, H, W, device, variant) -> free engine_backbone.BackboneEngine list
+        self._owner = None            # the engine whose stores the parameters and BatchNorm buffers are views of
+        self._alias_ptr = None        # data pointers of the parameters and buffers when they were last aliased
+        self._wgen = 0                # bumped when the parameters are re-pointed, reloaded or marked dirty (see _acquire)
+        self._names = None
+
+    def __getstate__(self):
+        # copies (copy.deepcopy, pickling) get their own engines on first use
+        state = self.__dict__.copy()
+        state.update(_pools={}, _owner=None, _alias_ptr=None)
+        return state
+
+    def load_state_dict(self, *a, **k):
+        r = super().load_state_dict(*a, **k)
+        self._wgen += 1
+        return r
+
+    def mark_weights_dirty(self):
+        """Call after writing parameters behind autograd's back (through `p.data`, which has a version counter of its
+        own): the next call then re-packs the bf16 weights.  In-place updates of the parameters themselves
+        (optimizer.step, `p.mul_()` under no_grad, load_state_dict) and `p.data = ...` re-assignments are seen without it."""
+        self._wgen += 1
+
+    def _store_names(self):
+        """The engine-store names of the parameters, in registration order."""
+        if self._names is None:
+            pre = _engine_backbone().PREFIX
+            self._names = [f"{pre}.{n}" for n, _ in self.named_parameters()]
+        return self._names
+
+    def _pointers(self):
+        return tuple(t.data_ptr() for t in self.parameters()) + tuple(b.data_ptr() for b in self.buffers())
+
+    def _alias(self, owner):
+        """Points every parameter / BatchNorm buffer at owner's flat stores (again after .cuda() / .to() moved them, or a
+        `p.data = ...` / buffer assignment replaced one of them)."""
+        if self._alias_ptr == self._pointers():
+            return
+        pre = _engine_backbone().PREFIX
+        with torch.no_grad():
+            for name, p in self.named_parameters():
+                v = owner.train.view(f"{pre}.{name}")
+                v.copy_(p.data)
+                p.data = v
+            nbt = []
+            for mname, mod in self.named_modules():
+                if isinstance(mod, (nn.BatchNorm1d, nn.BatchNorm3d)):
+                    for b in ("running_mean", "running_var"):
+                        v = owner.bufs.view(f"{pre}.{mname}.{b}")
+                        v.copy_(mod._buffers[b])
+                        mod._buffers[b] = v
+                    nbt.append(mod)
+            flat = torch.stack([m._buffers["num_batches_tracked"].to(owner.device) for m in nbt])
+            for i, m in enumerate(nbt):
+                m._buffers["num_batches_tracked"] = flat[i]
+            self._nbt = flat
+        self._alias_ptr = self._pointers()
+        self._wgen += 1
+
+    def _acquire(self, B, T, H, W, device, variant):
+        """A free engine of this geometry and variant ("grad", "nograd", "eval"), with the current weights packed."""
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        if self._owner is not None and self._owner.device != device:
+            self._reset_engines()
+        key = (B, T, H, W, device, variant)
+        pool = self._pools.setdefault(key, [])
+        if pool:
+            eng = pool.pop()
+        else:
+            opts = {k: v for k, v in getattr(self, "engine_options", {}).items()
+                    if k in ("record", "overlap", "fuse_apply", "fuse_min_positions", "fuse_policy")}
+            eng = _engine_backbone().BackboneEngine(B, T, H, W, device=device, proj=bool(self.proj_flag),
+                                                    grads=variant == "grad", eval_mode=variant == "eval",
+                                                    share=self._owner, **opts)
+            if self._owner is None:
+                self._owner = eng
+                self._alias_ptr = None
+        self._alias(self._owner)
+        # the parameters are views of the owner's flat store, but `p.data = view` leaves each parameter its own version
+        # counter: an in-place update through a parameter bumps that counter, not the store's -- key on both
+        key = (self._owner.train.data._version, sum(p._version for p in self.parameters()), self._wgen)
+        if getattr(eng, "_packed_key", None) != key:
+            eng.pack_online()
+            eng._packed_key = key
+        return pool, eng
+
+    def forward(self, x):
+        ops = _engine_mod.ops
+        if self._in_parent:
+            raise RuntimeError("this R2Plus1DNet holds parameters of its R21DBYOL's engine: call the parent's forward / "
+                               "train_step, or take its features with cstp_b200.evaluate.video_features(model, ...); a "
+                               "standalone R2Plus1DNet(...) runs on its own")
+        ops.require_device(x)
+        if x.dim() != 5 or x.shape[1] != 3 or x.dtype != torch.float32:
+            raise ops.L.CstpError(f"R2Plus1DNet takes fp32 clips (B, 3, T, H, W), got {x.dtype} {tuple(x.shape)}")
+        B, _, T, H, W = x.shape
+        if H % 2 or W % 4:
+            raise ops.L.CstpError("clip height must be even and its width a multiple of 4 (1x7x7 stride-2 stem over "
+                                  "packed rows)")
+        x = x.contiguous()
+        if not self.training:
+            if torch.is_grad_enabled() and x.requires_grad:
+                raise ops.L.CstpError("an eval-mode R2Plus1DNet call is forward only; the input gradient needs train()")
+            return self._forward_eval(x)
+        params = list(self.parameters())
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params)):
+            pool, eng = self._acquire(B, T, H, W, x.device, "grad")
+            out = _BackboneFn.apply(self._store_names(), _Lease(pool, eng), x, *params)
+        else:
+            pool, eng = self._acquire(B, T, H, W, x.device, "nograd")
+            try:
+                eng.forward(x)
+                out = eng.feat.clone()
+                if eng.proj:
+                    out = (out, eng.proj_out[:, :512].clone())
+            finally:
+                pool.append(eng)
+        self._nbt += 1
+        return out
+
+    def _forward_eval(self, x):
+        from ... import engine_ft
+        n, _, T, H, W = x.shape
+        pool, eng = self._acquire(engine_ft.inference_capacity(n), T, H, W, x.device, "eval")
+        try:
+            eng.forward(x)
+            feat = eng.feat[:n].clone()
+            return (feat, eng.proj_out[:n, :512].clone()) if eng.proj else feat
+        finally:
+            pool.append(eng)
 
 
 class _LossComFn(torch.autograd.Function):
@@ -184,6 +388,7 @@ class R21DBYOL(nn.Module):
             self.momentum = momentum
             self.online_net = R2Plus1DNet(layer_sizes=(1, 1, 1, 1), proj_flag=True)
             self.target_net = R2Plus1DNet(layer_sizes=(1, 1, 1, 1), proj_flag=True)
+            self.target_net._in_parent = True
             self.predictor = Predictor(dim=512, prediction_size=512, prediction_hidden_size=4096)
             for p in self.target_net.parameters():
                 p.requires_grad = False
@@ -198,6 +403,7 @@ class R21DBYOL(nn.Module):
             self.cls_bn = kwargs["cls_bn"]
             if self.cls_bn:
                 self.cls_bn = nn.BatchNorm1d(512)
+        self.online_net._in_parent = True
         # r21d_byol.py:301-329: every Linear / Conv3d / BatchNorm weight (BN gamma included) is redrawn
         # U(+-sqrt(6/(fan_in+fan_out))); 1-D tensors use fan_in = fan_out = C/2.
         with torch.no_grad():

@@ -906,6 +906,24 @@ def stem_pack(x: torch.Tensor, P: torch.Tensor) -> None:
     L.check(L.load().cstp_stem_pack(_ptr(x), N, T, H, W, _ptr(P), _stream()))
 
 
+def stem_dgrad(g: torch.Tensor, w: torch.Tensor, dx: torch.Tensor) -> None:
+    """Input gradient of the 1x7x7 s(1,2,2) p(0,3,3) stem: g, the stem unit's bf16 d(raw) (N, T, H/2, W/2, Cg), and the
+    fp32 (cout, 3, 1, 7, 7) weight -> fp32 NCDHW dx (N, 3, T, H, W), overwritten (include/cstp_b200.h cstp_stem_dgrad)."""
+    _require_cuda(g, w, dx)
+    if dx.dtype != torch.float32 or dx.dim() != 5 or dx.shape[1] != 3 or not dx.is_contiguous():
+        raise L.CstpError(f"stem input gradient: dx must be contiguous fp32 (N, 3, T, H, W), got {dx.dtype} {tuple(dx.shape)}")
+    N, _, T, H, W = dx.shape
+    if H % 2 or W % 4:
+        raise L.CstpError(f"stem input gradient: H must be even and W a multiple of 4, got {H} x {W}")
+    if g.dtype != torch.bfloat16 or not g.is_contiguous() or tuple(g.shape[:4]) != (N, T, H // 2, W // 2):
+        raise L.CstpError(f"stem input gradient: d(raw) must be contiguous bf16 ({N}, {T}, {H // 2}, {W // 2}, C), "
+                          f"got {g.dtype} {tuple(g.shape)}")
+    if w.dtype != torch.float32 or not w.is_contiguous() or tuple(w.shape[1:]) != (3, 1, 7, 7) or w.shape[0] > g.shape[4]:
+        raise L.CstpError(f"stem input gradient: weight must be contiguous fp32 (cout <= {g.shape[4]}, 3, 1, 7, 7), "
+                          f"got {w.dtype} {tuple(w.shape)}")
+    L.check(L.load().cstp_stem_dgrad(_ptr(g), g.shape[4], _ptr(w), w.shape[0], _ptr(dx), N, T, H, W, _stream()))
+
+
 BN_REDUCE_CTAS_PER_SM = 2         # per statistics group (co-residency sweep: profiles/r01_overlap_sweep.txt)
 
 

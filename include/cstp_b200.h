@@ -289,6 +289,14 @@ int cstp_pack_weights_batched(const int64_t* jobs_dev, const int64_t* prefix_dev
  * implicit GEMM over P (row pairs ho-2 .. ho+1) whose packed weights come from cstp_pack_weight(s) with transpose = 2
  * and whose weight gradient is scattered by cstp_wgrad_finalize layout 1. */
 int cstp_stem_pack(const float* x, int N, int T, int H, int W, void* P, void* stream);
+/* Input gradient of the same convolution: g is the stem unit's d(raw), bf16 (N,T,H/2,W/2,Cg) with Cg even and >= cout;
+ * w the fp32 (cout, 3, 1, 7, 7) weight (rounded to bf16 on load, as the packed weights of every dgrad are); dx the fp32
+ * NCDHW (N,3,T,H,W) clip gradient, overwritten.  dx[n][c][t][h][w] = sum of g[n][t][oh][ow][co] * w[co][c][0][kh][kw]
+ * over oh = (h + 3 - kh) / 2, ow = (w + 3 - kw) / 2 integral and in range, summed in a fixed order (channel pairs, kh,
+ * kw, channel) with one fmaf per term and no atomics (csrc/stem_dgrad.cu).  H even, W a multiple of 4, cout <= 128,
+ * g 4-byte and dx 16-byte aligned. */
+int cstp_stem_dgrad(const void* g, int Cg, const float* w, int cout, float* dx, int N, int T, int H, int W,
+                    void* stream);
 
 /* ---- BatchNorm (training mode), fused with ReLU / residual ---------------------------------------------
  * Replaces nn.BatchNorm3d / BatchNorm1d forward+backward and the ReLU / residual adds around them
