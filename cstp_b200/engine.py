@@ -20,6 +20,10 @@ Data layout in HBM
 
 Everything is launched on the current CUDA stream through the C ABI (cstp_b200.ops); torch is only used for
 memory, streams and torch.distributed.  There is no CPU path.
+
+Classes: ProgramEngine holds what every engine shares (stores, program builders, backward, weight packs, CUDA-graph
+capture); OptimizerEngine adds the fused optimiser; StepEngine is the pretraining step.  The finetune, inference and
+backbone engines (engine_ft, engine_backbone) build on the same two bases.
 """
 from __future__ import annotations
 
@@ -160,13 +164,11 @@ def trainable_param_specs():
 def bn_buffer_specs(param_specs):
     """running_mean / running_var for every BatchNorm (a 1-D `.weight` whose sibling `.bias` is also 1-D and whose
     module is not a Linear: identified by the absence of a 2-D/5-D weight under the same module name)."""
-    shapes = dict(param_specs)
     out = []
     for name, shape in param_specs:
         if name.endswith(".weight") and len(shape) == 1:
             mod = name[:-len(".weight")]
             out += [(mod + ".running_mean", shape), (mod + ".running_var", shape)]
-    del shapes
     return out
 
 
@@ -206,31 +208,29 @@ class _Timed:
         prof.append((self.kind, self.flops, len(self.plans), a, b, self.tag, ops.kernel_name(self.plans[0])))
 
 
-class StepEngine:
-    """See the module docstring.  `B` is the per-GPU batch (samples; each sample is two views)."""
+class ProgramEngine:
+    """What every engine shares: the clip geometry, the flat parameter and BatchNorm-buffer stores, the builders of the
+    backbone / MLP launch programs over them, the backward program with its gradient buckets, the bf16 weight packs and
+    the CUDA-graph capture of a program.  `B` is the batch (samples; each sample is VIEWS clips, one BatchNorm statistics
+    group each).  `specs`: the parameters of the `train` store; `share`: an engine whose parameter and BatchNorm-buffer
+    stores this one reads (None: they are allocated here); `grads`: the engine builds a backward program and has a `grad`
+    store; `bn_specs`: parameters outside `train` whose BatchNorm running statistics live in `bufs` too."""
 
-    VIEWS = 2          # clips per sample pushed through the backbone = BatchNorm statistics groups
+    VIEWS = 1          # clips per sample pushed through the backbone = BatchNorm statistics groups
 
-    def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", momentum_ema: float = 0.996,
+    def __init__(self, B: int, T: int, H: int, W: int, device, specs, *, grads: bool, share=None, bn_specs=(),
                  record: bool = False, overlap: bool = True, bn_sync=None, fuse_apply: bool | None = None,
-                 ntxent: dict | None = None, fuse_min_positions: int | None = None, fuse_policy: str | None = None,
-                 graph: bool | None = None, collapse_stats: bool = False):
+                 fuse_min_positions: int | None = None, fuse_policy: str | None = None, graph: bool | None = None):
         if H % 2 or W % 4:
             raise ops.L.CstpError("clip height must be even and its width a multiple of 4 (1x7x7 stride-2 stem over packed rows)")
         self.B, self.T, self.H, self.W = B, T, H, W
         self.N = self.VIEWS * B
         self.device = torch.device(device)
-        self.momentum_ema = momentum_ema
         self.record = record
         self.eval_mode = False       # True: BatchNorm uses its running statistics (finetune validation / test)
         # None: per-GPU BatchNorm statistics (what the reference's --sync_bn actually does, SURVEY.md 0.2);
         # a cstp_b200.parallel.BnSync: statistics over every rank of the data-parallel group (north-star SyncBN)
         self.bn_sync = bn_sync
-        # optional NT-Xent term on the online projector outputs of the two views (north-star extension: the reference
-        # builds NTXentLoss but never calls it, SURVEY.md 0.1): dict(weight, temperature, gather) -- with gather the
-        # embeddings of every rank are all-gathered first, so each rank contrasts against the GLOBAL batch
-        # (loss/NTXent.py:46-62 with batch_size = opts.batch_size, main_byol.py:191-196)
-        self.ntxent = dict(ntxent) if ntxent else None
         # Two-stream schedule (CUDA only): the target network's forward runs beside the online network's, and every
         # weight-gradient GEMM runs beside the BatchNorm-backward streaming kernels of the next unit, so HBM-bound and
         # tensor-bound kernels share the machine.  Results are unchanged (same kernels, same reduction orders).
@@ -244,10 +244,9 @@ class StepEngine:
                 bn_sync.register_side_stream(self._s2)
         self._wg_recorded = [False, False]     # has _ev_wg[b] been recorded during the CURRENT backward pass?
         self.use_graph = (USE_GRAPH if graph is None else bool(graph)) and self.device.type == "cuda" and not record
-        self._graph = None
-        self._graph_key = None
-        self._graph_launches = 0
-        self._eager_steps = 0
+        self._graphs: dict[str, tuple] = {}    # purpose -> (key, CUDA graph, launches per replay): see _captured
+        self._ran_eager: set[str] = set()      # purposes whose program has run eagerly once
+        self._packed_key = None                # see repack
         self.fuse_apply = FUSE_BN_APPLY if fuse_apply is None else bool(fuse_apply)
         self.fuse_min_positions = FUSE_MIN_POSITIONS if fuse_min_positions is None else int(fuse_min_positions)
         self.fuse_policy = fuse_policy or FUSE_POLICY
@@ -258,13 +257,17 @@ class StepEngine:
         self.named: dict[str, torch.Tensor] = {}      # name -> activation / gradient tensors (parity tests)
         self.units: list[dict] = []                   # every conv+BN unit in build order (parity tests, profiling)
         self._prof = None                             # list of (kind, flops, launches, ev0, ev1) while profiling
-        f32 = dict(device=self.device, dtype=torch.float32)
 
-        self._make_stores()
-        self.first_step = True       # no optimiser state yet (SGD momentum / Adam moments)
-        self.optim_kind = "sgd"      # the optimiser the state belongs to (OPTIMIZERS)
-        self.adam_step = 0           # Adam / AdamW steps taken (torch's per-parameter `step`)
-        self.exp_avg = self.exp_avg_sq = self.adam_hyper = None
+        # ---- flat parameter / gradient / BatchNorm-buffer stores
+        if share is None:
+            self.train = FlatStore(specs, self.device)
+            self.bufs = FlatStore(bn_buffer_specs(list(specs) + list(bn_specs)), self.device)
+            for name in self.bufs.slots:
+                if name.endswith("running_var"):
+                    self.bufs.view(name).fill_(1.0)
+        else:
+            self.train, self.bufs = share.train, share.bufs
+        self.grad = self.train.like() if grads else None
 
         # ---- scratch shared by all layers
         self._g_numel = 0            # bf16 d(raw) scratch, sized while building
@@ -282,35 +285,6 @@ class StepEngine:
         # ---- inputs
         # stem input: the seven kw taps x three channels of every output column, two frame rows per pixel (ops.stem_pack)
         self.stem_rows = torch.zeros(self.N, T, H // 2, W // 2, ops.STEM_CHANNELS, device=self.device, dtype=ACT_DTYPE)
-        self.weights5 = torch.tensor([0.1, 1.0, 1.0, 1.0, 1.0], **f32)
-        self.losses = torch.zeros(8, **f32)       # [0..5] CE, [6] weighted CE sum, [7] BYOL loss
-        # collapse statistics (cstp_repr_stats) of the last forward run with collapse_stats on: [view][REPR_STATS].
-        # Changing the flag changes the step program: drop a captured graph first (R21DBYOL.train_step does).
-        self.collapse_stats = bool(collapse_stats)
-        self.step_stats = torch.zeros(2, len(REPR_STATS), **f32)
-        self.norm_out = torch.zeros(2, **f32)
-        self.sgd_ws = torch.zeros(2048, **f32)
-        # static inputs of the captured step: integer labels (spa, tem, pb, rot1, rot2) and the optimiser's hyper-parameters
-        # {lr, momentum, wd, max_norm, do_clip, first_step} (cstp_sgd_clip_step_dev)
-        self.labels_static = tuple(torch.zeros(B, dtype=torch.int64, device=self.device) for _ in range(5))
-        self.hyper = torch.zeros(8, **f32)
-        self._hyper_host = None
-
-        self._build()
-
-    def _make_stores(self):
-        """Flat parameter / gradient / momentum / buffer stores (overridden by the finetune engine)."""
-        tspecs = trainable_param_specs()
-        self.train = FlatStore(tspecs, self.device)
-        self.grad = self.train.like()
-        self.mom = self.train.like()
-        self.target = FlatStore(backbone_param_specs("target_net"), self.device)
-        self.online_numel = FlatStore(backbone_param_specs("online_net"), "meta").numel
-        assert self.online_numel == self.target.numel
-        self.bufs = FlatStore(bn_buffer_specs(tspecs) + bn_buffer_specs(backbone_param_specs("target_net")), self.device)
-        for name in self.bufs.slots:
-            if name.endswith("running_var"):
-                self.bufs.view(name).fill_(1.0)
 
     # ------------------------------------------------------------------------------------------ helpers
     def _act(self, *shape) -> torch.Tensor:
@@ -351,6 +325,53 @@ class StepEngine:
         (self._pack_jobs_online if store is self.train else self._pack_jobs_target).append((w, wp, wt, 2 if stem else 0))
         return wp, wt
 
+    def _bn_forward(self, raw, site: _Site, fused_blocks: int = 0):
+        """BatchNorm forward of `site` over raw: in eval mode (model.eval()) the affine map of the running statistics,
+        nothing is updated; otherwise the batch statistics, which also update the running buffers."""
+        if self.eval_mode:
+            ops.bn_eval_coeffs(site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS)
+        else:
+            ops.bn_forward_stats(raw, site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS, BN_MOMENTUM,
+                                 fused_blocks=fused_blocks, sync=self.bn_sync)
+
+    def _captured(self, purpose: str, key, body) -> None:
+        """Runs body() -- a program that reads and writes engine-owned buffers only -- eagerly the first time this engine
+        runs a program for `purpose` (one-time kernel attributes, NCCL / peer-memory channel set-up), captures it into a
+        CUDA graph on the next call and replays that graph from then on.  Another `key` captures again; each purpose keeps
+        one graph.  Inputs are written into the static buffers body() reads before the call, outside the graph."""
+        held = self._graphs.get(purpose)
+        if held is not None and held[0] == key:
+            held[1].replay()
+            ops.note_replayed(held[2])
+            return
+        if purpose not in self._ran_eager or not self.use_graph:
+            self._ran_eager.add(purpose)
+            body()
+            return
+        torch.cuda.synchronize(self.device)
+        before = ops.launch_count()
+        g = torch.cuda.CUDAGraph()
+        try:
+            # thread_local: NCCL's watchdog thread and the data loader's copy stream keep issuing CUDA calls meanwhile
+            with torch.cuda.graph(g, capture_error_mode="thread_local"):
+                body()
+        except Exception as e:          # e.g. a collective backend that cannot be captured: stay eager, say so once
+            import warnings
+            warnings.warn(f"cstp_b200: CUDA-graph capture of the {purpose} program failed ({e!r}); running eagerly")
+            self.use_graph = False
+            torch.cuda.synchronize(self.device)
+            body()
+            return
+        launches = ops.launch_count() - before
+        self._graphs[purpose] = (key, g, launches)
+        ops.note_replayed(-launches)       # the capture pass counted launches that did not run
+        g.replay()
+        ops.note_replayed(launches)
+
+    def _forward_program(self):
+        for op in self.fwd_online:
+            op()
+
     # ------------------------------------------------------------------------------------------ conv + BN unit
     def _conv_bn(self, prog, store, grads, x, wname, bnname, geom: ConvGeom, cin, cout, *, relu=True, res=None,
                  res_site=None, apply=True, tag="", skip_dgrad=False, stem=False):
@@ -383,11 +404,7 @@ class StepEngine:
 
         def fwd():
             plan.run()
-            if self.eval_mode:       # model.eval(): running statistics as an affine map, nothing is updated
-                ops.bn_eval_coeffs(site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS)
-            else:
-                ops.bn_forward_stats(raw, site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS, BN_MOMENTUM,
-                                     fused_blocks=fused, sync=self.bn_sync)
+            self._bn_forward(raw, site, fused)
             if keep_act:
                 ops.bn_apply(raw, site.st, act, relu=relu, res=res, res_state=res_state, res_relu=res_pro is not None)
         prog.append(fwd)
@@ -567,11 +584,7 @@ class StepEngine:
 
         def fwd():
             p0.run()
-            if self.eval_mode:       # model.eval() of a standalone R2Plus1DNet's projector (engine_backbone)
-                ops.bn_eval_coeffs(site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS)
-            else:
-                ops.bn_forward_stats(raw, site.st, site.gamma, site.beta, site.rm, site.rv, BN_EPS, BN_MOMENTUM,
-                                     sync=self.bn_sync)
+            self._bn_forward(raw, site)
             ops.bn_apply(raw, site.st, h, relu=True)
             p3.run()
         prog.append(fwd)
@@ -627,6 +640,232 @@ class StepEngine:
             return bwd
         res["make_backward"] = make_backward
         return res
+
+    # ------------------------------------------------------------------------------------------ build
+    def _finish_build(self):
+        """Shared scratch + deferred plan creation, once every forward / backward closure exists."""
+        f32 = dict(device=self.device, dtype=torch.float32)
+        # d(raw) scratch: two buffers, alternating in RUN order, so that a unit's weight-gradient GEMM (side stream) can
+        # still read its d(raw) while the next unit's BatchNorm backward writes the other buffer
+        turn = 0
+        for op in self.bwd:
+            h = getattr(op, "holder", None)
+            if h is not None:
+                h["gbuf"] = turn
+                turn ^= 1 if self.overlap else 0
+        self._gbufs = [self._act(self._g_numel)]
+        self._gbufs.append(self._act(self._g_numel) if self.overlap else self._gbufs[0])
+        self._wg = torch.zeros(self._wg_numel, **f32)
+        for fn in self._deferred:
+            fn()
+        self._deferred.clear()
+        self._plan_grad_buckets()
+
+    GRAD_BUCKET_MIN = 3_000_000      # elements (12 MB of fp32): below this an all-reduce is latency, not bandwidth
+
+    def _plan_grad_buckets(self):
+        """Where the data-parallel gradient all-reduce can start before the backward pass has finished.  The flat gradient
+        buffer is laid out in registration order and the backward program runs (roughly) in the reverse order, so after
+        closure i every slot at or above a low-water mark is final: {closure index: (lo, hi)} hands the newly finished
+        tail [lo, hi) to the communication stream whenever it has grown past GRAD_BUCKET_MIN; the last closure sends the
+        rest.  (DDP's bucketed hooks, models/model.py:97-103, on one contiguous buffer.)"""
+        slots = self.train.slots
+        order = sorted(slots.items(), key=lambda kv: kv[1][0])           # (name, (offset, shape)) by offset
+        remaining = {n: 0 for n in slots}
+        for op in self.bwd:
+            for n in getattr(op, "writes", ()):
+                if n in remaining:
+                    remaining[n] += 1
+        never = {n for n, c in remaining.items() if c == 0}              # parameters no closure writes (frozen backbone)
+        self._grad_buckets, sent = {}, self.train.numel
+        for i, op in enumerate(self.bwd):
+            for n in getattr(op, "writes", ()):
+                if n in remaining:
+                    remaining[n] -= 1
+            mark = self.train.numel
+            for n, (off, _) in reversed(order):
+                if remaining[n] > 0 and n not in never:
+                    break
+                mark = off
+            last = i == len(self.bwd) - 1
+            if last:
+                mark = 0
+            if sent - mark >= (1 if last else self.GRAD_BUCKET_MIN):
+                self._grad_buckets[i] = (mark, sent)
+                sent = mark
+        if self.device.type == "cuda":
+            self._bucket_events = {i: torch.cuda.Event() for i in self._grad_buckets}
+
+    # ------------------------------------------------------------------------------------------ programs
+    def _pack_list(self, jobs):
+        flat = []
+        for w, wp, wt, mode in jobs:
+            flat.append((w, wp, mode))
+            if wt is not None:
+                flat.append((w, wt, 1))
+        return ops.PackList(flat, self.device)
+
+    def pack_online(self):
+        """fp32 master weights -> bf16 tensor-core copies (forward and dgrad-transposed), one launch for the network."""
+        if getattr(self, "_pl_online", None) is None:
+            self._pl_online = self._pack_list(self._pack_jobs_online)
+        self._pl_online.run()
+
+    def pack_target(self):
+        if getattr(self, "_pl_target", None) is None:
+            self._pl_target = self._pack_list(self._pack_jobs_target)
+        self._pl_target.run()
+
+    def repack(self, key, packed: bool = False) -> None:
+        """Re-packs the bf16 weights unless they were last packed at `key`, the caller's version of the fp32 parameters
+        (which other engines may share and change); packed=True only records that they are current at `key` (the
+        optimiser step that changed them re-packed them)."""
+        if key != self._packed_key and not packed:
+            self.pack_online()
+        self._packed_key = key
+
+    def backward(self, grad_sync=None):
+        """Runs the backward program.  `grad_sync` (a parallel.GradSync): finished tails of the flat gradient buffer are
+        all-reduced on its communication stream while the rest of the backward pass still runs (call grad_sync.finish()
+        before the optimiser); returns True when the buffer was handed over that way."""
+        bucketed = grad_sync is not None and hasattr(grad_sync, "bucket") and self._prof is None
+        side = self.overlap and self._prof is None
+        self._wg_recorded = [False, False]
+        for i, op in enumerate(self.bwd):
+            op()
+            if bucketed and i in self._grad_buckets:
+                lo, hi = self._grad_buckets[i]
+                events = []
+                if self.device.type == "cuda":
+                    ev = self._bucket_events[i]
+                    ev.record()
+                    events = [ev] + ([e for e, r in zip(self._ev_wg, self._wg_recorded) if r] if side else [])
+                grad_sync.bucket(self.grad[lo:hi], events)
+        if side:
+            main = torch.cuda.current_stream()
+            for e, r in zip(self._ev_wg, self._wg_recorded):
+                if r:
+                    main.wait_event(e)
+        return bucketed
+
+
+class OptimizerEngine(ProgramEngine):
+    """An engine that steps an optimiser over its whole flat parameter buffer (the pretraining and finetune engines):
+    global-norm clip + SGD momentum or Adam / AdamW, with their state mirroring `train`, then the bf16 re-pack."""
+
+    def __init__(self, *args, **kwargs):
+        super().__init__(*args, grads=True, **kwargs)
+        f32 = dict(device=self.device, dtype=torch.float32)
+        self.mom = self.train.like()
+        self.first_step = True       # no optimiser state yet (SGD momentum / Adam moments)
+        self.optim_kind = "sgd"      # the optimiser the state belongs to (OPTIMIZERS)
+        self.adam_step = 0           # Adam / AdamW steps taken (torch's per-parameter `step`)
+        self.exp_avg = self.exp_avg_sq = self.adam_hyper = None
+        self.norm_out = torch.zeros(2, **f32)
+        self.sgd_ws = torch.zeros(2048, **f32)
+        # the hyper-parameters of a captured SGD step {lr, momentum, wd, max_norm, do_clip, first_step}
+        # (cstp_sgd_clip_step_dev)
+        self.hyper = torch.zeros(8, **f32)
+        self._hyper_host = None
+
+    def select_optimizer(self, kind: str) -> None:
+        """Binds the optimiser `kind` (OPTIMIZERS) for the next step.  Adam's state buffers (exp_avg / exp_avg_sq mirrors
+        of the trainable buffer) are allocated when Adam first runs, so an SGD run holds nothing extra.  Optimiser state
+        belongs to one kind: asking for another while it exists raises ValueError."""
+        if kind not in OPTIMIZERS:
+            raise ValueError(f"optimizer {kind!r}: expected one of {OPTIMIZERS}")
+        if kind != self.optim_kind and not self.first_step:
+            raise ValueError(f"the engine holds {self.optim_kind} optimiser state; it cannot continue as {kind}")
+        self.optim_kind = kind
+        if kind == "sgd":
+            return
+        if self.exp_avg is None:
+            self.exp_avg, self.exp_avg_sq = self.train.like(), self.train.like()
+            self.adam_hyper = torch.zeros(len(ops.L.AdamHyper._fields_), device=self.device, dtype=torch.float32)
+        elif self.first_step:
+            self.exp_avg.zero_()
+            self.exp_avg_sq.zero_()
+        if self.first_step:
+            self.adam_step = 0
+
+    def _next_adam(self, lr, betas, eps, wd, max_norm, clip) -> tuple:
+        self.adam_step += 1
+        return adam_scalars(self.adam_step, lr, betas, eps, wd, self.optim_kind == "adamw", max_norm, clip)
+
+    def take_optimizer_state(self, other: "StepEngine") -> None:
+        """Continues the optimiser of `other`, an engine of another batch geometry over the same parameter layout that is
+        about to be dropped (its Adam moments are taken over, not copied)."""
+        self.mom.copy_(other.mom)
+        self.first_step, self.optim_kind, self.adam_step = other.first_step, other.optim_kind, other.adam_step
+        self.exp_avg, self.exp_avg_sq, self.adam_hyper = other.exp_avg, other.exp_avg_sq, other.adam_hyper
+
+    def optimizer_step(self, lr, momentum=0.9, wd=5e-4, max_norm=18.0, clip=True, optimizer="sgd", betas=(0.9, 0.999),
+                       eps=1e-8):
+        """clip_grad_norm_ + SGD.step (main_byol.py:88-91,229-232), or + Adam / AdamW.step (`momentum` unused), on the flat
+        buffers, then re-pack the bf16 weights."""
+        self.select_optimizer(optimizer)
+        n = self.train.numel
+        if optimizer == "sgd":
+            ops.sgd_clip_step(self.train.data[:n], self.grad[:n], self.mom[:n], lr, momentum, wd, max_norm, clip,
+                              self.first_step, self.norm_out, self.sgd_ws)
+        else:
+            ops.adam_clip_step(self.train.data[:n], self.grad[:n], self.exp_avg[:n], self.exp_avg_sq[:n],
+                               self._next_adam(lr, betas, eps, wd, max_norm, clip), self.norm_out, self.sgd_ws)
+        self.first_step = False
+        self.pack_online()
+
+    def set_hyper(self, lr, momentum, wd, max_norm, clip) -> None:
+        """Writes the optimiser's hyper-parameters (and the first-step flag) into device memory when they changed."""
+        h = (float(lr), float(momentum), float(wd), float(max_norm), 1.0 if clip else 0.0, 1.0 if self.first_step else 0.0)
+        if h != self._hyper_host:
+            self.hyper[:6].copy_(torch.tensor(h, dtype=torch.float32), non_blocking=False)
+            self._hyper_host = h
+
+    def set_adam_hyper(self, lr, betas, eps, wd, max_norm, clip) -> None:
+        """Writes the scalars of the next Adam / AdamW step into device memory, in stream order ahead of the step (through
+        pinned memory, which torch's host allocator keeps until the copy has run: the host does not wait)."""
+        h = torch.tensor(self._next_adam(lr, betas, eps, wd, max_norm, clip), dtype=torch.float32)
+        self.adam_hyper.copy_(h.pin_memory(), non_blocking=True)
+
+
+class StepEngine(OptimizerEngine):
+    """See the module docstring.  `B` is the per-GPU batch (samples; each sample is two views)."""
+
+    VIEWS = 2
+
+    def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", momentum_ema: float = 0.996,
+                 record: bool = False, overlap: bool = True, bn_sync=None, fuse_apply: bool | None = None,
+                 ntxent: dict | None = None, fuse_min_positions: int | None = None, fuse_policy: str | None = None,
+                 graph: bool | None = None, collapse_stats: bool = False):
+        target_specs = backbone_param_specs("target_net")
+        super().__init__(B, T, H, W, device, trainable_param_specs(), bn_specs=target_specs, record=record,
+                         overlap=overlap, bn_sync=bn_sync, fuse_apply=fuse_apply, fuse_min_positions=fuse_min_positions,
+                         fuse_policy=fuse_policy, graph=graph)
+        self.momentum_ema = momentum_ema
+        # optional NT-Xent term on the online projector outputs of the two views (north-star extension: the reference
+        # builds NTXentLoss but never calls it, SURVEY.md 0.1): dict(weight, temperature, gather) -- with gather the
+        # embeddings of every rank are all-gathered first, so each rank contrasts against the GLOBAL batch
+        # (loss/NTXent.py:46-62 with batch_size = opts.batch_size, main_byol.py:191-196)
+        self.ntxent = dict(ntxent) if ntxent else None
+        self.target = FlatStore(target_specs, self.device)
+        self.online_numel = FlatStore(backbone_param_specs("online_net"), "meta").numel
+        assert self.online_numel == self.target.numel
+        f32 = dict(device=self.device, dtype=torch.float32)
+        self.weights5 = torch.tensor([0.1, 1.0, 1.0, 1.0, 1.0], **f32)
+        self.losses = torch.zeros(8, **f32)       # [0..5] CE, [6] weighted CE sum, [7] BYOL loss
+        # collapse statistics (cstp_repr_stats) of the last forward run with collapse_stats on: [view][REPR_STATS].
+        # Changing the flag changes the step program: drop a captured graph first (R21DBYOL.train_step does).
+        self.collapse_stats = bool(collapse_stats)
+        self.step_stats = torch.zeros(2, len(REPR_STATS), **f32)
+        # static integer labels (spa, tem, pb, rot1, rot2) of the captured step
+        self.labels_static = tuple(torch.zeros(B, dtype=torch.int64, device=self.device) for _ in range(5))
+        self._build()
+
+    @property
+    def _graph(self):
+        """The captured training step (graphed_step); None until it has been captured."""
+        held = self._graphs.get("step")
+        return held and held[1]
 
     # ------------------------------------------------------------------------------------------ build
     def _build(self):
@@ -688,60 +927,6 @@ class StepEngine:
         # ---------------- shared scratch + deferred plan creation
         self._finish_build()
 
-    def _finish_build(self):
-        """Shared scratch + deferred plan creation, once every forward / backward closure exists."""
-        f32 = dict(device=self.device, dtype=torch.float32)
-        # d(raw) scratch: two buffers, alternating in RUN order, so that a unit's weight-gradient GEMM (side stream) can
-        # still read its d(raw) while the next unit's BatchNorm backward writes the other buffer
-        turn = 0
-        for op in self.bwd:
-            h = getattr(op, "holder", None)
-            if h is not None:
-                h["gbuf"] = turn
-                turn ^= 1 if self.overlap else 0
-        self._gbufs = [self._act(self._g_numel)]
-        self._gbufs.append(self._act(self._g_numel) if self.overlap else self._gbufs[0])
-        self._wg = torch.zeros(self._wg_numel, **f32)
-        for fn in self._deferred:
-            fn()
-        self._deferred.clear()
-        self._plan_grad_buckets()
-
-    GRAD_BUCKET_MIN = 3_000_000      # elements (12 MB of fp32): below this an all-reduce is latency, not bandwidth
-
-    def _plan_grad_buckets(self):
-        """Where the data-parallel gradient all-reduce can start before the backward pass has finished.  The flat gradient
-        buffer is laid out in registration order and the backward program runs (roughly) in the reverse order, so after
-        closure i every slot at or above a low-water mark is final: {closure index: (lo, hi)} hands the newly finished
-        tail [lo, hi) to the communication stream whenever it has grown past GRAD_BUCKET_MIN; the last closure sends the
-        rest.  (DDP's bucketed hooks, models/model.py:97-103, on one contiguous buffer.)"""
-        slots = self.train.slots
-        order = sorted(slots.items(), key=lambda kv: kv[1][0])           # (name, (offset, shape)) by offset
-        remaining = {n: 0 for n in slots}
-        for op in self.bwd:
-            for n in getattr(op, "writes", ()):
-                if n in remaining:
-                    remaining[n] += 1
-        never = {n for n, c in remaining.items() if c == 0}              # parameters no closure writes (frozen backbone)
-        self._grad_buckets, sent = {}, self.train.numel
-        for i, op in enumerate(self.bwd):
-            for n in getattr(op, "writes", ()):
-                if n in remaining:
-                    remaining[n] -= 1
-            mark = self.train.numel
-            for n, (off, _) in reversed(order):
-                if remaining[n] > 0 and n not in never:
-                    break
-                mark = off
-            last = i == len(self.bwd) - 1
-            if last:
-                mark = 0
-            if sent - mark >= (1 if last else self.GRAD_BUCKET_MIN):
-                self._grad_buckets[i] = (mark, sent)
-                sent = mark
-        if self.device.type == "cuda":
-            self._bucket_events = {i: torch.cuda.Event() for i in self._grad_buckets}
-
     # ------------------------------------------------------------------------------------------ NT-Xent term
     def _ntxent_setup(self):
         import torch.distributed as dist
@@ -783,26 +968,6 @@ class StepEngine:
         a = float(self.ntxent["weight"]) * W
         self.dproj[:B, :512].add_(dz[1, r], alpha=a)
         self.dproj[B:, :512].add_(dz[0, r], alpha=a)
-
-    # ------------------------------------------------------------------------------------------ programs
-    def _pack_list(self, jobs):
-        flat = []
-        for w, wp, wt, mode in jobs:
-            flat.append((w, wp, mode))
-            if wt is not None:
-                flat.append((w, wt, 1))
-        return ops.PackList(flat, self.device)
-
-    def pack_online(self):
-        """fp32 master weights -> bf16 tensor-core copies (forward and dgrad-transposed), one launch for the network."""
-        if getattr(self, "_pl_online", None) is None:
-            self._pl_online = self._pack_list(self._pack_jobs_online)
-        self._pl_online.run()
-
-    def pack_target(self):
-        if getattr(self, "_pl_target", None) is None:
-            self._pl_target = self._pack_list(self._pack_jobs_target)
-        self._pl_target.run()
 
     def load_clips(self, x1: torch.Tensor, x2: torch.Tensor):
         """fp32 NCDHW clips (B,3,T,H,W) -> bf16 packed stem rows (shared by the online and target nets)."""
@@ -855,90 +1020,7 @@ class StepEngine:
         spa, tem, pb, r1, r2 = labels5
         ops.pretext_ce(self.logits6, (spa, tem, pb, pb, r1, r2), self.dlogits6, self.B, 5, self.weights5, self.losses)
 
-    def backward(self, grad_sync=None):
-        """Runs the backward program.  `grad_sync` (a parallel.GradSync): finished tails of the flat gradient buffer are
-        all-reduced on its communication stream while the rest of the backward pass still runs (call grad_sync.finish()
-        before the optimiser); returns True when the buffer was handed over that way."""
-        bucketed = grad_sync is not None and hasattr(grad_sync, "bucket") and self._prof is None
-        side = self.overlap and self._prof is None
-        self._wg_recorded = [False, False]
-        for i, op in enumerate(self.bwd):
-            op()
-            if bucketed and i in self._grad_buckets:
-                lo, hi = self._grad_buckets[i]
-                events = []
-                if self.device.type == "cuda":
-                    ev = self._bucket_events[i]
-                    ev.record()
-                    events = [ev] + ([e for e, r in zip(self._ev_wg, self._wg_recorded) if r] if side else [])
-                grad_sync.bucket(self.grad[lo:hi], events)
-        if side:
-            main = torch.cuda.current_stream()
-            for e, r in zip(self._ev_wg, self._wg_recorded):
-                if r:
-                    main.wait_event(e)
-        return bucketed
-
-    def select_optimizer(self, kind: str) -> None:
-        """Binds the optimiser `kind` (OPTIMIZERS) for the next step.  Adam's state buffers (exp_avg / exp_avg_sq mirrors
-        of the trainable buffer) are allocated when Adam first runs, so an SGD run holds nothing extra.  Optimiser state
-        belongs to one kind: asking for another while it exists raises ValueError."""
-        if kind not in OPTIMIZERS:
-            raise ValueError(f"optimizer {kind!r}: expected one of {OPTIMIZERS}")
-        if kind != self.optim_kind and not self.first_step:
-            raise ValueError(f"the engine holds {self.optim_kind} optimiser state; it cannot continue as {kind}")
-        self.optim_kind = kind
-        if kind == "sgd":
-            return
-        if self.exp_avg is None:
-            self.exp_avg, self.exp_avg_sq = self.train.like(), self.train.like()
-            self.adam_hyper = torch.zeros(len(ops.L.AdamHyper._fields_), device=self.device, dtype=torch.float32)
-        elif self.first_step:
-            self.exp_avg.zero_()
-            self.exp_avg_sq.zero_()
-        if self.first_step:
-            self.adam_step = 0
-
-    def _next_adam(self, lr, betas, eps, wd, max_norm, clip) -> tuple:
-        self.adam_step += 1
-        return adam_scalars(self.adam_step, lr, betas, eps, wd, self.optim_kind == "adamw", max_norm, clip)
-
-    def take_optimizer_state(self, other: "StepEngine") -> None:
-        """Continues the optimiser of `other`, an engine of another batch geometry over the same parameter layout that is
-        about to be dropped (its Adam moments are taken over, not copied)."""
-        self.mom.copy_(other.mom)
-        self.first_step, self.optim_kind, self.adam_step = other.first_step, other.optim_kind, other.adam_step
-        self.exp_avg, self.exp_avg_sq, self.adam_hyper = other.exp_avg, other.exp_avg_sq, other.adam_hyper
-
-    def optimizer_step(self, lr, momentum=0.9, wd=5e-4, max_norm=18.0, clip=True, optimizer="sgd", betas=(0.9, 0.999),
-                       eps=1e-8):
-        """clip_grad_norm_ + SGD.step (main_byol.py:88-91,229-232), or + Adam / AdamW.step (`momentum` unused), on the flat
-        buffers, then re-pack the bf16 weights."""
-        self.select_optimizer(optimizer)
-        n = self.train.numel
-        if optimizer == "sgd":
-            ops.sgd_clip_step(self.train.data[:n], self.grad[:n], self.mom[:n], lr, momentum, wd, max_norm, clip,
-                              self.first_step, self.norm_out, self.sgd_ws)
-        else:
-            ops.adam_clip_step(self.train.data[:n], self.grad[:n], self.exp_avg[:n], self.exp_avg_sq[:n],
-                               self._next_adam(lr, betas, eps, wd, max_norm, clip), self.norm_out, self.sgd_ws)
-        self.first_step = False
-        self.pack_online()
-
     # ------------------------------------------------------------------------------------------ captured step
-    def set_hyper(self, lr, momentum, wd, max_norm, clip) -> None:
-        """Writes the optimiser's hyper-parameters (and the first-step flag) into device memory when they changed."""
-        h = (float(lr), float(momentum), float(wd), float(max_norm), 1.0 if clip else 0.0, 1.0 if self.first_step else 0.0)
-        if h != self._hyper_host:
-            self.hyper[:6].copy_(torch.tensor(h, dtype=torch.float32), non_blocking=False)
-            self._hyper_host = h
-
-    def set_adam_hyper(self, lr, betas, eps, wd, max_norm, clip) -> None:
-        """Writes the scalars of the next Adam / AdamW step into device memory, in stream order ahead of the step (through
-        pinned memory, which torch's host allocator keeps until the copy has run: the host does not wait)."""
-        h = torch.tensor(self._next_adam(lr, betas, eps, wd, max_norm, clip), dtype=torch.float32)
-        self.adam_hyper.copy_(h.pin_memory(), non_blocking=True)
-
     def _step_body(self, grad_sync, after):
         """forward (behind the input pass) -> pretext losses -> backward (+ gradient all-reduce) -> optimiser -> re-pack,
         on engine-owned buffers only: the program graphed_step captures."""
@@ -974,37 +1056,11 @@ class StepEngine:
             self.set_hyper(lr, momentum, wd, max_norm, clip)
         else:
             self.set_adam_hyper(lr, betas, eps, wd, max_norm, clip)
-        key = (id(grad_sync), optimizer)
-        if self._graph is not None and self._graph_key == key:
-            self._graph.replay()
-            ops.note_replayed(self._graph_launches)
-        elif self._eager_steps < 1 or not self.use_graph:
-            self._step_body(grad_sync, after)
-            self._eager_steps += 1
-        else:
-            torch.cuda.synchronize(self.device)
-            before = ops.launch_count()
-            g = torch.cuda.CUDAGraph()
-            try:
-                # thread_local: NCCL's watchdog thread and the data loader's copy stream keep issuing CUDA calls meanwhile
-                with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                    self._step_body(grad_sync, after)
-            except Exception as e:          # e.g. a collective backend that cannot be captured: stay eager, say so once
-                import warnings
-                warnings.warn(f"cstp_b200: CUDA-graph capture of the step failed ({e!r}); running eagerly")
-                self.use_graph = False
-                torch.cuda.synchronize(self.device)
-                self._step_body(grad_sync, after)
-            else:
-                self._graph, self._graph_key = g, key
-                self._graph_launches = ops.launch_count() - before
-                ops.note_replayed(-self._graph_launches)       # the capture pass counted launches that did not run
-                g.replay()
-                ops.note_replayed(self._graph_launches)
+        self._captured("step", (id(grad_sync), optimizer), lambda: self._step_body(grad_sync, after))
         self.first_step = False
 
     def drop_graph(self) -> None:
-        self._graph, self._graph_key = None, None
+        self._graphs.pop("step", None)
 
     def profile_tensor_launches(self, x1, x2):
         """Runs one forward + backward with CUDA events around every backbone tensor-core launch group.

@@ -2,7 +2,7 @@
 average pool and, with `proj`, the projector -- over ONE BatchNorm statistics group, for the standalone
 models.pace.r21d_byol.R2Plus1DNet module.
 
-It reuses the builders of the pretraining engine (StepEngine._backbone, StepEngine._mlp) and is built in three variants:
+It reuses the builders every engine shares (ProgramEngine._backbone, ProgramEngine._mlp) and is built in three variants:
 
     grads=True                     train mode with a backward program: d feat (+ d proj) -> parameter gradients, and on
                                    request the gradient of the input clip (ops.stem_dgrad)
@@ -21,39 +21,24 @@ from __future__ import annotations
 import torch
 
 from . import engine as E
-from .engine import FlatStore, StepEngine, backbone_param_specs, bn_buffer_specs
+from .engine import ProgramEngine, backbone_param_specs
 
 PREFIX = "online_net"
 
 
-class BackboneEngine(StepEngine):
-    VIEWS = 1
-
+class BackboneEngine(ProgramEngine):
     def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", *, proj: bool = False,
                  grads: bool = True, eval_mode: bool = False, share: "BackboneEngine | None" = None,
                  record: bool = False, overlap: bool = True, fuse_apply: bool | None = None,
                  fuse_min_positions: int | None = None, fuse_policy: str | None = None):
         if grads and eval_mode:
             raise ValueError("an eval-mode backbone engine is forward only")
-        self.proj, self.grads, self._share = bool(proj), bool(grads), share
-        super().__init__(B, T, H, W, device=device, record=record, overlap=bool(overlap) and self.grads,
-                         fuse_apply=fuse_apply, fuse_min_positions=fuse_min_positions, fuse_policy=fuse_policy,
-                         graph=False)
+        self.proj, self.grads = bool(proj), bool(grads)
+        super().__init__(B, T, H, W, device, backbone_param_specs(PREFIX, project=self.proj), grads=self.grads,
+                         share=share, record=record, overlap=bool(overlap) and self.grads, fuse_apply=fuse_apply,
+                         fuse_min_positions=fuse_min_positions, fuse_policy=fuse_policy, graph=False)
         self.eval_mode = bool(eval_mode)
-
-    def _make_stores(self):
-        specs = backbone_param_specs(PREFIX, project=self.proj)
-        if self._share is None:
-            self.train = FlatStore(specs, self.device)
-            self.bufs = FlatStore(bn_buffer_specs(specs), self.device)
-            for name in self.bufs.slots:
-                if name.endswith("running_var"):
-                    self.bufs.view(name).fill_(1.0)
-        else:
-            self.train, self.bufs = self._share.train, self._share.bufs
-        self.target = None
-        self.grad = self.train.like() if self.grads else None
-        self.mom = None
+        self._build()
 
     # ------------------------------------------------------------------------------------------ build
     def _build(self):
@@ -89,8 +74,7 @@ class BackboneEngine(StepEngine):
         """fp32 NCDHW clips (n, 3, T, H, W), n <= B -> rows [0, n) of self.feat (and self.proj_out)."""
         n = x.shape[0]
         E.ops.stem_pack(x, self.stem_rows[:n])
-        for op in self.fwd_online:
-            op()
+        self._forward_program()
 
     def backward_from(self, dfeat, dproj=None, dx: torch.Tensor | None = None) -> None:
         """Backward program of the last forward: dfeat fp32 [B][512] (and dproj) -> self.grad (every parameter,

@@ -3,9 +3,9 @@ driven by main_ft_mp.py:179-289 (train / validation) and test.py:76-93 (multi-cl
 
     logits = classify(cls_bn(F.normalize(online_net(x), p=2, dim=1)))            R21DBYOL(pretrain=False, num_classes, cls_bn)
 
-Reuses the backbone program builder and every kernel of the pretraining engine (cstp_b200.engine.StepEngine) with ONE
-view per sample (one BatchNorm statistics group) and no target network; adds the L2-normalise / BatchNorm1d / Linear
-head, the n-way cross-entropy, and an eval mode in which every BatchNorm is the affine map of its running statistics
+Builds on cstp_b200.engine.ProgramEngine (the backbone program builder and every kernel of the pretraining engine)
+with ONE view per sample (one BatchNorm statistics group) and no target network; adds the L2-normalise / BatchNorm1d /
+Linear head, the n-way cross-entropy, and an eval mode in which every BatchNorm is the affine map of its running statistics
 (model.eval()): forward only, no statistics kernels, nothing updated.
 """
 from __future__ import annotations
@@ -13,7 +13,7 @@ from __future__ import annotations
 import torch
 
 from . import engine as E
-from .engine import FlatStore, StepEngine, backbone_param_specs, bn_buffer_specs, pad16
+from .engine import OptimizerEngine, ProgramEngine, backbone_param_specs, pad16
 
 
 def finetune_param_specs(num_classes: int, cls_bn: bool):
@@ -25,109 +25,91 @@ def finetune_param_specs(num_classes: int, cls_bn: bool):
     return s
 
 
-class FinetuneEngine(StepEngine):
-    VIEWS = 1
-    FORWARD_ONLY = False             # InferenceEngine: no backward program, no gradient / momentum store
+def _build_classifier(eng, grads: bool, backbone_grads: bool) -> None:
+    """The program of `eng`: online_net -> avgpool -> F.normalize -> cls_bn -> classify, and with `grads` the head's
+    backward into eng.grad (classify; with `backbone_grads` also cls_bn, the normalisation, the pool and the backbone)."""
+    ops = E.ops
+    B = eng.B
+    f32 = dict(device=eng.device, dtype=torch.float32)
+    x5, bw_backbone = eng._backbone(eng.fwd_online, eng.train, "online_net", backbone_grads, "online")
+    C = eng.num_classes
+    Cp = pad16(C)
+    eng.feat = torch.zeros(B, 512, **f32)
+    eng.norms = torch.zeros(B, **f32)
+    eng.nfeat = eng._act(B, 512)                     # F.normalize(feat) as bf16 rows
+    eng.hfeat = eng._act(B, 512) if eng.cls_bn else eng.nfeat
+    eng.logits = torch.zeros(B, Cp, **f32)
+    eng.dlogits = torch.zeros(B, Cp, **f32) if grads else None
+    eng.loss = torch.zeros(1, **f32)
+    eng.ce_ws = torch.zeros(max(B, 16), **f32)
+    wc, wct = eng._packed(eng.train, "classify.weight", grads)
+    bias = eng.train.slot("classify.bias")
+    p_cls = ops.linear_plan(eng.hfeat, wc, None, out_f32=eng.logits, bias=bias)
+    site = eng._site(eng.train, grads, "cls_bn", 512, 1, B) if eng.cls_bn else None
+    eng._rec("head.feat", eng.feat)
+    eng._rec("head.nfeat", eng.nfeat)
+    eng._rec("head.hfeat", eng.hfeat)
+    eng._rec("head.logits", eng.logits)
 
+    def head_fwd():
+        ops.avgpool_fwd(x5, eng.feat, None)
+        ops.l2norm_fwd(eng.feat, eng.nfeat, eng.norms, 512)
+        if site is not None:
+            eng._bn_forward(eng.nfeat, site)
+            ops.bn_apply(eng.nfeat, site.st, eng.hfeat, relu=False)
+        p_cls.run()
+    eng.fwd_online.append(head_fwd)
+    if not grads:
+        eng._finish_build()
+        return
+
+    # ---------------- backward program: head -> pool -> backbone
+    g_out = eng._act(B, Cp)
+    d_h = eng._act(B, 512)
+    g_n = eng._act(B, 512) if eng.cls_bn else d_h
+    eng.dfeat = torch.zeros(B, 512, **f32)
+    dWc = eng.train.view("classify.weight", eng.grad)
+    dbc = eng.train.view("classify.bias", eng.grad)
+    g1 = ops.ConvGeom((1, 1, 1))
+    h5, go5 = eng.hfeat.view(1, 1, 1, B, 512), g_out.view(1, 1, 1, B, Cp)
+    eng._wg_numel = max(eng._wg_numel, eng._wgrad_need(h5, go5, g1))
+    pd_h = ops.linear_plan(g_out, wct, d_h)
+    holder = {}
+    eng._deferred.append(lambda: holder.__setitem__("wg", ops.wgrad_plan(h5, go5, g1, C, 512, eng._wg)))
+    eng._rec("head.g_out", g_out)
+    eng._rec("head.d_h", d_h)
+    eng._rec("head.g_n", g_n)
+    eng._rec("head.dfeat", eng.dfeat)
+    d_x5 = eng._dbuf(x5)
+
+    def head_bwd():
+        ops.cast_pad(eng.dlogits, g_out, cols=C)
+        ops.colsum(g_out, C, dbc)
+        holder["wg"].run(dWc)
+        if not backbone_grads:
+            return
+        pd_h.run()
+        if site is not None:
+            ops.bn_backward(d_h, None, eng.nfeat, site.st, site.gamma, site.dgamma, site.dbeta, g_n,
+                            sync=eng.bn_sync)
+        ops.l2norm_bwd(eng.feat, eng.norms, g_n, eng.dfeat, 512)
+        ops.avgpool_bwd(eng.dfeat, d_x5)
+    eng.bwd.append(head_bwd)
+    if backbone_grads:
+        eng.bwd.extend(reversed(bw_backbone))
+    eng._finish_build()
+
+
+class FinetuneEngine(OptimizerEngine):
     def __init__(self, B: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", num_classes: int = 101,
                  cls_bn: bool = True, record: bool = False, overlap: bool = True, backbone_grads: bool = True,
                  bn_sync=None, fuse_apply: bool | None = None, fuse_min_positions: int | None = None,
                  fuse_policy: str | None = None):
         self.num_classes, self.cls_bn, self.backbone_grads = num_classes, bool(cls_bn), backbone_grads
-        super().__init__(B, T, H, W, device=device, record=record, overlap=overlap, bn_sync=bn_sync, fuse_apply=fuse_apply,
-                         fuse_min_positions=fuse_min_positions, fuse_policy=fuse_policy)
-
-    def _make_stores(self):
-        self._make_param_stores()
-        self.grad = self.train.like()
-        self.mom = self.train.like()
-
-    def _make_param_stores(self):
-        specs = finetune_param_specs(self.num_classes, self.cls_bn)
-        self.train = FlatStore(specs, self.device)
-        self.target = None
-        self.bufs = FlatStore(bn_buffer_specs(specs), self.device)
-        for name in self.bufs.slots:
-            if name.endswith("running_var"):
-                self.bufs.view(name).fill_(1.0)
-
-    # ------------------------------------------------------------------------------------------ build
-    def _build(self):
-        ops = E.ops
-        B = self.B
-        f32 = dict(device=self.device, dtype=torch.float32)
-        x5, bw_backbone = self._backbone(self.fwd_online, self.train, "online_net", self.backbone_grads, "online")
-        C = self.num_classes
-        Cp = pad16(C)
-        self.feat = torch.zeros(B, 512, **f32)
-        self.norms = torch.zeros(B, **f32)
-        self.nfeat = self._act(B, 512)                     # F.normalize(feat) as bf16 rows
-        self.hfeat = self._act(B, 512) if self.cls_bn else self.nfeat
-        head_grads = not self.FORWARD_ONLY
-        self.logits = torch.zeros(B, Cp, **f32)
-        self.dlogits = torch.zeros(B, Cp, **f32) if head_grads else None
-        self.loss = torch.zeros(1, **f32)
-        self.ce_ws = torch.zeros(max(B, 16), **f32)
-        wc, wct = self._packed(self.train, "classify.weight", head_grads)
-        bias = self.train.slot("classify.bias")
-        p_cls = ops.linear_plan(self.hfeat, wc, None, out_f32=self.logits, bias=bias)
-        site = self._site(self.train, head_grads, "cls_bn", 512, 1, B) if self.cls_bn else None
-        self._rec("head.feat", self.feat)
-        self._rec("head.nfeat", self.nfeat)
-        self._rec("head.hfeat", self.hfeat)
-        self._rec("head.logits", self.logits)
-
-        def head_fwd():
-            ops.avgpool_fwd(x5, self.feat, None)
-            ops.l2norm_fwd(self.feat, self.nfeat, self.norms, 512)
-            if site is not None:
-                if self.eval_mode:
-                    ops.bn_eval_coeffs(site.st, site.gamma, site.beta, site.rm, site.rv, E.BN_EPS)
-                else:
-                    ops.bn_forward_stats(self.nfeat, site.st, site.gamma, site.beta, site.rm, site.rv, E.BN_EPS,
-                                         E.BN_MOMENTUM, sync=self.bn_sync)
-                ops.bn_apply(self.nfeat, site.st, self.hfeat, relu=False)
-            p_cls.run()
-        self.fwd_online.append(head_fwd)
-        if not head_grads:
-            self._finish_build()
-            return
-
-        # ---------------- backward program: head -> pool -> backbone
-        g_out = self._act(B, Cp)
-        d_h = self._act(B, 512)
-        g_n = self._act(B, 512) if self.cls_bn else d_h
-        self.dfeat = torch.zeros(B, 512, **f32)
-        dWc = self.train.view("classify.weight", self.grad)
-        dbc = self.train.view("classify.bias", self.grad)
-        g1 = ops.ConvGeom((1, 1, 1))
-        h5, go5 = self.hfeat.view(1, 1, 1, B, 512), g_out.view(1, 1, 1, B, Cp)
-        self._wg_numel = max(self._wg_numel, self._wgrad_need(h5, go5, g1))
-        pd_h = ops.linear_plan(g_out, wct, d_h)
-        holder = {}
-        self._deferred.append(lambda: holder.__setitem__("wg", ops.wgrad_plan(h5, go5, g1, C, 512, self._wg)))
-        self._rec("head.g_out", g_out)
-        self._rec("head.d_h", d_h)
-        self._rec("head.g_n", g_n)
-        self._rec("head.dfeat", self.dfeat)
-        d_x5 = self._dbuf(x5)
-
-        def head_bwd():
-            ops.cast_pad(self.dlogits, g_out, cols=C)
-            ops.colsum(g_out, C, dbc)
-            holder["wg"].run(dWc)
-            if not self.backbone_grads:
-                return
-            pd_h.run()
-            if site is not None:
-                ops.bn_backward(d_h, None, self.nfeat, site.st, site.gamma, site.dgamma, site.dbeta, g_n,
-                                sync=self.bn_sync)
-            ops.l2norm_bwd(self.feat, self.norms, g_n, self.dfeat, 512)
-            ops.avgpool_bwd(self.dfeat, d_x5)
-        self.bwd.append(head_bwd)
-        if self.backbone_grads:
-            self.bwd.extend(reversed(bw_backbone))
-        self._finish_build()
+        super().__init__(B, T, H, W, device, finetune_param_specs(num_classes, self.cls_bn), record=record,
+                         overlap=overlap, bn_sync=bn_sync, fuse_apply=fuse_apply, fuse_min_positions=fuse_min_positions,
+                         fuse_policy=fuse_policy)
+        _build_classifier(self, True, backbone_grads)
 
     # ------------------------------------------------------------------------------------------ programs
     def load_clip(self, x: torch.Tensor):
@@ -138,28 +120,19 @@ class FinetuneEngine(StepEngine):
         if repack:
             self.pack_online()
         self.load_clip(x)
-        for op in self.fwd_online:
-            op()
+        self._forward_program()
         return self.logits
 
     def forward_eval(self, x, use_graph: bool = True):
         """model.eval() forward.  The ~75 small launches of a batch-1 clip are launch-bound (1.2 ms eager), so the
-        program is captured once into a CUDA graph over a static input buffer and replayed (weights are re-packed outside
-        the graph into the same buffers, so the graph survives weight updates)."""
+        program behind the input pass is replayed from a CUDA graph (weights are re-packed outside the graph into the
+        same buffers, so the graph survives weight updates)."""
         self.eval_mode = True
-        if not use_graph or self.device.type != "cuda":
-            return self.forward(x)
-        if getattr(self, "_graph", None) is None:
-            self._x_static = torch.empty_like(x)
-            self._x_static.copy_(x)
-            self.forward(self._x_static)                   # eager warm-up: one-time kernel attribute calls happen here
-            torch.cuda.synchronize(self.device)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self.forward(self._x_static)
-            self._graph = g
-        self._x_static.copy_(x)
-        self._graph.replay()
+        self.load_clip(x)
+        if use_graph:
+            self._captured("eval", None, self._forward_program)
+        else:
+            self._forward_program()
         return self.logits
 
     def cross_entropy(self, labels):
@@ -171,13 +144,10 @@ class FinetuneEngine(StepEngine):
         slots are adjacent.  optim.SGD skips parameters without a gradient entirely -- no weight decay, no momentum
         (r21d_byol.py:10-35 sets requires_grad = False on everything but `classify` for ft_fc)."""
         runs: list[list[int]] = []
-        for name, (off, shape) in self.train.slots.items():
+        for name, (off, _) in self.train.slots.items():
             if name in frozen_names:
                 continue
-            n = 1
-            for d in shape:
-                n *= d
-            n = (n + 15) // 16 * 16
+            n = self.train.slot(name).numel()
             if runs and runs[-1][0] + runs[-1][1] == off:
                 runs[-1][1] += n
             else:
@@ -215,7 +185,7 @@ def inference_capacity(n: int) -> int:
     return 1 << (n - 1).bit_length() if n <= 64 else (n + 63) // 64 * 64
 
 
-class InferenceEngine(FinetuneEngine):
+class InferenceEngine(ProgramEngine):
     """Forward-only eval engine (model.eval(): every BatchNorm is the affine map of its running statistics) of a fixed
     batch `capacity` that evaluates any n <= capacity clips: `run(n)` computes rows [0, n) of `x_static` and leaves the
     other rows unread.  Eval BatchNorm couples no samples and the forward convolutions have no split-K, so a clip's
@@ -224,45 +194,27 @@ class InferenceEngine(FinetuneEngine):
     share: an engine whose parameter and BatchNorm running-statistics stores this one reads (the module's bound training
     engine); None allocates them here.  Either way the packed bf16 weights are this engine's own (pack_online)."""
 
-    FORWARD_ONLY = True
-
     def __init__(self, capacity: int, T: int = 16, H: int = 112, W: int = 112, device="cuda", num_classes: int = 101,
-                 cls_bn: bool = True, share: FinetuneEngine | None = None, **options):
-        self._share = share
+                 cls_bn: bool = True, share: ProgramEngine | None = None, **options):
+        self.num_classes, self.cls_bn = num_classes, bool(cls_bn)
         options["overlap"] = False              # one stream: there is no target network and no backward pass
-        super().__init__(capacity, T, H, W, device=device, num_classes=num_classes, cls_bn=cls_bn, backbone_grads=False,
-                         **options)
+        super().__init__(capacity, T, H, W, device, finetune_param_specs(num_classes, self.cls_bn), grads=False,
+                         share=share, **options)
         self.capacity = capacity
         self.eval_mode = True
         self.x_static = torch.zeros(capacity, 3, T, H, W, device=self.device, dtype=torch.float32)
+        self._build()
 
-    def _make_stores(self):
-        if self._share is None:
-            self._make_param_stores()
-        else:
-            self.train, self.bufs, self.target = self._share.train, self._share.bufs, None
-        self.grad = self.mom = None
+    def _build(self):
+        _build_classifier(self, False, False)
 
     def run(self, n: int) -> torch.Tensor:
         """Eval forward of rows [0, n) of x_static; returns self.logits, whose rows [0, n) are valid.  The program behind
-        the input pass is replayed from a CUDA graph captured on the first call."""
+        the input pass is replayed from a CUDA graph (ProgramEngine._captured)."""
         if not 1 <= n <= self.capacity:
             raise ValueError(f"{n} clips do not fit an inference engine of capacity {self.capacity}")
         E.ops.stem_pack(self.x_static[:n], self.stem_rows[:n])
-        if not self.use_graph:
-            for op in self.fwd_online:
-                op()
-            return self.logits
-        if self._graph is None:
-            for op in self.fwd_online:           # eager warm-up: one-time kernel attribute calls happen here
-                op()
-            torch.cuda.synchronize(self.device)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                for op in self.fwd_online:
-                    op()
-            self._graph = g
-        self._graph.replay()
+        self._captured("eval", None, self._forward_program)
         return self.logits
 
     def forward_batch(self, x: torch.Tensor) -> torch.Tensor:

@@ -54,6 +54,38 @@ class _Holder(nn.Module):
                            "(the computation runs in the cstp_b200 CUDA engine, there is no per-module path)")
 
 
+def _device(device) -> torch.device:
+    """torch.device(device), a bare "cuda" resolved to the current CUDA device (the key of an engine cache)."""
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    return device
+
+
+def _alias(module, train, bufs, prefix="", target=None):
+    """Points every parameter and BatchNorm running buffer of module's tree at its slot (`prefix` + its name) of the
+    engine stores `train` / `bufs` -- parameters under `target_net.` at `target` when given -- keeping their values, and
+    stacks every num_batches_tracked into one device tensor, which it returns (the modules hold its rows)."""
+    with torch.no_grad():
+        for name, p in module.named_parameters():
+            store = target if target is not None and name.startswith("target_net.") else train
+            v = store.view(prefix + name)
+            v.copy_(p.data)
+            p.data = v
+        nbt = []
+        for mname, mod in module.named_modules():
+            if isinstance(mod, (nn.BatchNorm1d, nn.BatchNorm3d)):
+                for b in ("running_mean", "running_var"):
+                    v = bufs.view(f"{prefix}{mname}.{b}")
+                    v.copy_(mod._buffers[b])
+                    mod._buffers[b] = v
+                nbt.append(mod)
+        flat = torch.stack([m._buffers["num_batches_tracked"].to(train.data.device) for m in nbt])
+        for i, m in enumerate(nbt):
+            m._buffers["num_batches_tracked"] = flat[i]
+    return flat
+
+
 def _triple(v):
     return tuple(v) if isinstance(v, (tuple, list)) else (v, v, v)
 
@@ -231,32 +263,13 @@ class R2Plus1DNet(nn.Module):
         `p.data = ...` / buffer assignment replaced one of them)."""
         if self._alias_ptr == self._pointers():
             return
-        pre = _engine_backbone().PREFIX
-        with torch.no_grad():
-            for name, p in self.named_parameters():
-                v = owner.train.view(f"{pre}.{name}")
-                v.copy_(p.data)
-                p.data = v
-            nbt = []
-            for mname, mod in self.named_modules():
-                if isinstance(mod, (nn.BatchNorm1d, nn.BatchNorm3d)):
-                    for b in ("running_mean", "running_var"):
-                        v = owner.bufs.view(f"{pre}.{mname}.{b}")
-                        v.copy_(mod._buffers[b])
-                        mod._buffers[b] = v
-                    nbt.append(mod)
-            flat = torch.stack([m._buffers["num_batches_tracked"].to(owner.device) for m in nbt])
-            for i, m in enumerate(nbt):
-                m._buffers["num_batches_tracked"] = flat[i]
-            self._nbt = flat
+        self._nbt = _alias(self, owner.train, owner.bufs, prefix=_engine_backbone().PREFIX + ".")
         self._alias_ptr = self._pointers()
         self._wgen += 1
 
     def _acquire(self, B, T, H, W, device, variant):
         """A free engine of this geometry and variant ("grad", "nograd", "eval"), with the current weights packed."""
-        device = torch.device(device)
-        if device.type == "cuda" and device.index is None:
-            device = torch.device("cuda", torch.cuda.current_device())
+        device = _device(device)
         if self._owner is not None and self._owner.device != device:
             self._reset_engines()
         key = (B, T, H, W, device, variant)
@@ -275,10 +288,7 @@ class R2Plus1DNet(nn.Module):
         self._alias(self._owner)
         # the parameters are views of the owner's flat store, but `p.data = view` leaves each parameter its own version
         # counter: an in-place update through a parameter bumps that counter, not the store's -- key on both
-        key = (self._owner.train.data._version, sum(p._version for p in self.parameters()), self._wgen)
-        if getattr(eng, "_packed_key", None) != key:
-            eng.pack_online()
-            eng._packed_key = key
+        eng.repack((self._owner.train.data._version, sum(p._version for p in self.parameters()), self._wgen))
         return pool, eng
 
     def forward(self, x):
@@ -449,25 +459,11 @@ class R21DBYOL(nn.Module):
             self._alias_ptr = None
         sentinel = self.online_net.conv1.spatial_conv.weight
         if self._alias_ptr != sentinel.data_ptr():
-            with torch.no_grad():
-                for name, p in self.named_parameters():
-                    store = eng.target if name.startswith("target_net.") else eng.train
-                    v = store.view(name)
-                    v.copy_(p.data)
-                    p.data = v
-                nbt, inc = [], []
-                for mname, mod in self.named_modules():
-                    if isinstance(mod, (nn.BatchNorm1d, nn.BatchNorm3d)):
-                        for b in ("running_mean", "running_var"):
-                            v = eng.bufs.view(f"{mname}.{b}")
-                            v.copy_(mod._buffers[b])
-                            mod._buffers[b] = v
-                        nbt.append(mod)
-                        inc.append(1 if mname in ("overlap_spa.1", "overlap_tem.1") else 2)
-                flat = torch.stack([m._buffers["num_batches_tracked"].to(x1.device) for m in nbt])
-                for i, m in enumerate(nbt):
-                    m._buffers["num_batches_tracked"] = flat[i]
-                self._nbt, self._nbt_inc = flat, torch.tensor(inc, device=x1.device, dtype=flat.dtype)
+            self._nbt = _alias(self, eng.train, eng.bufs, target=eng.target)
+            # the BatchNorms of the pair heads see one batch per step, every other one a batch per view
+            inc = [1 if n in ("overlap_spa.1", "overlap_tem.1") else 2 for n, m in self.named_modules()
+                   if isinstance(m, (nn.BatchNorm1d, nn.BatchNorm3d))]
+            self._nbt_inc = torch.tensor(inc, device=x1.device, dtype=self._nbt.dtype)
             eng.drop_graph()                     # a captured step holds the old num_batches_tracked tensors
             self._alias_ptr = sentinel.data_ptr()
             self._dirty = True
@@ -503,23 +499,8 @@ class R21DBYOL(nn.Module):
         """Points every parameter / BatchNorm buffer at eng's flat stores (again after .cuda() / .to() moved them)."""
         sentinel = self.online_net.conv1.spatial_conv.weight
         if getattr(self, "_alias_ptr", None) != sentinel.data_ptr():
-            with torch.no_grad():
-                for name, p in self.named_parameters():
-                    v = eng.train.view(name)
-                    v.copy_(p.data)
-                    p.data = v
-                nbt = []
-                for mname, mod in self.named_modules():
-                    if isinstance(mod, (nn.BatchNorm1d, nn.BatchNorm3d)):
-                        for b in ("running_mean", "running_var"):
-                            v = eng.bufs.view(f"{mname}.{b}")
-                            v.copy_(mod._buffers[b])
-                            mod._buffers[b] = v
-                        nbt.append(mod)
-                flat = torch.stack([m._buffers["num_batches_tracked"].to(eng.device) for m in nbt])
-                for i, m in enumerate(nbt):
-                    m._buffers["num_batches_tracked"] = flat[i]
-                self._nbt, self._nbt_inc = flat, torch.ones_like(flat)
+            self._nbt = _alias(self, eng.train, eng.bufs)
+            self._nbt_inc = torch.ones_like(self._nbt)
             self._alias_ptr = sentinel.data_ptr()
             self._dirty = True
 
@@ -534,9 +515,7 @@ class R21DBYOL(nn.Module):
             return self._feature_engine(capacity, T, H, W, device)
         if not isinstance(self.cls_bn, nn.Module):
             raise TypeError("'bool' object is not callable")
-        device = torch.device(device)
-        if device.type == "cuda" and device.index is None:
-            device = torch.device("cuda", torch.cuda.current_device())
+        device = _device(device)
         owner = self._engine
         if owner is None:
             owner = self._infer_owner
@@ -564,9 +543,7 @@ class R21DBYOL(nn.Module):
             raise _engine_mod.ops.L.CstpError(
                 "the features of a pretraining model are those of its live step engine: run train_step (or "
                 "train.load_checkpoint with example_clip) before extracting them")
-        device = torch.device(device)
-        if device.type == "cuda" and device.index is None:
-            device = torch.device("cuda", torch.cuda.current_device())
+        device = _device(device)
         if eng.device != device:
             raise _engine_mod.ops.L.CstpError(f"the bound engine lives on {eng.device}, not {device}")
         key = (capacity, T, H, W, device)
@@ -596,10 +573,7 @@ class R21DBYOL(nn.Module):
         if self._dirty:
             self._wgen += 1
             self._dirty = self.pretrain          # a pretraining model's step engine re-packs (and clears it) in train_step
-        key = (eng.train.data._version, self._wgen)
-        if getattr(eng, "_packed_key", None) != key:
-            eng.pack_online()
-            eng._packed_key = key
+        eng.repack((eng.train.data._version, self._wgen))
 
     def _forward_ft(self, x1):
         if not self.training:
@@ -662,7 +636,7 @@ class R21DBYOL(nn.Module):
         eng.optimizer_step(lr, momentum, weight_decay, ranges=self._ft_ranges, optimizer=optimizer, betas=betas, eps=eps)
         self._nbt += self._nbt_inc
         self._wgen += 1                          # the kernel updated the weights: other engines must re-pack
-        eng._packed_key = (eng.train.data._version, self._wgen)       # optimizer_step re-packed this one
+        eng.repack((eng.train.data._version, self._wgen), packed=True)       # optimizer_step re-packed this one
         self._last_engine = eng
         return eng.loss
 

@@ -167,14 +167,14 @@ def test_test_videos_packing_equals_per_video_loop(emu):
 
 # ------------------------------------------------------------------------------------------ engines of the drop-in
 def _count_builds(monkeypatch):
-    from cstp_b200 import engine_ft
+    from cstp_b200 import engine
     built = []
-    init = engine_ft.FinetuneEngine.__init__
+    init = engine.ProgramEngine.__init__
 
     def spy(self, B, *a, **k):
         built.append((type(self).__name__, B))
         init(self, B, *a, **k)
-    monkeypatch.setattr(engine_ft.FinetuneEngine, "__init__", spy)
+    monkeypatch.setattr(engine.ProgramEngine, "__init__", spy)
     return built
 
 

@@ -53,14 +53,15 @@ def model():
 
 
 def count_builds():
-    from cstp_b200 import engine_ft
+    from cstp_b200 import engine
+    base = getattr(engine, "ProgramEngine", None) or engine.StepEngine     # every engine's constructor (older trees: StepEngine)
     built = []
-    init = engine_ft.FinetuneEngine.__init__
+    init = base.__init__
 
     def spy(self, B, *a, **k):
         built.append(B)
         init(self, B, *a, **k)
-    engine_ft.FinetuneEngine.__init__ = spy
+    base.__init__ = spy
     return built
 
 
