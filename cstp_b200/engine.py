@@ -217,6 +217,7 @@ class ProgramEngine:
     store; `bn_specs`: parameters outside `train` whose BatchNorm running statistics live in `bufs` too."""
 
     VIEWS = 1          # clips per sample pushed through the backbone = BatchNorm statistics groups
+    EVAL_BACKWARD = False   # True: BatchNorm states in the layout of ops.bn_backward_eval (engine_ft.ExplainEngine)
 
     def __init__(self, B: int, T: int, H: int, W: int, device, specs, *, grads: bool, share=None, bn_specs=(),
                  record: bool = False, overlap: bool = True, bn_sync=None, fuse_apply: bool | None = None,
@@ -302,23 +303,28 @@ class ProgramEngine:
             self.named[name] = t
 
     def _site(self, store: FlatStore, grads: bool, name: str, C: int, groups: int, rows_per_group: int) -> _Site:
-        st = ops.BNState.alloc(C, pad16(C), groups, rows_per_group, self.device, backward=grads)
+        st = ops.BNState.alloc(C, pad16(C), groups, rows_per_group, self.device, backward=grads,
+                               eval_backward=self.EVAL_BACKWARD)
         return _Site(name, C, store.view(name + ".weight"), store.view(name + ".bias"),
                      self.bufs.view(name + ".running_mean"), self.bufs.view(name + ".running_var"), st,
                      store.view(name + ".weight", self.grad) if grads else None,
                      store.view(name + ".bias", self.grad) if grads else None)
 
-    def _packed(self, store: FlatStore, name: str, grads: bool, rows_pad: int | None = None, stem: bool = False):
+    def _packed(self, store: FlatStore, name: str, grads: bool, rows_pad: int | None = None, stem: bool = False,
+                forward: bool = True):
         """bf16 packed forward (and dgrad-transposed) copies of a conv / linear weight; registers the re-pack job.
         stem: the (Cout, 3, 1, 7, 7) weight in the layout of the packed stem row pairs -- four taps of 64 (hpar, kw, c)
-        channels (include/cstp_b200.h cstp_pack_weight transpose = 2); it has no dgrad copy."""
+        channels (include/cstp_b200.h cstp_pack_weight transpose = 2); it has no dgrad copy.  forward=False: only the
+        dgrad copy (a weight whose forward copy another call registered); (None, wt) is returned."""
         w = store.view(name)
         cout, cin = w.shape[0], w.shape[1]
         taps = w.numel() // (cout * cin)
         if stem:
             assert not grads
             cin, taps = ops.STEM_CHANNELS, 4
-        wp = torch.zeros(rows_pad or pad16(cout), taps * pad64(pad16(cin)), device=self.device, dtype=ACT_DTYPE)
+        wp = None
+        if forward:
+            wp = torch.zeros(rows_pad or pad16(cout), taps * pad64(pad16(cin)), device=self.device, dtype=ACT_DTYPE)
         wt = None
         if grads:
             wt = torch.zeros(pad16(cin), taps * pad64(pad16(cout)), device=self.device, dtype=ACT_DTYPE)
@@ -427,27 +433,35 @@ class ProgramEngine:
             out = raw
         return raw, out, site, unit
 
-    def _unit_backward(self, unit, d_out, *, act_for_mask, dz=None, dx_accumulate=False):
-        """Backward closure of one conv+BN unit: BN backward -> wgrad -> dgrad (see _conv_bn)."""
+    def _unit_backward(self, unit, d_out, *, act_for_mask, dz=None, dx_accumulate=False, eval_dgrad=False):
+        """Backward closure of one conv+BN unit: BN backward -> wgrad -> dgrad (see _conv_bn).  eval_dgrad: the eval-mode,
+        data-gradient-only flavour (engine_ft.ExplainEngine): the derivative of the running-statistics BatchNorm map
+        (ops.bn_backward_eval), then dgrad with a transposed weight packed here; no weight or BatchNorm-parameter
+        gradient."""
         x, raw, site, geom = unit["x"], unit["raw"], unit["site"], unit["geom"]
         dw = self.train.view(unit["wname"], self.grad)
+        wt = unit["wt"]
+        if eval_dgrad and not unit["skip_dgrad"]:
+            wt = self._packed(self.train, unit["wname"], True, forward=False)[1]
         holder = {}
 
         def prepare():
             g = self._gbufs[holder["gbuf"]][:raw.numel()].view(raw.shape)
             holder["g"] = g
-            holder["wg"] = _Timed(self, "wgrad", unit["flops"],
-                                  [ops.wgrad_plan(x, g, geom, unit["cout"], ops.STEM_CHANNELS if unit["stem"] else unit["cin"], self._wg,
-                                                  prologue=unit["pro"], layout=1 if unit["stem"] else 0)],
-                                  unit["tag"])
+            if not eval_dgrad:
+                holder["wg"] = _Timed(self, "wgrad", unit["flops"],
+                                      [ops.wgrad_plan(x, g, geom, unit["cout"], ops.STEM_CHANNELS if unit["stem"] else unit["cin"],
+                                                      self._wg, prologue=unit["pro"], layout=1 if unit["stem"] else 0)],
+                                      unit["tag"])
             if not unit["skip_dgrad"]:
                 dx = self._dbuf(x)
-                plans, covers = ops.conv_dgrad_plans(g, unit["wt"], dx, geom, accumulate=dx_accumulate)
+                plans, covers = ops.conv_dgrad_plans(g, wt, dx, geom, accumulate=dx_accumulate)
                 holder["dg"] = _Timed(self, "conv_dgrad", unit["flops"], plans, unit["tag"])
                 holder["zero"], holder["dx"] = (not covers and not dx_accumulate), dx
                 self._rec(unit["tag"] + ".dx", dx)
         self._deferred.append(prepare)
-        self._wg_numel = max(self._wg_numel, self._wgrad_need(x, raw, geom))
+        if not eval_dgrad:
+            self._wg_numel = max(self._wg_numel, self._wgrad_need(x, raw, geom))
 
         self._rec(unit["tag"] + ".d_out", d_out)
         # plain BN -> ReLU units recompute the mask from raw; block outputs (residual in the pre-activation) read act
@@ -455,14 +469,19 @@ class ProgramEngine:
 
         def bwd():
             g = holder["g"]
-            if self.overlap and self._prof is None and self._wg_recorded[holder["gbuf"]]:
-                # the weight-gradient GEMM that last read this d(raw) buffer (two units ago) must have finished
-                torch.cuda.current_stream().wait_event(self._ev_wg[holder["gbuf"]])
-            ops.bn_backward(d_out, act_for_mask, raw, site.st, site.gamma, site.dgamma, site.dbeta, g, dz=dz,
-                            mask_from_raw=from_raw, sync=self.bn_sync)
+            if eval_dgrad:
+                ops.bn_backward_eval(d_out, act_for_mask, raw, site.st, g, dz=dz, mask_from_raw=from_raw)
+            else:
+                if self.overlap and self._prof is None and self._wg_recorded[holder["gbuf"]]:
+                    # the weight-gradient GEMM that last read this d(raw) buffer (two units ago) must have finished
+                    torch.cuda.current_stream().wait_event(self._ev_wg[holder["gbuf"]])
+                ops.bn_backward(d_out, act_for_mask, raw, site.st, site.gamma, site.dgamma, site.dbeta, g, dz=dz,
+                                mask_from_raw=from_raw, sync=self.bn_sync)
             if self.record:      # parity tests: the shared d(raw) scratch is overwritten by a later unit
                 self.named[unit["tag"] + ".g"] = g.clone()
-            if self.overlap and self._prof is None:
+            if eval_dgrad:       # no weight gradient
+                pass
+            elif self.overlap and self._prof is None:
                 b = holder["gbuf"]
                 main = torch.cuda.current_stream()
                 self._ev_g[b].record(main)
@@ -478,7 +497,7 @@ class ProgramEngine:
                     holder["dx"].zero_()
                 holder["dg"].run()
         bwd.holder = holder
-        bwd.writes = [unit["wname"], unit["bnname"] + ".weight", unit["bnname"] + ".bias"]
+        bwd.writes = [] if eval_dgrad else [unit["wname"], unit["bnname"] + ".weight", unit["bnname"] + ".bias"]
         return bwd
 
     @staticmethod
@@ -487,31 +506,44 @@ class ProgramEngine:
         return ops.wgrad_partials_need(tuple(x.shape), tuple(raw.shape), geom)
 
     # ------------------------------------------------------------------------------------------ backbone
-    def _backbone(self, prog, store, prefix, grads, tag):
+    DGRAD_LEVELS = ("input", "conv1") + tuple(s[0] for s in STAGES)
+
+    def _backbone(self, prog, store, prefix, grads, tag, dgrad_to: str | None = None):
         """R2Plus1DNet.forward (r21d_byol.py:215-229) over both views.  Returns (last block act, backward closures in
-        forward order)."""
+        forward order).  dgrad_to (without grads): the closures are the eval-mode, data-gradient-only flavour
+        (_unit_backward eval_dgrad) of the parts above that level of DGRAD_LEVELS -- "conv5": none, "conv3": the conv4 and
+        conv5 blocks, "input": every unit down to the stem's d(raw)."""
         N, T = self.N, self.T
         Ho, Wo = self.H // 2, self.W // 2
         bw: list = []
+
+        def builder(level):
+            if grads:
+                return self._unit_backward
+            if dgrad_to is not None and self.DGRAD_LEVELS.index(level) > self.DGRAD_LEVELS.index(dgrad_to):
+                return lambda *a, **k: self._unit_backward(*a, eval_dgrad=True, **k)
+            return None
+        ub = builder("conv1")
         # stem spatial 1x7x7 s(1,2,2) p(0,3,3) (r21d_byol.py:198): a four-tap stride-1 implicit GEMM over packed row pairs,
         # whose 64 channels hold the (kw, c) taps of every output column for two frame rows -- no im2col matrix in HBM
         _, a0, site, u = self._conv_bn(prog, store, grads, self.stem_rows, f"{prefix}.conv1.spatial_conv.weight",
                                        f"{prefix}.conv1.bn", ops.STEM_GEOM, 3, 83, tag=f"{tag}.conv1.spatial",
                                        skip_dgrad=True, stem=True)
         assert tuple(a0.shape[:4]) == (N, T, Ho, Wo)
-        if grads:
-            bw.append(self._unit_backward(u, self._dbuf(a0), act_for_mask=a0))
+        if ub is not None:
+            bw.append(ub(u, self._dbuf(a0), act_for_mask=a0))
         raw, x, site, u = self._conv_bn(prog, store, grads, a0, f"{prefix}.conv1.temporal_conv.weight", f"{prefix}.bn1",
                                         ConvGeom((3, 1, 1), (1, 1, 1), (1, 0, 0)), 83, 64, tag=f"{tag}.conv1.temporal")
-        if grads:
-            bw.append(self._unit_backward(u, self._dbuf(x), act_for_mask=x))
+        if ub is not None:
+            bw.append(ub(u, self._dbuf(x), act_for_mask=x))
         for stage, cin, cout, down in STAGES:
             x = self._block(prog, store, f"{prefix}.{stage}.block1", grads, x, cin, cout, down, bw,
-                            f"{tag}.{stage}.block1")
+                            f"{tag}.{stage}.block1", unit_backward=builder(stage))
         return x, bw
 
-    def _block(self, prog, store, pre, grads, xin, cin, cout, down, bw, tag):
-        """SpatioTemporalResBlock.forward (r21d_byol.py:141-148)."""
+    def _block(self, prog, store, pre, grads, xin, cin, cout, down, bw, tag, unit_backward=None):
+        """SpatioTemporalResBlock.forward (r21d_byol.py:141-148).  unit_backward: the builder of the backward closures
+        appended to bw (None: _unit_backward with grads, no closures without)."""
         s = 2 if down else 1
         mid1 = intermed_channels(cin, cout, (3, 3, 3))
         mid2 = intermed_channels(cout, cout, (3, 3, 3))
@@ -538,28 +570,29 @@ class ProgramEngine:
             _, out, _, u4 = self._conv_bn(prog, store, grads, c, f"{pre}.conv2.temporal_conv.weight", f"{pre}.bn2", tp(1),
                                           mid2, cout, relu=True, res=xin, tag=f"{tag}.conv2.temporal")
         self._rec(tag + ".out", out)
-        if grads:
+        ub = unit_backward or (self._unit_backward if grads else None)
+        if ub is not None:
             d_out = self._dbuf(out)
             if down:
                 dz = self._act(*out.shape)          # masked upstream gradient, shared by bn2 and downsamplebn
                 self._rec(tag + ".dz", dz)
                 # forward order: u1 u2 u3 u5 u6 u4  -> reversed at run time
-                bw.append(self._unit_backward(u1, self._dbuf(a), act_for_mask=a))                 # writes d(xin)
-                bw.append(self._unit_backward(u2, self._dbuf(b), act_for_mask=b))
-                bw.append(self._unit_backward(u3, self._dbuf(c), act_for_mask=c))
+                bw.append(ub(u1, self._dbuf(a), act_for_mask=a))                 # writes d(xin)
+                bw.append(ub(u2, self._dbuf(b), act_for_mask=b))
+                bw.append(ub(u3, self._dbuf(c), act_for_mask=c))
                 # run order is reversed, so u5/u6 must come BEFORE u1 in the list to run AFTER it: they accumulate
                 # into d(xin) that u1 has overwritten.  Insert them ahead of u1.
                 k = len(bw) - 3
-                bw.insert(k, self._unit_backward(u5, self._dbuf(d1), act_for_mask=d1, dx_accumulate=True))
-                bw.insert(k + 1, self._unit_backward(u6, dz, act_for_mask=None))
-                bw.append(self._unit_backward(u4, d_out, act_for_mask=out, dz=dz))
+                bw.insert(k, ub(u5, self._dbuf(d1), act_for_mask=d1, dx_accumulate=True))
+                bw.insert(k + 1, ub(u6, dz, act_for_mask=None))
+                bw.append(ub(u4, d_out, act_for_mask=out, dz=dz))
             else:
                 # bn2 backward writes the masked upstream gradient straight into d(xin) (identity shortcut); the conv1
                 # spatial dgrad then accumulates into it.
-                bw.append(self._unit_backward(u1, self._dbuf(a), act_for_mask=a, dx_accumulate=True))
-                bw.append(self._unit_backward(u2, self._dbuf(b), act_for_mask=b))
-                bw.append(self._unit_backward(u3, self._dbuf(c), act_for_mask=c))
-                bw.append(self._unit_backward(u4, d_out, act_for_mask=out, dz=self._dbuf(xin)))
+                bw.append(ub(u1, self._dbuf(a), act_for_mask=a, dx_accumulate=True))
+                bw.append(ub(u2, self._dbuf(b), act_for_mask=b))
+                bw.append(ub(u3, self._dbuf(c), act_for_mask=c))
+                bw.append(ub(u4, d_out, act_for_mask=out, dz=self._dbuf(xin)))
         return out
 
     # ------------------------------------------------------------------------------------------ MLP heads
@@ -700,7 +733,8 @@ class ProgramEngine:
     def _pack_list(self, jobs):
         flat = []
         for w, wp, wt, mode in jobs:
-            flat.append((w, wp, mode))
+            if wp is not None:
+                flat.append((w, wp, mode))
             if wt is not None:
                 flat.append((w, wt, 1))
         return ops.PackList(flat, self.device)

@@ -25,13 +25,16 @@ def finetune_param_specs(num_classes: int, cls_bn: bool):
     return s
 
 
-def _build_classifier(eng, grads: bool, backbone_grads: bool) -> None:
+def _build_classifier(eng, grads: bool, backbone_grads: bool, dgrad_to: str | None = None) -> None:
     """The program of `eng`: online_net -> avgpool -> F.normalize -> cls_bn -> classify, and with `grads` the head's
-    backward into eng.grad (classify; with `backbone_grads` also cls_bn, the normalisation, the pool and the backbone)."""
+    backward into eng.grad (classify; with `backbone_grads` also cls_bn, the normalisation, the pool and the backbone).
+    dgrad_to (without grads): an eval-mode, data-gradient-only backward program from eng.dlogits down to that level of
+    ProgramEngine.DGRAD_LEVELS, with no parameter gradient (ExplainEngine)."""
     ops = E.ops
     B = eng.B
     f32 = dict(device=eng.device, dtype=torch.float32)
-    x5, bw_backbone = eng._backbone(eng.fwd_online, eng.train, "online_net", backbone_grads, "online")
+    explain = dgrad_to is not None
+    x5, bw_backbone = eng._backbone(eng.fwd_online, eng.train, "online_net", backbone_grads, "online", dgrad_to=dgrad_to)
     C = eng.num_classes
     Cp = pad16(C)
     eng.feat = torch.zeros(B, 512, **f32)
@@ -39,10 +42,10 @@ def _build_classifier(eng, grads: bool, backbone_grads: bool) -> None:
     eng.nfeat = eng._act(B, 512)                     # F.normalize(feat) as bf16 rows
     eng.hfeat = eng._act(B, 512) if eng.cls_bn else eng.nfeat
     eng.logits = torch.zeros(B, Cp, **f32)
-    eng.dlogits = torch.zeros(B, Cp, **f32) if grads else None
+    eng.dlogits = torch.zeros(B, Cp, **f32) if grads or explain else None
     eng.loss = torch.zeros(1, **f32)
     eng.ce_ws = torch.zeros(max(B, 16), **f32)
-    wc, wct = eng._packed(eng.train, "classify.weight", grads)
+    wc, wct = eng._packed(eng.train, "classify.weight", grads or explain)
     bias = eng.train.slot("classify.bias")
     p_cls = ops.linear_plan(eng.hfeat, wc, None, out_f32=eng.logits, bias=bias)
     site = eng._site(eng.train, grads, "cls_bn", 512, 1, B) if eng.cls_bn else None
@@ -59,7 +62,7 @@ def _build_classifier(eng, grads: bool, backbone_grads: bool) -> None:
             ops.bn_apply(eng.nfeat, site.st, eng.hfeat, relu=False)
         p_cls.run()
     eng.fwd_online.append(head_fwd)
-    if not grads:
+    if not grads and not explain:
         eng._finish_build()
         return
 
@@ -68,6 +71,21 @@ def _build_classifier(eng, grads: bool, backbone_grads: bool) -> None:
     d_h = eng._act(B, 512)
     g_n = eng._act(B, 512) if eng.cls_bn else d_h
     eng.dfeat = torch.zeros(B, 512, **f32)
+    if explain:
+        pd_h = ops.linear_plan(g_out, wct, d_h)
+        d_x5 = eng._dbuf(x5)
+
+        def head_dgrad():
+            ops.cast_pad(eng.dlogits, g_out, cols=C)
+            pd_h.run()
+            if site is not None:
+                ops.bn_backward_eval(d_h, None, eng.nfeat, site.st, g_n)
+            ops.l2norm_bwd(eng.feat, eng.norms, g_n, eng.dfeat, 512)
+            ops.avgpool_bwd(eng.dfeat, d_x5)
+        eng.bwd.append(head_dgrad)
+        eng.bwd.extend(reversed(bw_backbone))
+        eng._finish_build()
+        return
     dWc = eng.train.view("classify.weight", eng.grad)
     dbc = eng.train.view("classify.bias", eng.grad)
     g1 = ops.ConvGeom((1, 1, 1))
@@ -242,3 +260,73 @@ class FeatureEngine(InferenceEngine):
         self._rec("head.feat", self.feat)
         self.fwd_online.append(lambda: E.ops.avgpool_fwd(x5, self.feat, None))
         self._finish_build()
+
+
+EXPLAIN_STAGES = ("conv2", "conv3", "conv4", "conv5")
+
+
+class ExplainEngine(ProgramEngine):
+    """Grad-CAM engine (cstp_b200.explain) of a fixed batch `capacity`: the InferenceEngine's eval forward, then the
+    gradient of the score logits[b, k_b] (k_b given or the argmax) through an eval-mode, data-gradient-only backward
+    program -- the one-hot seed, the classifier dgrad, the cls_bn running-statistics map, l2norm_bwd, avgpool_bwd and the
+    backbone's dgrad closures down to the output of `stage` (or, with `input_grad`, to the stem's d(raw) and the clip) --
+    then the class-activation map of that stage, upsampled to the clip and min-max normalised.  Eval BatchNorm couples no
+    clips, so one backward pass serves every row.  There are no weight gradients, no BatchNorm statistics and no
+    running-statistics writes; transposed weights are packed only for the units the backward pass runs.
+
+    share: the engine whose parameter and running-statistics stores this one reads (as InferenceEngine)."""
+
+    EVAL_BACKWARD = True
+
+    def __init__(self, capacity: int, T: int = 16, H: int = 112, W: int = 112, stage: str = "conv5",
+                 input_grad: bool = False, device="cuda", num_classes: int = 101, cls_bn: bool = True,
+                 share: ProgramEngine | None = None, **options):
+        if stage not in EXPLAIN_STAGES:
+            raise ValueError(f"stage {stage!r}: expected one of {EXPLAIN_STAGES}")
+        self.num_classes, self.cls_bn = num_classes, bool(cls_bn)
+        self.stage, self.input_grad = stage, bool(input_grad)
+        options["overlap"] = False
+        super().__init__(capacity, T, H, W, device, finetune_param_specs(num_classes, self.cls_bn), grads=False,
+                         share=share, **options)
+        self.capacity = capacity
+        self.eval_mode = True
+        f32 = dict(device=self.device, dtype=torch.float32)
+        self.x_static = torch.zeros(capacity, 3, T, H, W, **f32)
+        self.classes_in = torch.zeros(capacity, device=self.device, dtype=torch.int64)
+        self.classes = torch.zeros(capacity, device=self.device, dtype=torch.int64)
+        _build_classifier(self, False, False, dgrad_to="input" if self.input_grad else stage)
+        unit = next(u for u in self.units if u["tag"] == f"online.{stage}.block1.conv2.temporal")
+        self.stage_act = unit["act"]                       # the block output after its ReLU
+        self.stage_grad = self._dbuf(self.stage_act)       # its gradient, left by the backward program
+        self.stage_channels = unit["cout"]
+        N, t, h, w, _ = self.stage_act.shape
+        self.alpha = torch.zeros(capacity, self.stage_channels, **f32)
+        self.cam_small = torch.zeros(capacity, t, h, w, **f32)
+        self.cam = torch.zeros(capacity, T, H, W, **f32)
+        self.dx = torch.zeros(capacity, 3, T, H, W, **f32) if self.input_grad else None
+
+    def _program(self, n: int, given: bool):
+        ops = E.ops
+        self._forward_program()
+        ops.cam_seed(self.logits, n, self.num_classes, self.classes_in if given else None, self.classes, self.dlogits)
+        for op in self.bwd:
+            op()
+        ops.gradcam(self.stage_act, self.stage_grad, n, self.stage_channels, self.alpha, self.cam_small)
+        ops.cam_upsample(self.cam_small, n, self.cam)
+        if self.input_grad:
+            g = self.bwd[-1].holder["g"]                   # the stem unit's d(raw)
+            ops.stem_dgrad(g[:n], self.train.view("online_net.conv1.spatial_conv.weight"), self.dx[:n])
+
+    def run(self, x: torch.Tensor, classes: torch.Tensor | None = None) -> None:
+        """Clips x (n, 3, T, H, W), n <= capacity, and optionally their classes (int64 [n], on the device) -> rows [0, n)
+        of logits, classes, cam (and dx).  The program behind the input pass is replayed from a CUDA graph
+        (ProgramEngine._captured), one per (n, classes given)."""
+        n = x.shape[0]
+        if not 1 <= n <= self.capacity:
+            raise ValueError(f"{n} clips do not fit an explain engine of capacity {self.capacity}")
+        self.x_static[:n].copy_(x)
+        if classes is not None:
+            self.classes_in[:n].copy_(classes)
+        E.ops.stem_pack(self.x_static[:n], self.stem_rows[:n])
+        given = classes is not None
+        self._captured("explain", (n, given), lambda: self._program(n, given))

@@ -245,6 +245,9 @@ SIGNATURES = {
     "cstp_l2_normalize_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "cstp_knn_partial": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "cstp_knn_merge": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "cstp_cam_seed": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "cstp_gradcam": (_i, [_vp, _vp, _i, C.c_longlong, _i, _i, _vp, _vp, _vp]),
+    "cstp_cam_upsample": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
     "cstp_jpeg_workspace_bytes": (C.c_longlong, [_i, _i]),
     "cstp_jpeg_decode": (_i, [_vp, _vp, _i, _vp, _vp, C.c_longlong, _vp]),
     "cstp_bn_sync_buffer_bytes": (C.c_longlong, [_i, _i, _i]),

@@ -513,6 +513,24 @@ class R21DBYOL(nn.Module):
         from ... import engine_ft
         if self.pretrain:
             return self._feature_engine(capacity, T, H, W, device)
+        return self._eval_engine((capacity, T, H, W), device, lambda owner, dev: engine_ft.InferenceEngine(
+            capacity, T, H, W, device=dev, num_classes=self.num_classes, cls_bn=True, share=owner,
+            **getattr(self, "engine_options", {})))
+
+    def explain_engine(self, capacity: int, T: int, H: int, W: int, device, stage: str, input_grad: bool):
+        """The cached Grad-CAM engine (engine_ft.ExplainEngine) of this batch capacity, clip size, stage and input-gradient
+        setting; it reads the parameters and running statistics as inference_engine's engines do, and
+        free_inference_engines releases it with them."""
+        from ... import engine_ft
+        return self._eval_engine(("explain", capacity, T, H, W, stage, bool(input_grad)), device,
+                                 lambda owner, dev: engine_ft.ExplainEngine(
+                                     capacity, T, H, W, stage=stage, input_grad=input_grad, device=dev,
+                                     num_classes=self.num_classes, cls_bn=True, share=owner,
+                                     **getattr(self, "engine_options", {})))
+
+    def _eval_engine(self, key, device, build):
+        """An eval engine of the finetune model, cached in _infer under key + (device,): build(owner, device) makes it
+        over the stores of the bound engine or, while none is bound, of the first such engine (see inference_engine)."""
         if not isinstance(self.cls_bn, nn.Module):
             raise TypeError("'bool' object is not callable")
         device = _device(device)
@@ -524,12 +542,10 @@ class R21DBYOL(nn.Module):
                 owner = None
         elif owner.device != device:
             raise _engine_mod.ops.L.CstpError(f"the bound engine lives on {owner.device}, not {device}")
-        key = (capacity, T, H, W, device)
+        key = key + (device,)
         eng = self._infer.get(key)
         if eng is None:
-            eng = engine_ft.InferenceEngine(capacity, T, H, W, device=device, num_classes=self.num_classes, cls_bn=True,
-                                            share=owner, **getattr(self, "engine_options", {}))
-            self._infer[key] = eng
+            eng = self._infer[key] = build(owner, device)
             if owner is None:
                 self._infer_owner = owner = eng
                 self._alias_ptr = None

@@ -948,9 +948,18 @@ class BNState:
     compact: torch.Tensor = field(default=None)      # [groups][2][Cp] row exchanged by world-synchronised BatchNorm
 
     @staticmethod
-    def alloc(C_: int, Cp: int, groups: int, rows_per_group: int, device, backward: bool = True) -> "BNState":
+    def alloc(C_: int, Cp: int, groups: int, rows_per_group: int, device, backward: bool = True,
+              eval_backward: bool = False) -> "BNState":
+        """eval_backward: the layout bn_backward_eval needs -- coef = [scale | 0 | 0] with `scale` a view of its first row
+        (which the eval forward's bn_eval_coeffs fills), zero mean and invstd; one statistics group."""
         nb = bn_nblocks(rows_per_group, Cp)
         f = dict(dtype=torch.float32, device=device)
+        if eval_backward:
+            if groups != 1:
+                raise L.CstpError("an eval-mode BatchNorm backward state holds one statistics group")
+            coef = torch.zeros(3 * Cp, **f)
+            return BNState(C_, Cp, 1, nb, torch.empty(max(nb, 160) * 2 * Cp, **f), coef[:Cp], torch.empty(Cp, **f),
+                           torch.zeros(Cp, **f), torch.zeros(Cp, **f), coef, torch.empty(2 * Cp, **f))
         # (room for the fused-statistics path too: one partial row per CTA of a persistent conv kernel, <= 148 + slack)
         return BNState(C_, Cp, groups, nb, torch.empty(max(nb, 160) * groups * 2 * Cp, **f), torch.empty(groups * Cp, **f),
                        torch.empty(groups * Cp, **f), torch.empty(groups * Cp, **f), torch.empty(groups * Cp, **f),
@@ -1019,6 +1028,21 @@ def bn_backward(d, act, raw, st: BNState, gamma, dgamma, dbeta, g_out, *, dz=Non
                                          int(accumulate), _ptr(st.coef), _stream()))
     L.check(lib.cstp_bn_bwd_apply(_ptr(d), _ptr(act), _ptr(raw), rows, st.Cp, st.groups, _ptr(st.mean), _ptr(st.invstd),
                                   _ptr(st.coef), _ptr(ms), _ptr(mb), _ptr(g_out), _ptr(dz), _stream()))
+
+
+def bn_backward_eval(d, act, raw, st: BNState, g_out, *, dz=None, mask_from_raw: bool = False) -> None:
+    """g_out = dL/d(raw) of an eval-mode BatchNorm, the affine map of the running statistics: bf16(scale * dy), dy = d
+    masked as in bn_backward (dz receives it).  One cstp_bn_bwd_apply launch with the coefficient row (scale, 0, 0) and
+    zero mean / invstd of a BNState.alloc(eval_backward=True) state: its g = fmaf(A, dy, fmaf(Bc, x, Cc)) then has
+    Bc = Cc = +0, so g = bf16(scale * dy) with a zero product stored as +0.  No statistics, no dgamma / dbeta."""
+    if st.coef is None or st.groups != 1 or st.scale.data_ptr() != st.coef.data_ptr():
+        raise L.CstpError("bn_backward_eval needs a BNState.alloc(eval_backward=True) state")
+    rows = raw.numel() // st.Cp
+    ms, mb = (st.scale, st.shift) if mask_from_raw else (None, None)
+    if mask_from_raw:
+        act = None
+    L.check(L.load().cstp_bn_bwd_apply(_ptr(d), _ptr(act), _ptr(raw), rows, st.Cp, 1, _ptr(st.mean), _ptr(st.invstd),
+                                       _ptr(st.coef), _ptr(ms), _ptr(mb), _ptr(g_out), _ptr(dz), _stream()))
 
 
 def avgpool_fwd(x, out_f32, out_bf16, rows_out: int | None = None, ld_out: int | None = None) -> None:
@@ -1142,6 +1166,60 @@ def video_finalize(sums, fin, topk_out, labels=None, mean_out=None, hits=None) -
     L.check(L.load().cstp_video_finalize(_ptr(sums), n_slots, n_cls, _ptr(fin), fin.shape[0], topk_out.shape[0],
                                          topk_out.shape[1], _ptr(labels), _ptr(mean_out), _ptr(topk_out), _ptr(hits),
                                          _stream()))
+
+
+CAM_MAX_CHANNELS = 512
+
+
+def cam_seed(logits, n: int, n_cls: int, classes_in, classes_out, dlogits) -> None:
+    """Seed of the Grad-CAM backward pass: for rows b < n the class classes_in[b] (int64, optional) or the argmax of the
+    n_cls valid columns of logits (fp32 [B][ld]; ties to the lower class) -> classes_out[b] (int64 [B]) and the one-hot
+    row dlogits[b] (fp32 [B][ld]); rows >= n get class 0 and zeros (include/cstp_b200.h cstp_cam_seed)."""
+    _require_cuda(logits, classes_in, classes_out, dlogits)
+    B, ld = logits.shape
+    if logits.dtype != torch.float32 or not logits.is_contiguous() or dlogits.dtype != torch.float32 \
+            or tuple(dlogits.shape) != (B, ld) or not dlogits.is_contiguous():
+        raise L.CstpError(f"cam_seed: logits and dlogits must be contiguous fp32 [B][ld], got {logits.dtype} "
+                          f"{tuple(logits.shape)} and {dlogits.dtype} {tuple(dlogits.shape)}")
+    for t, what in ((classes_out, "classes_out"), (classes_in, "classes_in")):
+        if t is not None and (t.dtype != torch.int64 or not t.is_contiguous() or t.numel() < B):
+            raise L.CstpError(f"cam_seed: {what} must be contiguous int64 with {B} entries, got {t.dtype} {tuple(t.shape)}")
+    if not 1 <= n <= B or not 1 <= n_cls <= ld:
+        raise L.CstpError(f"cam_seed: n = {n} and n_cls = {n_cls} must lie in [1, {B}] and [1, {ld}]")
+    L.check(L.load().cstp_cam_seed(_ptr(logits), B, ld, n, n_cls, _ptr(classes_in), _ptr(classes_out), _ptr(dlogits),
+                                   _stream()))
+
+
+def gradcam(act, grad, n: int, C_: int, alpha, cam) -> None:
+    """Grad-CAM of one stage over clips [0, n): act and grad bf16 NDHWC (N, t, h, w, Cp), the first C_ channels valid ->
+    alpha fp32 [>= n][C_] (the position means of grad) and cam fp32 (>= n, t, h, w) = relu(sum_c alpha_c * act_c), in the
+    fixed orders of include/cstp_b200.h cstp_gradcam."""
+    _require_cuda(act, grad, alpha, cam)
+    if act.dtype != torch.bfloat16 or grad.dtype != torch.bfloat16 or act.dim() != 5 or grad.shape != act.shape \
+            or not act.is_contiguous() or not grad.is_contiguous():
+        raise L.CstpError(f"gradcam: act and grad must be contiguous bf16 NDHWC tensors of one shape, got {act.dtype} "
+                          f"{tuple(act.shape)} and {grad.dtype} {tuple(grad.shape)}")
+    N, t, h, w, Cp = act.shape
+    if not 1 <= n <= N or C_ % 8 or not 0 < C_ <= min(Cp, CAM_MAX_CHANNELS) or Cp % 8 or act.data_ptr() % 16:
+        raise L.CstpError(f"gradcam: n = {n}, C = {C_} (a multiple of 8 up to {CAM_MAX_CHANNELS}) and Cp = {Cp} "
+                          f"do not fit an activation of {N} clips")
+    if alpha.dtype != torch.float32 or not alpha.is_contiguous() or alpha.numel() < n * C_ \
+            or cam.dtype != torch.float32 or not cam.is_contiguous() or cam.numel() < n * t * h * w:
+        raise L.CstpError("gradcam: alpha and cam must be contiguous fp32 with room for n x C and n x t x h x w values")
+    L.check(L.load().cstp_gradcam(_ptr(act), _ptr(grad), n, t * h * w, C_, Cp, _ptr(alpha), _ptr(cam), _stream()))
+
+
+def cam_upsample(cam, n: int, out) -> None:
+    """Trilinear upsampling (F.interpolate, align_corners=False) of cam fp32 (N, t, h, w) to out fp32 (N, T, H, W) and
+    per-clip min-max normalisation, over clips [0, n) (include/cstp_b200.h cstp_cam_upsample)."""
+    _require_cuda(cam, out)
+    if cam.dtype != torch.float32 or out.dtype != torch.float32 or cam.dim() != 4 or out.dim() != 4 \
+            or not cam.is_contiguous() or not out.is_contiguous() or not 1 <= n <= min(cam.shape[0], out.shape[0]):
+        raise L.CstpError(f"cam_upsample: cam and out must be contiguous fp32 (N, t, h, w) / (N, T, H, W) holding n = {n} "
+                          f"clips, got {cam.dtype} {tuple(cam.shape)} and {out.dtype} {tuple(out.shape)}")
+    _, t, h, w = cam.shape
+    _, T, H, W = out.shape
+    L.check(L.load().cstp_cam_upsample(_ptr(cam), n, t, h, w, T, H, W, _ptr(out), _stream()))
 
 
 KNN_MAX_K, KNN_MAX_SPLITS, KNN_QUERY_TILE, KNN_CTAS_PER_SM = 64, 32, 64, 3

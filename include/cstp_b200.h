@@ -428,6 +428,25 @@ int cstp_knn_merge(const float* part_val, const int32_t* part_idx, int nq, int k
                    float* sim_out, const int64_t* q_labels, const int64_t* g_labels, const int32_t* cutoffs, int n_cut,
                    int64_t* hits, void* stream);
 
+/* Grad-CAM of a finetuned classifier (csrc/explain.cu).  Every floating-point operation is one rounded _rn intrinsic in
+ * a fixed order, so a float32 stand-in reproduces the bits.
+ * cam_seed: for rows b < n, k = classes_in[b] (device int64, optional) or the argmax over the n_cls valid columns of
+ *   logits fp32 [B][ld] (ties to the lower class); classes_out[b] = k (int64), dlogits[b] = one-hot(k) fp32 [B][ld].
+ *   Rows >= n get class 0 and a zero row; padding columns are zero. */
+int cstp_cam_seed(const float* logits, int B, int ld, int n, int n_cls, const int64_t* classes_in, int64_t* classes_out,
+                  float* dlogits, void* stream);
+/* gradcam: act / grad bf16 NDHWC [n][P positions][Cp] (C valid channels, C % 8 == 0, C <= 512, act 16-byte aligned):
+ *   alpha[b][c] = (sum_p grad[b][p][c]) / P, the sum in eight interleaved position lanes (lane j: p = j, j + 8, ... in
+ *   order) then lane order; cam[b][p] = relu(sum_c alpha[b][c] * act[b][p][c]), rounded products added in channel order.
+ *   alpha fp32 [n][C], cam fp32 [n][P].  Two launches. */
+int cstp_gradcam(const void* act, const void* grad, int n, long long P, int C, int Cp, float* alpha, float* cam,
+                 void* stream);
+/* cam_upsample: cam fp32 [n][t][h][w] -> out fp32 [n][T][H][W], trilinear with torch's align_corners=False source index
+ *   (per axis: scale = in / out, src = max(scale * (d + 0.5) - 0.5, 0), i0 = (int)src, i1 = min(i0 + 1, in - 1),
+ *   l = src - i0; blends a + l * (b - a) along w, then h, then t), then per clip (v - min) / (max - min), zeros where
+ *   max == min. */
+int cstp_cam_upsample(const float* cam, int n, int t, int h, int w, int T, int H, int W, float* out, void* stream);
+
 /* ---- optimiser side -------------------------------------------------------------------------------------
  * EMA target update (r21d_byol.py:331-337): k = k*m + q*(1-m), bit-exact fp32 (two rounded products, one add). */
 int cstp_ema_update(float* k, const float* q, int64_t n, float m, float one_minus_m, void* stream);
